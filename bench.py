@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          our CUDA path
     python bench.py --impl reference ...                    the reference's CPU algorithm on the host cores
+    python bench.py ... --dump-outputs DIR                  also the last timed step's outputs, DIR/<name>.npy
 
 A step = one pass of the hot path over one batch of synthetic input of the shape
 BASELINE.json configs[1] names: `--states` random PR2 right-arm states plus as many
@@ -29,6 +30,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True     # no __pycache__: a benchmark run leaves the source tree as it found it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -289,16 +291,11 @@ def run_reference(args, rank, world):
     for _ in range(args.warmup):
         cpu_validity_rate(scene, q[: n // 8], q0[: n // 8], q1[: n // 8], threads, checkers)
     total_units, total_t = 0, 0.0
-    # bounded: the whole --steps K run must end within a few minutes whatever the host (a step is ~0.4 s on 16 threads)
-    budget_s = 150.0
-    steps_run = 0
-    for _ in range(args.steps):
+    steps_run = args.steps
+    for _ in range(steps_run):
         _, u, dt = cpu_validity_rate(scene, q, q0, q1, threads, checkers)
         total_units += u
         total_t += dt
-        steps_run += 1
-        if total_t > budget_s:
-            break
     value = total_units / total_t
     units_per_step = total_units // steps_run
     line = {
@@ -331,6 +328,24 @@ def wandering_paths(anchors, n_paths, dof, seed):
             pts = a + t * (b - a) * 0.4
         paths.append(np.ascontiguousarray(pts[:m]))
     return paths
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each equal-length device array as out_dir/<name>.npy in float32 (verdicts and waypoint counts are
+    exact in it).  Above DUMP_BYTES in all, every array keeps the same elements: a sorted sample drawn with seed 0,
+    so that two builds run with the same arguments still compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.cpu().numpy() for k, v in arrays.items()}
+    n = len(next(iter(host.values())))
+    room = (DUMP_BYTES - 128 * len(host)) // (4 * len(host))     # elements per array, 128-byte .npy headers included
+    if n > room:
+        idx = np.sort(np.random.default_rng(0).choice(n, room, replace=False))
+        host = {k: v[idx] for k, v in host.items()}
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.astype(np.float32))
 
 
 def timed_events(torch, fn, reps):
@@ -565,7 +580,8 @@ def dual_arm_leg(api, scenes, sharding, dist, torch, dev, args, rank, world, loc
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the validity sweep (the value); the e2e legs time max(3, steps // 2) steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="smpl_b200", choices=["smpl_b200", "reference"])
     ap.add_argument("--states", type=int, default=1 << 20, help="states (and edges) per step per GPU")
@@ -586,7 +602,14 @@ def main():
     ap.add_argument("--no-ingest", dest="ingest", action="store_false", help="skip the scene-ingest leg")
     ap.add_argument("--e2e-threads", type=int, default=0, help="host threads (= contexts) of the end-to-end leg; 0 = min(8, cores per rank)")
     ap.add_argument("--plan-threads", type=int, default=0, help="planner threads (= contexts) per GPU; 0 = 75 %% of the rank's cores, at most 6")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the verdicts and waypoint counts of the last timed step to DIR/<name>.npy (float32); with "
+                         "several ranks, rank 0's (each rank sweeps its own seeded batch)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "smpl_b200":
+        ap.error("--dump-outputs writes the outputs of --impl smpl_b200")
     args.warmup = max(args.warmup, 3) if args.impl == "smpl_b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -660,6 +683,8 @@ def main():
         ctx.is_edges_valid_dev(d_q.data_ptr(), d_q1.data_ptr(), n, d_ev.data_ptr(), d_cnt.data_ptr())
         ev[2 * s + 2].record()
     barrier()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"states_valid": d_v, "edges_valid": d_ev, "edges_waypoint_count": d_cnt})
     gpu_launches = ctx.launch_count() - launches0
     total_ms = ev[0].elapsed_time(ev[-1])
     states_ms = np.mean([ev[2 * s].elapsed_time(ev[2 * s + 1]) for s in range(args.steps)])

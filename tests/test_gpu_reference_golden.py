@@ -1,6 +1,6 @@
-"""The CUDA path against the REFERENCE's own collision checker: tests/golden/collision_reference.npz holds states,
-edges, verdicts and waypoint counts produced by sbpl_collision_checking compiled from /root/reference
-(oracle/_ref/libref_collision.so, tools/gen_golden_collision.py).  Everything goes through the C ABI
+"""The CUDA path against the REFERENCE's own collision checker: tests/golden/collision_reference.npz holds verdicts and
+waypoint counts for seeded states and edges (golden_inputs), produced by sbpl_collision_checking compiled from the
+reference sources (oracle/_ref/libref_collision.so, tools/gen_golden_collision.py).  Everything goes through the C ABI
 (smplgpu_is_states_valid / smplgpu_is_edges_valid) in both precision modes; verdicts and waypoint counts must be equal."""
 import os
 
@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 from smpl_b200 import api
-from test_oracle_collision import CASES, GOLDEN, case_scene
+from test_oracle_collision import CASES, GOLDEN, case_scene, golden_inputs
 
 pytestmark = pytest.mark.gpu
 
@@ -39,7 +39,7 @@ def test_cuda_verdicts_equal_reference_build(name):
     scene, attach = case_scene(name)
     ctx = setup(scene, attach)
     try:
-        q, q0, q1 = g[name + "/q"], g[name + "/q0"], g[name + "/q1"]
+        q, q0, q1 = golden_inputs(g, name)
         for mode in (api.GpuContext.CERTIFIED_F32, api.GpuContext.EXACT_F64):
             ctx.set_precision_mode(mode)
             v = ctx.is_states_valid(q)

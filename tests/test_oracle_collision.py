@@ -12,8 +12,8 @@ on the PR2 right arm (tabletop = config 1, clutter = config 2, box objects at ar
 CollisionSpace::insertObject, padding), the UBR1 arm with a box attached through CollisionSpace::attachObject and
 extra ACM entries (config 4 shape) and the 15-DOF torso + both arms group (config 5 shape, coarser grid).
 
-tests/golden/collision_reference.npz holds inputs + outputs of that reference build (tools/gen_golden_collision.py);
-the oracle is checked against it where oracle/_ref is absent.
+tests/golden/collision_reference.npz holds outputs of that reference build with what regenerates its inputs
+(tools/gen_golden_collision.py); the oracle is checked against it where oracle/_ref is absent.
 """
 import os
 
@@ -97,10 +97,10 @@ def make_restatement(scene, attach, with_kdl=False):
     return o
 
 
-def case_inputs(scene, r, n_states, n_edges, seed):
-    """Random states inside the limits the reference's model reports, lattice-sized edges plus long random edges
-    (many waypoints)."""
-    lo, hi, cont = r.limits()
+def case_inputs(scene, limits, n_states, n_edges, seed):
+    """Random states inside `limits` (lo, hi, continuous: what the reference's model reports), lattice-sized edges plus
+    long random edges (many waypoints)."""
+    lo, hi, cont = limits
     q = scenes.random_states(n_states, lo, hi, cont, seed=seed)
     rng = np.random.Generator(np.random.PCG64(seed + 1))
     q0 = q[:n_edges].copy()
@@ -109,6 +109,17 @@ def case_inputs(scene, r, n_states, n_edges, seed):
     prim = rng.integers(-7, 8, size=(half, scene.dof)) * np.pi / 180.0        # lattice moves of up to 7 degrees
     q1[:half] += prim * (np.asarray(hi) - np.asarray(lo) > 0.5)                  # prismatic torso: stays put
     q1[half:] = q0[half:] + rng.uniform(-0.6, 0.6, size=(n_edges - half, scene.dof)) * np.minimum(1.0, (np.asarray(hi) - np.asarray(lo)))
+    return q, q0, q1
+
+
+def golden_inputs(g, name):
+    """The states and edges the reference build checked for GOLDEN: case_inputs(seed=211) under the limits stored with
+    them.  The file keeps every 50th row of q and q1 rather than all of them; those rows must come out the same."""
+    scene, _ = case_scene(name)
+    limits = g[name + "/limits_lo"], g[name + "/limits_hi"], g[name + "/limits_continuous"]
+    q, q0, q1 = case_inputs(scene, limits, 1500, 600, seed=211)
+    assert np.array_equal(q[::50], g[name + "/q_rows"]) and np.array_equal(q1[::50], g[name + "/q1_rows"]), \
+        "regenerated inputs differ from the ones the reference build saw"
     return q, q0, q1
 
 
@@ -124,7 +135,7 @@ def test_restatement_equals_reference_build(name):
     nt_o, nt_r = o.node_table(), r.node_table()
     assert nt_o.shape == nt_r.shape and np.array_equal(nt_o, nt_r)
     assert np.array_equal(o.motion_weights()[0], r.motion_weights())
-    q, q0, q1 = case_inputs(scene, r, 3000, 1200, seed=101)
+    q, q0, q1 = case_inputs(scene, r.limits(), 3000, 1200, seed=101)
     # FK of every sphere-tree node: bit for bit
     c_o = np.asarray(o.sphere_centers(q[:300])).reshape(300, len(nt_r), 3)
     c_r = r.sphere_centers(q[:300], len(nt_r))
@@ -152,7 +163,7 @@ def test_detach_restores_verdicts():
     o = make_restatement(scene, attach)
     r_with = make_reference(scene, attach)
     r_without = make_reference(scene, None)
-    q, _, _ = case_inputs(scene, r_with, 1500, 10, seed=7)
+    q, _, _ = case_inputs(scene, r_with.limits(), 1500, 10, seed=7)
     with_body = r_with.is_states_valid(q)
     assert np.array_equal(with_body, o.is_states_valid(q))
     assert o.detach("object") == 0
@@ -167,10 +178,11 @@ def test_restatement_equals_golden_reference_outputs():
     for name in CASES:
         scene, attach = case_scene(name)
         o = make_restatement(scene, attach)
-        q, q0, q1 = g[name + "/q"], g[name + "/q0"], g[name + "/q1"]
+        q, q0, q1 = golden_inputs(g, name)
         assert np.array_equal(o.node_table(), g[name + "/node_table"])
         n_nodes = len(g[name + "/node_table"])
-        assert np.array_equal(np.asarray(o.sphere_centers(q[:64])).reshape(64, n_nodes, 3), g[name + "/centers"])
+        k = len(g[name + "/centers"])
+        assert np.array_equal(np.asarray(o.sphere_centers(q[:k])).reshape(k, n_nodes, 3), g[name + "/centers"])
         assert np.array_equal(o.is_states_valid(q), g[name + "/states_valid"])
         e, n = o.is_edges_valid(q0, q1)
         assert np.array_equal(e, g[name + "/edges_valid"])
@@ -223,7 +235,7 @@ def test_collision_distance_equals_reference_build(name):
     scene, attach = case_scene(name)
     o = make_restatement(scene, attach)
     r = make_reference(scene, attach)
-    q, _, _ = case_inputs(scene, r, 2000, 10, seed=5)
+    q, _, _ = case_inputs(scene, r.limits(), 2000, 10, seed=5)
     d_o, d_r = o.collision_distance(q), r.collision_distance(q)
     assert np.array_equal(d_o, d_r)
     # a clearance of 0 is what an invalid state gets from the field term (a failing leaf has obs_dist < 0)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Writes tests/golden/collision_reference.npz: inputs + outputs of the REFERENCE's own collision checker
-(oracle/_ref/libref_collision.so, built by `make -C oracle ref` from /root/reference; see
-oracle/ref_collision_shim.cpp) for the cases of tests/test_oracle_collision.py.  Run in the authoring container."""
+"""Writes tests/golden/collision_reference.npz: outputs of the REFERENCE's own collision checker and what regenerates
+its inputs (oracle/_ref/libref_collision.so, built by `make -C oracle ref REF=<checkout of the reference sources>`;
+see oracle/ref_collision_shim.cpp) for the cases of tests/test_oracle_collision.py.  Needs that build."""
 import os
 import sys
 
@@ -19,12 +19,16 @@ def main():
     for name in T.CASES:
         scene, attach = T.case_scene(name)
         r = T.make_reference(scene, attach)
-        q, q0, q1 = T.case_inputs(scene, r, 1500, 600, seed=211)
+        lo, hi, cont = r.limits()
+        q, q0, q1 = T.case_inputs(scene, (lo, hi, cont), 1500, 600, seed=211)
         nt = r.node_table()
         e, n = r.is_edges_valid(q0, q1)
-        out[name + "/q"] = q
-        out[name + "/q0"] = q0
-        out[name + "/q1"] = q1
+        # the inputs are regenerated from the seed (T.golden_inputs); every 50th row is kept to check that
+        out[name + "/limits_lo"] = lo
+        out[name + "/limits_hi"] = hi
+        out[name + "/limits_continuous"] = cont
+        out[name + "/q_rows"] = q[::50]
+        out[name + "/q1_rows"] = q1[::50]
         out[name + "/node_table"] = nt
         out[name + "/centers"] = r.sphere_centers(q[:64], len(nt))
         out[name + "/states_valid"] = r.is_states_valid(q)

@@ -24,7 +24,7 @@ def main():
     for name in CASES:
         scene, attach = case_scene(name)
         r = make_reference(scene, attach)
-        q, _, _ = case_inputs(scene, r, 1500, 10, seed=77)
+        q, _, _ = case_inputs(scene, r.limits(), 1500, 10, seed=77)
         out[name + "/q"] = q
         out[name + "/distance"] = r.collision_distance(q)
         print(name, "min %.4f max %.4f zero %.2f" % (out[name + "/distance"].min(), out[name + "/distance"].max(),
