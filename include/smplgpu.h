@@ -38,6 +38,8 @@ extern "C" {
 #define SMPLGPU_ERR_NO_DEVICE   -4  /* no usable CUDA device */
 #define SMPLGPU_ERR_LIMIT       -5  /* table exceeds a compiled-in limit */
 
+#define SMPLGPU_MAX_DOF 16          /* planning variables */
+
 /* BFS_3D cell values (smpl/bfs3d/bfs3d.h:50-51) */
 #define SMPLGPU_BFS_WALL          0x7FFFFFFF
 #define SMPLGPU_BFS_UNDISCOVERED  (-1)
@@ -400,9 +402,36 @@ int smplgpu_lattice_max_slots(smplgpu_ctx* ctx, int max_states);
 int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* params, int n_slots);
 /* setGoal + setStart bookkeeping for n queries: slot[i] gets an empty lattice, goal position goals_xyz[i] and start
  * state starts[i] (id 1) whose metric goal distance is start_goal_dist_cells[i] (smplgpu_expand_batch reports it).
+ * The goal is an XYZ goal with the xyz_tolerance of smplgpu_lattice_params.
  * The slot's BFS (smplgpu_bfs_bank_run_slots*) must have run. */
 int smplgpu_lattice_begin(smplgpu_ctx* ctx, const int32_t* slots, const double* starts,
                           const int32_t* start_goal_dist_cells, const double* goals_xyz, int n);
+
+/* GoalConstraint (smpl/planning_params.h; smpl_b200/host/smpl/interfaces.h:49-62) and the three branches of
+ * ManipLattice::isGoal (manip_lattice.cpp:1582-1696).  `pose` of a state is the target-offset planning-frame pose
+ * x y z roll pitch yaw (smplgpu_planning_frame_fk).
+ *   SMPLGPU_GOAL_XYZ          |pose[a] - goal.pose[a]| <= xyz_tolerance[a], a = 0, 1, 2
+ *   SMPLGPU_GOAL_XYZ_RPY      the XYZ test, then theta < rpy_tolerance, where theta = normalize_angle(2 acos(q . qg)),
+ *                             q and qg = AngleAxis(yaw, Z) * AngleAxis(pitch, Y) * AngleAxis(roll, X) of the state's
+ *                             and of the goal's rpy, qg negated when q . qg < 0 (no clamp: |q . qg| > 1 is no goal)
+ *   SMPLGPU_GOAL_JOINT_STATE  |state[i] - angles[i]| <= angle_tolerances[i] for every planning variable (no wrapping)
+ * A type reads only its own fields.  The BFS heuristic is seeded at the goal position: pose[0..2], or for a joint goal
+ * the target-offset position of `angles` (ManipLattice::setGoalConfiguration), which the caller computes. */
+#define SMPLGPU_GOAL_XYZ          0
+#define SMPLGPU_GOAL_XYZ_RPY      1
+#define SMPLGPU_GOAL_JOINT_STATE  2
+typedef struct smplgpu_goal {
+    int32_t type;                              /* SMPLGPU_GOAL_* */
+    double  pose[6];                           /* x y z roll pitch yaw (XYZ, XYZ_RPY) */
+    double  xyz_tolerance[3];                  /* metres (XYZ, XYZ_RPY) */
+    double  rpy_tolerance;                     /* radians (XYZ_RPY) */
+    double  angles[SMPLGPU_MAX_DOF];           /* [dof] (JOINT_STATE) */
+    double  angle_tolerances[SMPLGPU_MAX_DOF]; /* [dof] (JOINT_STATE) */
+} smplgpu_goal;
+/* smplgpu_lattice_begin with a goal record per query (types may be mixed).  The goal quaternion of an XYZ_RPY goal is
+ * computed here, on the host.  An unknown type, or a NaN or negative tolerance the type reads, is SMPLGPU_ERR_INVALID. */
+int smplgpu_lattice_begin_goals(smplgpu_ctx* ctx, const int32_t* slots, const double* starts,
+                                const int32_t* start_goal_dist_cells, const smplgpu_goal* goals, int n);
 /* One round: expansion i expands state parent_id[i] of the query in slot[i] (at most one expansion per slot and
  * round).  submit queues the work and returns; wait blocks and hands out pointers into page-locked memory valid
  * until the next submit on `buffer` (0 .. SMPLGPU_EXPAND_BUFFERS - 1):
@@ -439,7 +468,6 @@ int smplgpu_is_lattice_edges_valid(smplgpu_ctx* ctx, const int16_t* parent_coord
  * every successor parent + deltas[k] (info[1 + k]) of the table given to smplgpu_set_motion_primitives.  The
  * adapters of smpl_b200/host/gpu_adapters.cpp call it on a cache miss and serve the following virtual calls
  * from the record. */
-#define SMPLGPU_MAX_DOF 16
 typedef struct smplgpu_succ_info {
     double  state[SMPLGPU_MAX_DOF]; /* info[0]: the parent; info[1+k]: deltas[k][j] + parent[j] (one IEEE addition) */
     double  pose[6];                /* computePlanningLinkFK + getTargetOffsetPose of `state`: x y z roll pitch yaw */

@@ -108,6 +108,15 @@ int smplhost_plan_batch_multi(smplgpu_ctx* const* ctxs, int n_ctx, const smplhos
                               const double* starts, const double* goals, int nq, int max_concurrent_per_ctx,
                               int32_t* summary, int32_t* path_ids, int max_path, double* stats, double* path_states);
 
+/* smplhost_plan_batch_multi with one GoalConstraint per query (smplgpu_goal; types may be mixed): pose goals with an
+ * orientation tolerance and joint-configuration goals besides XYZ goals (params->xyz_tolerance is not read).  The
+ * goal positions of all joint goals are computed in one smplgpu_planning_frame_fk call before the first query starts.
+ * n_ctx = 1 is the single-context case.  An unknown goal type or a NaN or negative tolerance is SMPLGPU_ERR_INVALID
+ * before anything is planned. */
+int smplhost_plan_batch_goals(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* params,
+                              const double* starts, const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx,
+                              int32_t* summary, int32_t* path_ids, int max_path, double* stats, double* path_states);
+
 /* ---- drop-in adapters (smpl_b200/host/gpu_adapters.h): the reference's CollisionChecker / RobotModel /
  * RobotHeuristic virtuals implemented over the C ABI.  These shims drive the C++ objects one virtual call at
  * a time, the way the reference's planner does (n = 1 per call); a C++ caller uses the classes directly. ---- */

@@ -43,6 +43,51 @@ class SuccInfoC(C.Structure):
                 ("limits_ok", C.c_uint8), ("state_valid", C.c_uint8), ("is_parent", C.c_uint8)]
 
 
+MAX_DOF = 16   # SMPLGPU_MAX_DOF
+GOAL_XYZ, GOAL_XYZ_RPY, GOAL_JOINT_STATE = 0, 1, 2   # SMPLGPU_GOAL_*
+
+
+class GoalC(C.Structure):
+    """smplgpu_goal (include/smplgpu.h): GoalConstraint of one query."""
+    _fields_ = [("type", C.c_int32), ("pose", C.c_double * 6), ("xyz_tolerance", C.c_double * 3),
+                ("rpy_tolerance", C.c_double), ("angles", C.c_double * MAX_DOF),
+                ("angle_tolerances", C.c_double * MAX_DOF)]
+
+
+GOAL_DTYPE = np.dtype(GoalC)   # goal records as a numpy structured array: concatenate / index them like any array
+
+
+def pose_goals(poses, xyz_tolerance=(0.015, 0.015, 0.015), rpy_tolerance=None):
+    """Goal records for target-offset poses.  poses: (n, 3) positions or (n, 6) x y z roll pitch yaw.
+    rpy_tolerance None: XYZ goals (orientation ignored); a number: XYZ_RPY goals, the state is a goal when its
+    orientation is within that angle of the goal's (ManipLattice::isGoal)."""
+    poses = np.asarray(poses, np.float64)
+    poses = poses.reshape(-1, poses.shape[-1])
+    if rpy_tolerance is not None and poses.shape[1] != 6:
+        raise ValueError("pose goals with an orientation tolerance need x y z roll pitch yaw")
+    out = np.zeros(len(poses), GOAL_DTYPE)
+    out["type"] = GOAL_XYZ if rpy_tolerance is None else GOAL_XYZ_RPY
+    out["pose"][:, :poses.shape[1]] = poses
+    out["xyz_tolerance"] = np.broadcast_to(np.asarray(xyz_tolerance, np.float64), (len(poses), 3))
+    out["rpy_tolerance"] = 0.0 if rpy_tolerance is None else float(rpy_tolerance)
+    return out
+
+
+def joint_goals(angles, angle_tolerances):
+    """Goal records for joint configurations: angles (n, dof); angle_tolerances (dof,) or (n, dof).  The state is a
+    goal when every planning variable is within its tolerance (no angle wrapping)."""
+    angles = np.asarray(angles, np.float64)
+    angles = angles.reshape(-1, angles.shape[-1])
+    n, dof = angles.shape
+    if dof > MAX_DOF:
+        raise ValueError("more than %d planning variables" % MAX_DOF)
+    out = np.zeros(n, GOAL_DTYPE)
+    out["type"] = GOAL_JOINT_STATE
+    out["angles"][:, :dof] = angles
+    out["angle_tolerances"][:, :dof] = np.broadcast_to(np.asarray(angle_tolerances, np.float64), (n, dof))
+    return out
+
+
 class PlanParamsC(C.Structure):
     """smplhost_plan_params (include/smplhost.h)."""
     _fields_ = [("dof", C.c_int), ("resolutions", c_double_p), ("mprims", c_double_p), ("short_flags", c_uint8_p),
@@ -161,6 +206,9 @@ def host_lib():
                                           c_int32_p, c_int32_p, C.c_int, c_double_p, c_double_p]
         H.smplhost_plan_batch_multi.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PlanParamsC), c_double_p, c_double_p,
                                                 C.c_int, C.c_int, c_int32_p, c_int32_p, C.c_int, c_double_p, c_double_p]
+        H.smplhost_plan_batch_goals.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PlanParamsC), c_double_p,
+                                                C.POINTER(GoalC), C.c_int, C.c_int, c_int32_p, c_int32_p, C.c_int,
+                                                c_double_p, c_double_p]
         H.smplhost_shortcut_paths.argtypes = [vp, C.c_int, c_uint8_p, c_double_p, c_int32_p, C.c_int, C.c_int, c_int32_p,
                                               c_int32_p, c_double_p]
         H.smplhost_interpolate_paths.argtypes = [vp, vp, c_double_p, c_int32_p, C.c_int, c_double_p, C.c_int, c_int32_p,
@@ -769,12 +817,20 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
                want_states=False):
     """smplhost_plan_batch: many ARA* queries in lock step, one device call per round.
     params: smpl_b200.scenes.PlanParams.  Returns (list of dict per query, stats dict).
+    goals: (nq, 3) positions (XYZ goals with params.xyz_tolerance), or goal records of GOAL_DTYPE (pose_goals,
+    joint_goals; types may be mixed), which go through smplhost_plan_batch_goals.
     `ctx` may be a list of contexts (same GPU, same scene): one planner thread per context
     (smplhost_plan_batch_multi), max_concurrent is then per context."""
     H = host_lib()
     dof = tables.dof
     starts = np.ascontiguousarray(starts, dtype=np.float64).reshape(-1, dof)
-    goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(-1, 3)
+    records = isinstance(goals, np.ndarray) and goals.dtype == GOAL_DTYPE
+    if records:
+        goals = np.ascontiguousarray(goals.reshape(-1))
+    else:
+        goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(-1, 3)
+    if len(goals) != len(starts):
+        raise ValueError("%d starts, %d goals" % (len(starts), len(goals)))
     nq = len(starts)
     lo, hi, cont = tables.limits()
     res = np.ascontiguousarray(params.resolutions, dtype=np.float64)
@@ -803,7 +859,12 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
     stats = np.zeros(12)
     pstates = np.zeros((nq, max_path, dof), np.float64) if want_states else None
     ps_ptr = _dp(pstates) if want_states else None
-    if isinstance(ctx, (list, tuple)):
+    if records:
+        ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
+        arr = (C.c_void_p * len(ctxs))(*[c.h for c in ctxs])
+        r = H.smplhost_plan_batch_goals(arr, len(ctxs), C.byref(P), _dp(starts), goals.ctypes.data_as(C.POINTER(GoalC)), nq,
+                                        int(max_concurrent), _ip(summary), _ip(paths), int(max_path), _dp(stats), ps_ptr)
+    elif isinstance(ctx, (list, tuple)):
         arr = (C.c_void_p * len(ctx))(*[c.h for c in ctx])
         r = H.smplhost_plan_batch_multi(arr, len(ctx), C.byref(P), _dp(starts), _dp(goals), nq, int(max_concurrent),
                                         _ip(summary), _ip(paths), int(max_path), _dp(stats), ps_ptr)

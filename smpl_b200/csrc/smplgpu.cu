@@ -138,6 +138,7 @@ struct smplgpu_ctx
     LatticeBank lat{};
     LatticeParams lat_params{};
     LatticeVals lat_vals{};
+    double lat_xyz_tol[3] = { 0, 0, 0 };    // smplgpu_lattice_params::xyz_tolerance (the goals of smplgpu_lattice_begin)
     void* d_lat_aux = nullptr;              // deltas | long list | short list
     void* lat_in[SMPLGPU_EXPAND_BUFFERS] = { };  size_t lat_in_cap[SMPLGPU_EXPAND_BUFFERS] = { };   // pinned, mapped: slot | parent
     void* lat_out[SMPLGPU_EXPAND_BUFFERS] = { }; size_t lat_out_cap[SMPLGPU_EXPAND_BUFFERS] = { };  // pinned, mapped: succ | h | count | resolved
@@ -3051,7 +3052,7 @@ int smplgpu_expand_batch(smplgpu_ctx* ctx, const double* q0, const double* q1, c
 static size_t lattice_bytes_per_slot(int dof, int cap, int table_size)
 {
     return (size_t)cap * dof * (sizeof(double) + sizeof(int)) + (size_t)cap * sizeof(int) + (size_t)table_size * sizeof(int) +
-           sizeof(int) + 3 * sizeof(double);
+           sizeof(int) + sizeof(LatticeGoal);
 }
 
 static int lattice_table_size(int cap)
@@ -3111,7 +3112,7 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
         CU(cudaMalloc(&B.gdist, (size_t)n_slots * cap * sizeof(int)));
         CU(cudaMalloc(&B.table, (size_t)n_slots * tsize * sizeof(int)));
         CU(cudaMalloc(&B.count, (size_t)n_slots * sizeof(int)));
-        CU(cudaMalloc(&B.goal, (size_t)n_slots * 3 * sizeof(double)));
+        CU(cudaMalloc(&B.goal, (size_t)n_slots * sizeof(LatticeGoal)));
         CU(cudaMemset(B.count, 0, (size_t)n_slots * sizeof(int)));
     }
     LatticeBank& B = ctx->lat;
@@ -3121,7 +3122,7 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
     B.short_dist_thresh = p->short_dist_thresh;
     B.res = ctx->res;
     B.cost_per_cell = p->cost_per_cell;
-    for (int a = 0; a < 3; ++a) B.tol[a] = p->xyz_tolerance[a];
+    for (int a = 0; a < 3; ++a) ctx->lat_xyz_tol[a] = p->xyz_tolerance[a];
     // deltas | long list | short list
     const size_t db = (size_t)p->n_prims * dof * sizeof(double);
     const size_t lb = ((size_t)p->n_prims * sizeof(int) + 7) / 8 * 8;
@@ -3183,27 +3184,46 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
     return stride;
 }
 
-int smplgpu_lattice_begin(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
-                          const double* goals_xyz, int n)
+// Quaterniond(AngleAxisd(yaw, Z) * AngleAxisd(pitch, Y) * AngleAxisd(roll, X)), x y z w: the operation order of the
+// oracle's Eigen stand-in (oracle/goals/goal_lattice.cpp quatFromRpy), with the host's libm
+static void quat_from_rpy(double roll, double pitch, double yaw, double* q)
 {
-    if (!ctx || n < 0) return SMPLGPU_ERR_INVALID;
-    if (!ctx->has_lat) return fail(ctx, SMPLGPU_ERR_STATE, "lattices not created (smplgpu_lattice_create)");
-    if (n == 0) return 0;
-    if (!slots || !starts || !start_gd || !goals_xyz) return fail(ctx, SMPLGPU_ERR_INVALID, "null pointer");
-    for (int i = 0; i < n; ++i) {
-        if (slots[i] < 0 || slots[i] >= ctx->lat.n_slots) return fail(ctx, SMPLGPU_ERR_INVALID, "slot %d out of range", slots[i]);
-    }
+    const double hz = 0.5 * yaw, hy = 0.5 * pitch, hx = 0.5 * roll;
+    const double sz = std::sin(hz), sy = std::sin(hy), sx = std::sin(hx);
+    const double a[4] = { sz * 0.0, sz * 0.0, sz * 1.0, std::cos(hz) };
+    const double b[4] = { sy * 0.0, sy * 1.0, sy * 0.0, std::cos(hy) };
+    const double c[4] = { sx * 1.0, sx * 0.0, sx * 0.0, std::cos(hx) };
+    auto mul = [](const double* l, const double* r, double* o) {   // Eigen's generic quat_product
+        o[3] = l[3] * r[3] - l[0] * r[0] - l[1] * r[1] - l[2] * r[2];
+        o[0] = l[3] * r[0] + l[0] * r[3] + l[1] * r[2] - l[2] * r[1];
+        o[1] = l[3] * r[1] + l[1] * r[3] + l[2] * r[0] - l[0] * r[2];
+        o[2] = l[3] * r[2] + l[2] * r[3] + l[0] * r[1] - l[1] * r[0];
+    };
+    double ab[4];
+    mul(a, b, ab);
+    mul(ab, c, q);
+}
+
+static bool bad_tolerance(double t)
+{
+    return std::isnan(t) || t < 0.0;
+}
+
+static int lattice_begin_records(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
+                                 const std::vector<LatticeGoal>& goals, int n)
+{
     const int dof = ctx->h_model->dof;
-    const size_t sb = ((size_t)n * sizeof(int) + 7) / 8 * 8, qb = (size_t)n * dof * sizeof(double), gb = (size_t)n * 3 * sizeof(double);
+    const size_t sb = ((size_t)n * sizeof(int) + 7) / 8 * 8, qb = (size_t)n * dof * sizeof(double),
+                 gb = (size_t)n * sizeof(LatticeGoal);
     int r = grow(ctx, &ctx->d_misc, &ctx->misc_cap, 2 * sb + qb + gb + 64);
     if (r) return r;
     uint8_t* base = (uint8_t*)ctx->d_misc;
     double* d_starts = (double*)base;
-    double* d_goals = (double*)(base + qb);
+    LatticeGoal* d_goals = (LatticeGoal*)(base + qb);
     int* d_slots = (int*)(base + qb + gb);
     int* d_gd = (int*)(base + qb + gb + sb);
     CU(cudaMemcpyAsync(d_starts, starts, qb, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(d_goals, goals_xyz, gb, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_goals, goals.data(), gb, cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaMemcpyAsync(d_slots, slots, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaMemcpyAsync(d_gd, start_gd, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     const size_t total = (size_t)n * ctx->lat.table_size;
@@ -3214,6 +3234,72 @@ int smplgpu_lattice_begin(smplgpu_ctx* ctx, const int32_t* slots, const double* 
     CU(cudaGetLastError());
     CU(cudaStreamSynchronize(ctx->stream));   // the inputs may be pageable
     return 0;
+}
+
+static int lattice_begin_check(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
+                               const void* goals, int n)
+{
+    if (!ctx->has_lat) return fail(ctx, SMPLGPU_ERR_STATE, "lattices not created (smplgpu_lattice_create)");
+    if (n == 0) return 0;
+    if (!slots || !starts || !start_gd || !goals) return fail(ctx, SMPLGPU_ERR_INVALID, "null pointer");
+    for (int i = 0; i < n; ++i) {
+        if (slots[i] < 0 || slots[i] >= ctx->lat.n_slots) return fail(ctx, SMPLGPU_ERR_INVALID, "slot %d out of range", slots[i]);
+    }
+    return 0;
+}
+
+int smplgpu_lattice_begin(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
+                          const double* goals_xyz, int n)
+{
+    if (!ctx || n < 0) return SMPLGPU_ERR_INVALID;
+    int r = lattice_begin_check(ctx, slots, starts, start_gd, goals_xyz, n);
+    if (r || n == 0) return r;
+    std::vector<LatticeGoal> recs(n);   // zero-filled
+    for (int i = 0; i < n; ++i) {
+        LatticeGoal& g = recs[i];
+        g.type = SMPLGPU_GOAL_XYZ;
+        for (int a = 0; a < 3; ++a) {
+            g.xyz[a] = goals_xyz[3 * i + a];
+            g.xyz_tol[a] = ctx->lat_xyz_tol[a];
+        }
+    }
+    return lattice_begin_records(ctx, slots, starts, start_gd, recs, n);
+}
+
+int smplgpu_lattice_begin_goals(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
+                                const smplgpu_goal* goals, int n)
+{
+    if (!ctx || n < 0) return SMPLGPU_ERR_INVALID;
+    int r = lattice_begin_check(ctx, slots, starts, start_gd, goals, n);
+    if (r || n == 0) return r;
+    const int dof = ctx->h_model->dof;
+    std::vector<LatticeGoal> recs(n);   // zero-filled
+    for (int i = 0; i < n; ++i) {
+        const smplgpu_goal& in = goals[i];
+        LatticeGoal& g = recs[i];
+        g.type = in.type;
+        if (in.type == SMPLGPU_GOAL_XYZ || in.type == SMPLGPU_GOAL_XYZ_RPY) {
+            for (int a = 0; a < 3; ++a) {
+                if (bad_tolerance(in.xyz_tolerance[a])) return fail(ctx, SMPLGPU_ERR_INVALID, "goal %d: xyz tolerance %d is NaN or negative", i, a);
+                g.xyz[a] = in.pose[a];
+                g.xyz_tol[a] = in.xyz_tolerance[a];
+            }
+            if (in.type == SMPLGPU_GOAL_XYZ_RPY) {
+                if (bad_tolerance(in.rpy_tolerance)) return fail(ctx, SMPLGPU_ERR_INVALID, "goal %d: rpy tolerance is NaN or negative", i);
+                g.rpy_tol = in.rpy_tolerance;
+                quat_from_rpy(in.pose[3], in.pose[4], in.pose[5], g.qg);
+            }
+        } else if (in.type == SMPLGPU_GOAL_JOINT_STATE) {
+            for (int v = 0; v < dof; ++v) {
+                if (bad_tolerance(in.angle_tolerances[v])) return fail(ctx, SMPLGPU_ERR_INVALID, "goal %d: angle tolerance %d is NaN or negative", i, v);
+                g.angles[v] = in.angles[v];
+                g.angle_tol[v] = in.angle_tolerances[v];
+            }
+        } else {
+            return fail(ctx, SMPLGPU_ERR_INVALID, "goal %d: unknown goal type %d", i, in.type);
+        }
+    }
+    return lattice_begin_records(ctx, slots, starts, start_gd, recs, n);
 }
 
 int smplgpu_lattice_expand_submit(smplgpu_ctx* ctx, const int32_t* slot, const int32_t* parent_id, int n, int buffer)

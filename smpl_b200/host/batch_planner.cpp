@@ -323,7 +323,7 @@ void BatchPlanner::Pool::run(const std::function<void(int)>& f)
 // per-query steps
 ///////////////////////////////////////////////////////////////////////////////
 
-void BatchPlanner::initQuery(Query& Q, int index, int slot, const double* goal)
+void BatchPlanner::initQuery(Query& Q, int index, int slot, const smplgpu_goal* goal, const double* goal_xyz)
 {
     // keep the slot's allocations from the query it served before (growing a multi-megabyte vector means mmap +
     // copy + munmap, and every munmap interrupts all planner threads); a fresh slot reserves room up front
@@ -343,9 +343,10 @@ void BatchPlanner::initQuery(Query& Q, int index, int slot, const double* goal)
     Q.expanding = -1;
     Q.edge_begin = 0;
     Q.num_states = 1;   // id 0 = the goal state (manip_lattice.cpp:122)
-    for (int a = 0; a < 3; ++a) Q.goal[a] = goal[a];
+    Q.goal = goal;
+    for (int a = 0; a < 3; ++a) Q.goal_xyz[a] = goal_xyz[a];
     int cell[3];
-    worldToGrid(Q.goal, cell);
+    worldToGrid(Q.goal_xyz, cell);
     const bool inb = cell[0] >= 0 && cell[1] >= 0 && cell[2] >= 0 &&
                      cell[0] < m_cfg.dims[0] && cell[1] < m_cfg.dims[1] && cell[2] < m_cfg.dims[2];
     // the seed cell holds distance 0 even if it was a wall (bfs3d.cpp:181-187)
@@ -436,6 +437,20 @@ void BatchPlanner::absorbOne(Query& Q, const int32_t* succ, const int32_t* h, in
 
 bool BatchPlanner::plan(const double* starts, const double* goals, int nq, std::vector<QueryResult>& out, std::string* err)
 {
+    std::vector<smplgpu_goal> recs(nq);
+    for (int i = 0; i < nq; ++i) {
+        smplgpu_goal& g = recs[i];   // zero-filled
+        g.type = SMPLGPU_GOAL_XYZ;
+        for (int a = 0; a < 3; ++a) {
+            g.pose[a] = goals[3 * (size_t)i + a];
+            g.xyz_tolerance[a] = m_cfg.xyz_tolerance[a];
+        }
+    }
+    return plan(starts, recs.data(), nq, out, err);
+}
+
+bool BatchPlanner::plan(const double* starts, const smplgpu_goal* goals, int nq, std::vector<QueryResult>& out, std::string* err)
+{
     out.assign(nq, QueryResult());
     m_stats = BatchStats();
     if (nq == 0) {
@@ -447,6 +462,29 @@ bool BatchPlanner::plan(const double* starts, const double* goals, int nq, std::
         if (err) *err = smplgpu_last_error(m_ctx);
         return false;
     };
+    // where each query's BFS is seeded: the goal position, for a joint goal the target-offset position of its angles
+    // (ManipLattice::setGoalConfiguration), all joint goals in one device call
+    std::vector<double> goal_xyz((size_t)nq * 3);
+    {
+        std::vector<int> joint;
+        std::vector<double> angles;
+        for (int i = 0; i < nq; ++i) {
+            if (goals[i].type == SMPLGPU_GOAL_JOINT_STATE) {
+                joint.push_back(i);
+                angles.insert(angles.end(), goals[i].angles, goals[i].angles + dof);
+            } else {
+                std::copy(goals[i].pose, goals[i].pose + 3, goal_xyz.begin() + 3 * (size_t)i);
+            }
+        }
+        if (!joint.empty()) {
+            std::vector<double> pose6(joint.size() * 6);
+            if (smplgpu_planning_frame_fk(m_ctx, angles.data(), (int)joint.size(), pose6.data()) < 0) return fail_dev();
+            ++m_stats.device_calls;
+            for (size_t k = 0; k < joint.size(); ++k) {
+                std::copy(pose6.begin() + 6 * k, pose6.begin() + 6 * k + 3, goal_xyz.begin() + 3 * (size_t)joint[k]);
+            }
+        }
+    }
     const long long resolved0 = smplgpu_expand_batch_resolved(m_ctx);
     // a query creates at most (its expansions) x (successors per expansion) states besides the goal and the start
     const long long want_states = 2 + (long long)std::max(0, m_cfg.max_expansions) * std::max(1, m_stride);
@@ -648,7 +686,8 @@ bool BatchPlanner::plan(const double* starts, const double* goals, int nq, std::
         m_stats.device_calls += 2;
         // the valid starts become state 1 of a fresh lattice in their slot
         std::vector<int32_t> bslot, bgd;
-        std::vector<double> bq, bgoal;
+        std::vector<double> bq;
+        std::vector<smplgpu_goal> bgoal;
         for (int k = 0; k < nn; ++k) {
             Query& Q = S[pending[k]];
             const double* qs = &sq[(size_t)k * dof];
@@ -660,7 +699,7 @@ bool BatchPlanner::plan(const double* starts, const double* goals, int nq, std::
             bslot.push_back(pending[k]);
             bgd.push_back(sgd[k]);
             bq.insert(bq.end(), qs, qs + dof);
-            bgoal.insert(bgoal.end(), Q.goal, Q.goal + 3);
+            bgoal.push_back(*Q.goal);
             Q.num_states = 2;
             sstate(Q, 1);
             touch(Q, 1, sh[k]);
@@ -670,7 +709,7 @@ bool BatchPlanner::plan(const double* starts, const double* goals, int nq, std::
             heapPush(Q, 1);
         }
         if (!bslot.empty()) {
-            if (smplgpu_lattice_begin(m_ctx, bslot.data(), bq.data(), bgd.data(), bgoal.data(), (int)bslot.size()) < 0) return false;
+            if (smplgpu_lattice_begin_goals(m_ctx, bslot.data(), bq.data(), bgd.data(), bgoal.data(), (int)bslot.size()) < 0) return false;
             ++m_stats.device_calls;
         }
         {
@@ -703,12 +742,12 @@ bool BatchPlanner::plan(const double* starts, const double* goals, int nq, std::
                 if (occupied[s]) {
                     continue;
                 }
-                initQuery(S[s], next_query, s, goals + (size_t)next_query * 3);
+                initQuery(S[s], next_query, s, goals + next_query, &goal_xyz[3 * (size_t)next_query]);
                 ++next_query;
                 occupied[s] = 1;
                 pending.push_back(s);
                 int cell[3];
-                worldToGrid(S[s].goal, cell);
+                worldToGrid(S[s].goal_xyz, cell);
                 seeds.insert(seeds.end(), cell, cell + 3);
             }
             m_stats.host_seconds += t.lap();

@@ -92,8 +92,11 @@ class BatchPlanner
 public:
     BatchPlanner(smplgpu_ctx* ctx, const PlannerConfig& cfg, int max_concurrent);
 
-    /// starts: nq x dof, goals: nq x 3 (target-offset position in the planning frame)
+    /// starts: nq x dof, goals: nq x 3 (target-offset position in the planning frame); XYZ goals with
+    /// PlannerConfig::xyz_tolerance
     bool plan(const double* starts, const double* goals, int nq, std::vector<QueryResult>& out, std::string* err);
+    /// the same with one GoalConstraint per query (types may be mixed)
+    bool plan(const double* starts, const smplgpu_goal* goals, int nq, std::vector<QueryResult>& out, std::string* err);
 
     const BatchStats& stats() const { return m_stats; }
 
@@ -105,7 +108,8 @@ private:
     {
         int index;
         int slot;
-        double goal[3];
+        const smplgpu_goal* goal;
+        double goal_xyz[3];    // where the BFS is seeded: the goal position, for a joint goal that of its angles
         int goal_h;
         int num_states;        // lattice size on the device (ids handed out so far, goal and start included)
         std::vector<SState> search;
@@ -162,7 +166,7 @@ private:
     void percolateUp(Query& Q, size_t pivot);
     void percolateDown(Query& Q, size_t pivot);
     void finish(Query& Q, bool found);
-    void initQuery(Query& Q, int index, int slot, const double* goal);
+    void initQuery(Query& Q, int index, int slot, const smplgpu_goal* goal, const double* goal_xyz);
     void expandOne(Query& Q);   // pop the next state (no device work)
     void absorbOne(Query& Q, const int32_t* succ, const int32_t* h, int count);
     bool fetchPathStates(Query& Q, std::string* err);

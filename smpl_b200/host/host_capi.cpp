@@ -232,9 +232,9 @@ int smplhost_tables_pairs(smplhost_tables* h, int32_t* out, int max_pairs)
     return d->n_pairs;
 }
 
-int smplhost_plan_batch(smplgpu_ctx* ctx, const smplhost_plan_params* p, const double* starts,
-                        const double* goals, int nq, int max_concurrent, int32_t* summary, int32_t* path_ids,
-                        int max_path, double* stats, double* path_states)
+static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const double* starts,
+                          const smplgpu_goal* goals, int nq, int max_concurrent, int32_t* summary, int32_t* path_ids,
+                          int max_path, double* stats, double* path_states)
 {
     if (!ctx || !p || nq < 0 || (nq > 0 && (!starts || !goals || !summary))) {
         g_err = "smplhost_plan_batch: null argument";
@@ -310,17 +310,14 @@ int smplhost_plan_batch(smplgpu_ctx* ctx, const smplhost_plan_params* p, const d
     return 0;
 }
 
-int smplhost_plan_batch_multi(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p,
-                              const double* starts, const double* goals, int nq, int max_concurrent_per_ctx,
-                              int32_t* summary, int32_t* path_ids, int max_path, double* stats, double* path_states)
+// one planner thread per context, queries dealt round-robin
+static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
+                               const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
+                               int32_t* path_ids, int max_path, double* stats, double* path_states)
 {
-    if (!ctxs || n_ctx <= 0 || !p || nq < 0) {
-        g_err = "smplhost_plan_batch_multi: bad argument";
-        return SMPLGPU_ERR_INVALID;
-    }
     if (n_ctx == 1) {
-        return smplhost_plan_batch(ctxs[0], p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path, stats,
-                                   path_states);
+        return plan_batch_one(ctxs[0], p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path, stats,
+                              path_states);
     }
     const int dof = p->dof;
     std::vector<int> rc(n_ctx, 0);
@@ -341,19 +338,20 @@ int smplhost_plan_batch_multi(smplgpu_ctx* const* ctxs, int n_ctx, const smplhos
                 errs[t] = smplgpu_last_error(ctxs[t]);
                 return;
             }
-            std::vector<double> s((size_t)m * dof), g((size_t)m * 3);
+            std::vector<double> s((size_t)m * dof);
+            std::vector<smplgpu_goal> g(m);
             for (int k = 0; k < m; ++k) {
                 std::copy(starts + (size_t)mine[k] * dof, starts + (size_t)(mine[k] + 1) * dof, s.begin() + (size_t)k * dof);
-                std::copy(goals + (size_t)mine[k] * 3, goals + (size_t)(mine[k] + 1) * 3, g.begin() + (size_t)k * 3);
+                g[k] = goals[mine[k]];
             }
             std::vector<int32_t> sum((size_t)m * 5), paths(path_ids ? (size_t)m * max_path : 0);
             const size_t ps = (size_t)max_path * dof;
             std::vector<double> pstates(path_states ? (size_t)m * ps : 0);
             smplhost_plan_params pt = *p;
             pt.n_threads = 1;
-            rc[t] = smplhost_plan_batch(ctxs[t], &pt, s.data(), g.data(), m, max_concurrent_per_ctx, sum.data(),
-                                        path_ids ? paths.data() : nullptr, max_path, st[t].data(),
-                                        path_states ? pstates.data() : nullptr);
+            rc[t] = plan_batch_one(ctxs[t], &pt, s.data(), g.data(), m, max_concurrent_per_ctx, sum.data(),
+                                   path_ids ? paths.data() : nullptr, max_path, st[t].data(),
+                                   path_states ? pstates.data() : nullptr);
             if (rc[t] != 0) {
                 errs[t] = g_err;   // thread-local: copy it out
                 return;
@@ -388,6 +386,94 @@ int smplhost_plan_batch_multi(smplgpu_ctx* const* ctxs, int n_ctx, const smplhos
         }
     }
     return 0;
+}
+
+// XYZ goals with the parameters' tolerance
+static std::vector<smplgpu_goal> xyz_goals(const smplhost_plan_params* p, const double* goals_xyz, int nq)
+{
+    std::vector<smplgpu_goal> recs(nq > 0 && goals_xyz ? nq : 0);   // zero-filled
+    for (size_t i = 0; i < recs.size(); ++i) {
+        recs[i].type = SMPLGPU_GOAL_XYZ;
+        for (int a = 0; a < 3; ++a) {
+            recs[i].pose[a] = goals_xyz[3 * i + a];
+            recs[i].xyz_tolerance[a] = p->xyz_tolerance[a];
+        }
+    }
+    return recs;
+}
+
+int smplhost_plan_batch(smplgpu_ctx* ctx, const smplhost_plan_params* p, const double* starts,
+                        const double* goals, int nq, int max_concurrent, int32_t* summary, int32_t* path_ids,
+                        int max_path, double* stats, double* path_states)
+{
+    if (!ctx || !p || nq < 0 || (nq > 0 && (!starts || !goals || !summary))) {
+        g_err = "smplhost_plan_batch: null argument";
+        return SMPLGPU_ERR_INVALID;
+    }
+    const std::vector<smplgpu_goal> recs = xyz_goals(p, goals, nq);
+    return plan_batch_one(ctx, p, starts, recs.data(), nq, max_concurrent, summary, path_ids, max_path, stats, path_states);
+}
+
+int smplhost_plan_batch_multi(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p,
+                              const double* starts, const double* goals, int nq, int max_concurrent_per_ctx,
+                              int32_t* summary, int32_t* path_ids, int max_path, double* stats, double* path_states)
+{
+    if (!ctxs || n_ctx <= 0 || !p || nq < 0) {
+        g_err = "smplhost_plan_batch_multi: bad argument";
+        return SMPLGPU_ERR_INVALID;
+    }
+    if (nq > 0 && !goals) {
+        g_err = "smplhost_plan_batch: null argument";
+        return SMPLGPU_ERR_INVALID;
+    }
+    const std::vector<smplgpu_goal> recs = xyz_goals(p, goals, nq);
+    return plan_batch_contexts(ctxs, n_ctx, p, starts, recs.data(), nq, max_concurrent_per_ctx, summary, path_ids,
+                               max_path, stats, path_states);
+}
+
+static bool bad_tolerance(double t)
+{
+    return std::isnan(t) || t < 0.0;
+}
+
+int smplhost_plan_batch_goals(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
+                              const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
+                              int32_t* path_ids, int max_path, double* stats, double* path_states)
+{
+    if (!ctxs || n_ctx <= 0 || !p || nq < 0 || (nq > 0 && !goals)) {
+        g_err = "smplhost_plan_batch_goals: bad argument";
+        return SMPLGPU_ERR_INVALID;
+    }
+    for (int t = 0; t < n_ctx; ++t) {
+        if (!ctxs[t]) {
+            g_err = "smplhost_plan_batch_goals: null context";
+            return SMPLGPU_ERR_INVALID;
+        }
+    }
+    if (p->dof <= 0 || p->dof > SMPLGPU_MAX_DOF) {
+        g_err = "smplhost_plan_batch_goals: dof out of range";
+        return SMPLGPU_ERR_INVALID;
+    }
+    // the checks of smplgpu_lattice_begin_goals, before any query starts
+    for (int i = 0; i < nq; ++i) {
+        const smplgpu_goal& g = goals[i];
+        bool ok = true;
+        if (g.type == SMPLGPU_GOAL_XYZ || g.type == SMPLGPU_GOAL_XYZ_RPY) {
+            for (int a = 0; a < 3; ++a) ok = ok && !bad_tolerance(g.xyz_tolerance[a]);
+            ok = ok && (g.type == SMPLGPU_GOAL_XYZ || !bad_tolerance(g.rpy_tolerance));
+        } else if (g.type == SMPLGPU_GOAL_JOINT_STATE) {
+            for (int v = 0; v < p->dof; ++v) ok = ok && !bad_tolerance(g.angle_tolerances[v]);
+        } else {
+            g_err = "smplhost_plan_batch_goals: goal " + std::to_string(i) + " has unknown type " + std::to_string(g.type);
+            return SMPLGPU_ERR_INVALID;
+        }
+        if (!ok) {
+            g_err = "smplhost_plan_batch_goals: goal " + std::to_string(i) + " has a NaN or negative tolerance";
+            return SMPLGPU_ERR_INVALID;
+        }
+    }
+    return plan_batch_contexts(ctxs, n_ctx, p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path,
+                               stats, path_states);
 }
 
 struct smplhost_adapters

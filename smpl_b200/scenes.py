@@ -352,6 +352,25 @@ def ubr1_tabletop_queries(n, seed=13):
     return np.ascontiguousarray(starts), np.ascontiguousarray(goals)
 
 
+def lattice_walks(starts, params, k, seed, valid):
+    """Joint states a planner can reach: walker i starts at starts[i] and takes k random motion-primitive steps
+    (converses included) that valid(q0, q1) -> bool[n] accepts (joint limits and edge validity of the checker in use);
+    a walker that finds no valid step in 8 tries stays where it is for that step.  Goals built from these states
+    (their pose, or their joint values) are reachable by construction."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    prims = np.asarray(params.mprims, np.float64)
+    deltas = np.stack([prims, -prims], axis=1).reshape(-1, prims.shape[1])
+    q = np.array(starts, np.float64).reshape(-1, prims.shape[1])
+    for _ in range(k):
+        moved = np.zeros(len(q), bool)
+        for _ in range(8):
+            q1 = q + deltas[rng.integers(len(deltas), size=len(q))]
+            ok = ~moved & np.asarray(valid(q, q1), bool)
+            q[ok] = q1[ok]
+            moved |= ok
+    return np.ascontiguousarray(q)
+
+
 def lattice_discretisation(lo, hi, cont, resolutions):
     """ManipLattice::init (manip_lattice.cpp:125-139): (coord_vals, coord_deltas, base) per planning variable."""
     vals, deltas, base = [], [], []
