@@ -446,6 +446,40 @@ int smplgpu_lattice_expand_wait(smplgpu_ctx* ctx, int buffer, const int32_t** su
 /* joint values of lattice states (ManipLattice::extractPath): q_out[i] = state id[i] of slot[i] */
 int smplgpu_lattice_states(smplgpu_ctx* ctx, const int32_t* slot, const int32_t* id, int n, double* q_out);
 
+/* ---- planning-link IK and the snap-to-goal action ---- */
+/* The IK of the planning link: the batched counterpart of InverseKinematicsInterface::computeIK with
+ * ik_option::UNRESTRICTED.  The reference's solvers are third-party, so this IK is the project's own (DESIGN.md
+ * section 2): damped least squares from the seed, q += J^T (J J^T + 1e-6 I)^-1 e, where e is the target-offset position
+ * error and the rotation vector of R_goal R^T, J the planning link's geometric Jacobian at the target point (of
+ * smplgpu_planning_frame_fk's chain); bounded variables are clamped to their limits, continuous ones wrapped.  A
+ * problem converges when every |e_i| <= tolerance (metres / radians), within max_iterations steps. */
+typedef struct smplgpu_ik_params {
+    int32_t max_iterations;   /* >= 1; 100 by default */
+    double  tolerance;        /* > 0; 1e-6 by default */
+} smplgpu_ik_params;
+/* n problems: pose6[n][6] goal poses (x y z roll pitch yaw of the target-offset frame, as smplgpu_planning_frame_fk
+ * reports them), seeds[n][dof]; q_out[n][dof], ok[n] (1 = converged), iterations[n] (steps taken).  Returns the number
+ * that converged; bad parameters are SMPLGPU_ERR_INVALID. */
+int smplgpu_planning_link_ik(smplgpu_ctx* ctx, const double* pose6, const double* seeds, int n,
+                             const smplgpu_ik_params* params, double* q_out, uint8_t* ok, int32_t* iterations);
+/* The SNAP_TO_XYZ_RPY action of ManipLatticeActionSpace (manip_lattice_action_space.cpp:376-449, 507-573, 662-691):
+ * when the expanded state's metric goal distance (BFS cells * resolution, the quantity of the short-distance switch)
+ * is <= dist_thresh, its first successor is an IK solution for the goal pose (XYZ and XYZ_RPY goals; the full pose of
+ * the record, seeded at the expanded state) or the goal's angles (JOINT_STATE goals), checked like any action.  Call
+ * after smplgpu_lattice_create (which turns snaps off) and before the queries begin.  With snaps enabled, successor
+ * word 0 of every expansion is the snap's (-1 when inactive, failed or invalid) and words 1 .. are the primitives'
+ * (SMPLGPU_LATTICE_SHORT_FLAG keeps its meaning for them); the rounds run as a chain of kernels (SMPLGPU_LATTICE_FUSED
+ * has no snap form).  Returns the stride, 1 + the primitives' (the primitives' alone when disabled);
+ * SMPLGPU_ERR_LIMIT above the stride limit, SMPLGPU_ERR_INVALID for a NaN or negative threshold or bad IK parameters. */
+typedef struct smplgpu_snap_params {
+    int32_t enabled;
+    double  dist_thresh;      /* metres */
+    smplgpu_ik_params ik;
+} smplgpu_snap_params;
+int smplgpu_lattice_set_snap(smplgpu_ctx* ctx, const smplgpu_snap_params* params);
+/* IK solves the snap actions of this context's rounds ran so far, and how many converged (running totals) */
+int smplgpu_lattice_snap_counters(smplgpu_ctx* ctx, int64_t counters[2]);
+
 /* ---- lattice states on the wire as 16-bit coordinates ---- */
 /* The real caller of the validity path, ManipLattice, holds a state as dof small integers (RobotCoord) and forms the
  * joint values with coordToState (manip_lattice.cpp:1245-1261).  These entry points take the coordinates and do

@@ -117,6 +117,24 @@ int smplhost_plan_batch_goals(smplgpu_ctx* const* ctxs, int n_ctx, const smplhos
                               const double* starts, const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx,
                               int32_t* summary, int32_t* path_ids, int max_path, double* stats, double* path_states);
 
+/* The snap-to-goal action (SNAP_TO_XYZ_RPY, smplgpu_lattice_set_snap) in the batched planner: an expansion within
+ * dist_thresh metres of metric goal distance first tries to jump straight to the goal -- to an IK solution for a pose
+ * goal, to the angles of a joint goal -- at a cost of (int)(1000 * weight) (the reference registers it with weight
+ * 0.5).  enabled = 0 plans as without it. */
+typedef struct smplhost_snap_params {
+    int32_t enabled;
+    double  dist_thresh;        /* metres, >= 0 */
+    double  weight;             /* >= 0 */
+    smplgpu_ik_params ik;       /* max_iterations >= 1, tolerance > 0 */
+} smplhost_snap_params;
+/* smplhost_plan_batch_goals with the snap action.  counters[2] (nullable): IK solves the snaps ran, and how many
+ * converged (summed over the contexts).  Bad goal records or snap parameters are SMPLGPU_ERR_INVALID before anything
+ * is planned. */
+int smplhost_plan_batch_snap(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* params,
+                             const double* starts, const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx,
+                             int32_t* summary, int32_t* path_ids, int max_path, double* stats, double* path_states,
+                             const smplhost_snap_params* snap, int64_t* counters);
+
 /* ---- drop-in adapters (smpl_b200/host/gpu_adapters.h): the reference's CollisionChecker / RobotModel /
  * RobotHeuristic virtuals implemented over the C ABI.  These shims drive the C++ objects one virtual call at
  * a time, the way the reference's planner does (n = 1 per call); a C++ caller uses the classes directly. ---- */

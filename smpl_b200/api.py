@@ -98,6 +98,33 @@ class PlanParamsC(C.Structure):
                 ("res", C.c_double), ("dims", C.c_int * 3), ("n_threads", C.c_int), ("prim_weights", c_double_p)]
 
 
+class IkParamsC(C.Structure):
+    """smplgpu_ik_params (include/smplgpu.h)."""
+    _fields_ = [("max_iterations", C.c_int32), ("tolerance", C.c_double)]
+
+
+class SnapParamsC(C.Structure):
+    """smplhost_snap_params (include/smplhost.h)."""
+    _fields_ = [("enabled", C.c_int32), ("dist_thresh", C.c_double), ("weight", C.c_double), ("ik", IkParamsC)]
+
+
+class SnapParams:
+    """The snap-to-goal action of the batched planner (smplhost_snap_params): an expansion whose metric goal distance
+    is within dist_thresh metres first tries to jump straight to the goal -- to an IK solution for a pose goal, to the
+    angles of a joint goal -- at a cost of int(1000 * weight).  dist_thresh = 0.0 is the reference demo's setting."""
+
+    def __init__(self, enabled=True, dist_thresh=0.0, weight=0.5, max_iterations=100, tolerance=1e-6):
+        self.enabled = enabled
+        self.dist_thresh = dist_thresh
+        self.weight = weight
+        self.max_iterations = max_iterations
+        self.tolerance = tolerance
+
+    def c(self):
+        return SnapParamsC(int(bool(self.enabled)), float(self.dist_thresh), float(self.weight),
+                           IkParamsC(int(self.max_iterations), float(self.tolerance)))
+
+
 def gpu_lib():
     """libsmplgpu.so; raises when it has not been built (no fallback)."""
     global _gpu
@@ -143,6 +170,7 @@ def gpu_lib():
         L.smplgpu_goal_heuristics.argtypes = [vp, dp, i, i, ip]
         L.smplgpu_goal_heuristics_dev.argtypes = [vp, vp, i, i, vp]
         L.smplgpu_planning_frame_fk.argtypes = [vp, dp, i, dp]
+        L.smplgpu_planning_link_ik.argtypes = [vp, dp, dp, i, C.POINTER(IkParamsC), dp, bp, ip]
         L.smplgpu_is_mprim_edges_valid.argtypes = [vp, dp, ip, i, dp, i, bp, ip]
         L.smplgpu_is_indexed_edges_valid.argtypes = [vp, dp, i, ip, ip, i, bp, ip]
         L.smplgpu_set_precision_mode.argtypes = [vp, i]
@@ -209,6 +237,9 @@ def host_lib():
         H.smplhost_plan_batch_goals.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PlanParamsC), c_double_p,
                                                 C.POINTER(GoalC), C.c_int, C.c_int, c_int32_p, c_int32_p, C.c_int,
                                                 c_double_p, c_double_p]
+        H.smplhost_plan_batch_snap.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PlanParamsC), c_double_p,
+                                               C.POINTER(GoalC), C.c_int, C.c_int, c_int32_p, c_int32_p, C.c_int,
+                                               c_double_p, c_double_p, C.POINTER(SnapParamsC), C.POINTER(C.c_int64)]
         H.smplhost_shortcut_paths.argtypes = [vp, C.c_int, c_uint8_p, c_double_p, c_int32_p, C.c_int, C.c_int, c_int32_p,
                                               c_int32_p, c_double_p]
         H.smplhost_interpolate_paths.argtypes = [vp, vp, c_double_p, c_int32_p, C.c_int, c_double_p, C.c_int, c_int32_p,
@@ -616,6 +647,22 @@ class GpuContext:
         self._ck(self.L.smplgpu_planning_frame_fk(self.h, _dp(q), len(q), _dp(out)), "planning_frame_fk")
         return out
 
+    def planning_link_ik(self, poses, seeds, max_iterations=100, tolerance=1e-6):
+        """smplgpu_planning_link_ik: the planning link's IK for target-offset poses (n, 6) x y z roll pitch yaw,
+        seeded at seeds (n, dof).  Returns (q (n, dof), ok (n,) bool, iterations (n,))."""
+        poses = np.ascontiguousarray(poses, dtype=np.float64).reshape(-1, 6)
+        seeds = self._q(seeds)
+        if len(seeds) != len(poses):
+            raise ValueError("%d poses, %d seeds" % (len(poses), len(seeds)))
+        n = len(poses)
+        q = np.zeros_like(seeds)
+        ok = np.zeros(n, np.uint8)
+        it = np.zeros(n, np.int32)
+        prm = IkParamsC(int(max_iterations), float(tolerance))
+        self._ck(self.L.smplgpu_planning_link_ik(self.h, _dp(poses), _dp(seeds), n, C.byref(prm), _dp(q), _bp(ok),
+                                                 _ip(it)), "planning_link_ik")
+        return q, ok.astype(bool), it
+
 
     # ---- many queries at once ----
     def bfs_bank_create(self, n_slots, inflation_radius):
@@ -814,17 +861,22 @@ def clone_context(ctx, scene, tables, device=0):
 
 
 def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max_path=512, n_threads=1,
-               want_states=False):
+               want_states=False, snap=None):
     """smplhost_plan_batch: many ARA* queries in lock step, one device call per round.
     params: smpl_b200.scenes.PlanParams.  Returns (list of dict per query, stats dict).
     goals: (nq, 3) positions (XYZ goals with params.xyz_tolerance), or goal records of GOAL_DTYPE (pose_goals,
     joint_goals; types may be mixed), which go through smplhost_plan_batch_goals.
     `ctx` may be a list of contexts (same GPU, same scene): one planner thread per context
-    (smplhost_plan_batch_multi), max_concurrent is then per context."""
+    (smplhost_plan_batch_multi), max_concurrent is then per context.
+    snap: SnapParams -- the snap-to-goal action, through smplhost_plan_batch_snap (position goals become XYZ goal
+    records); the stats then also hold ik_attempted / ik_converged."""
     H = host_lib()
     dof = tables.dof
     starts = np.ascontiguousarray(starts, dtype=np.float64).reshape(-1, dof)
     records = isinstance(goals, np.ndarray) and goals.dtype == GOAL_DTYPE
+    if snap is not None and not records:
+        goals = pose_goals(np.asarray(goals, np.float64).reshape(-1, 3), params.xyz_tolerance)
+        records = True
     if records:
         goals = np.ascontiguousarray(goals.reshape(-1))
     else:
@@ -859,7 +911,15 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
     stats = np.zeros(12)
     pstates = np.zeros((nq, max_path, dof), np.float64) if want_states else None
     ps_ptr = _dp(pstates) if want_states else None
-    if records:
+    counters = np.zeros(2, np.int64)
+    if snap is not None:
+        ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
+        arr = (C.c_void_p * len(ctxs))(*[c.h for c in ctxs])
+        sp = snap.c()
+        r = H.smplhost_plan_batch_snap(arr, len(ctxs), C.byref(P), _dp(starts), goals.ctypes.data_as(C.POINTER(GoalC)), nq,
+                                       int(max_concurrent), _ip(summary), _ip(paths), int(max_path), _dp(stats), ps_ptr,
+                                       C.byref(sp), counters.ctypes.data_as(C.POINTER(C.c_int64)))
+    elif records:
         ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
         arr = (C.c_void_p * len(ctxs))(*[c.h for c in ctxs])
         r = H.smplhost_plan_batch_goals(arr, len(ctxs), C.byref(P), _dp(starts), goals.ctypes.data_as(C.POINTER(GoalC)), nq,
@@ -884,6 +944,8 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
               device_seconds=float(stats[3]), host_seconds=float(stats[4]), total_seconds=float(stats[5]),
               bfs_runs=int(stats[6]), edges_resolved_f64=int(stats[7]), setup_seconds=float(stats[8]),
               max_wait_seconds=float(stats[9]), n_threads=int(n_threads))
+    if snap is not None:
+        st.update(ik_attempted=int(counters[0]), ik_converged=int(counters[1]))
     return out, st
 
 

@@ -53,6 +53,39 @@ __device__ __forceinline__ void rot2(const double* v, double angle, double* M)
     M[6] = -m_st_1 + m_vt_0_2;  M[7] = m_st_0 + m_vt_1_2;   M[8] = ct + m_vt_2 * v[2];
 }
 
+// Segment::pose(q) = joint.pose(q) * f_tip of chain segment s: one factor of the planning-link chain (also the
+// per-lane part of the IK's chain, ik.cuh)
+__device__ __forceinline__ void segment_pose(const DevModel* __restrict__ M, int s, const double* __restrict__ q, KFrame& seg)
+{
+    const int v = M->seg_var[s];
+    double qq = 0.0;
+    if (v >= 0) {
+        qq = q[v];
+        if (M->var_type[v] == 1) {
+            qq = normalize_angle(qq); // KDLRobotModel::normalizeAngles (continuous joints only)
+        }
+    }
+    KFrame jp;
+    const int kind = M->seg_kind[s];
+    if (kind == 1) {
+        rot2(M->seg_axis[s], qq, jp.M);
+        jp.p[0] = M->seg_origin[s][0]; jp.p[1] = M->seg_origin[s][1]; jp.p[2] = M->seg_origin[s][2];
+    } else {
+#pragma unroll
+        for (int i = 0; i < 9; ++i) jp.M[i] = (i % 4 == 0) ? 1.0 : 0.0;
+        if (kind == 2) {
+            jp.p[0] = M->seg_origin[s][0] + M->seg_axis[s][0] * qq;
+            jp.p[1] = M->seg_origin[s][1] + M->seg_axis[s][1] * qq;
+            jp.p[2] = M->seg_origin[s][2] + M->seg_axis[s][2] * qq;
+        } else {
+            jp.p[0] = jp.p[1] = jp.p[2] = 0.0;
+        }
+    }
+    KFrame tip;
+    kframe_from12(M->seg_f_tip[s], tip);
+    kframe_mul(jp, tip, seg);
+}
+
 // computePlanningLinkFK + getTargetOffsetPose: pose6 = x y z roll pitch yaw of the target-offset
 // frame; link_xyz (optional) = position of the planning link itself (before the offset)
 __device__ void planning_frame_fk(const DevModel* __restrict__ M, const double* __restrict__ q, double* pose,
@@ -64,33 +97,8 @@ __device__ void planning_frame_fk(const DevModel* __restrict__ M, const double* 
     f1.p[0] = f1.p[1] = f1.p[2] = 0.0;
 
     for (int s = 0; s < M->n_segments; ++s) {
-        const int v = M->seg_var[s];
-        double qq = 0.0;
-        if (v >= 0) {
-            qq = q[v];
-            if (M->var_type[v] == 1) {
-                qq = normalize_angle(qq); // KDLRobotModel::normalizeAngles (continuous joints only)
-            }
-        }
-        KFrame jp;
-        const int kind = M->seg_kind[s];
-        if (kind == 1) {
-            rot2(M->seg_axis[s], qq, jp.M);
-            jp.p[0] = M->seg_origin[s][0]; jp.p[1] = M->seg_origin[s][1]; jp.p[2] = M->seg_origin[s][2];
-        } else {
-#pragma unroll
-            for (int i = 0; i < 9; ++i) jp.M[i] = (i % 4 == 0) ? 1.0 : 0.0;
-            if (kind == 2) {
-                jp.p[0] = M->seg_origin[s][0] + M->seg_axis[s][0] * qq;
-                jp.p[1] = M->seg_origin[s][1] + M->seg_axis[s][1] * qq;
-                jp.p[2] = M->seg_origin[s][2] + M->seg_axis[s][2] * qq;
-            } else {
-                jp.p[0] = jp.p[1] = jp.p[2] = 0.0;
-            }
-        }
-        KFrame tip, seg, nf;
-        kframe_from12(M->seg_f_tip[s], tip);
-        kframe_mul(jp, tip, seg);
+        KFrame seg, nf;
+        segment_pose(M, s, q, seg);
         kframe_mul(f1, seg, nf);
         f1 = nf;
     }

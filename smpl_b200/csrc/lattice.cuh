@@ -28,13 +28,15 @@ constexpr int LATTICE_MAX_STRIDE = 32;        // successors per expansion: one l
 constexpr int LATTICE_GOAL_FLAG = 1 << 30;    // in a successor word: the action reaches the goal region
 constexpr int LATTICE_SHORT_FLAG = 1 << 29;   // in a count word: the expansion used the short-distance primitives
 
-// The goal of one query (smplgpu_goal, as the device reads it).  qg is the goal orientation's quaternion x y z w,
-// computed on the host (smplgpu_lattice_begin_goals) so that only the state's quaternion rounds the device's way.
+// The goal of one query (smplgpu_goal, as the device reads it).  qg is the goal orientation's quaternion x y z w and R
+// its rotation matrix (the snap action's IK target), both computed on the host (smplgpu_lattice_begin_goals) so that
+// only the state's quaternion rounds the device's way.
 struct LatticeGoal
 {
     int type;                 // SMPLGPU_GOAL_*
     double xyz[3], xyz_tol[3];
     double qg[4];
+    double R[9];
     double rpy_tol;
     double angles[MAX_DOF], angle_tol[MAX_DOF];
 };
@@ -42,7 +44,7 @@ struct LatticeGoal
 struct LatticeBank
 {
     int n_slots, cap, table_size;             // states per slot, hash slots per slot (power of two)
-    int stride;                               // successor words per expansion = max(#long, #short primitives)
+    int stride;                               // successor words per expansion = snap + max(#long, #short primitives)
     int n_long, n_short;
     int use_short_dist;
     double short_dist_thresh, res;
@@ -56,6 +58,12 @@ struct LatticeBank
     const double* deltas;     // [n_prims][dof]
     const int* long_list;     // primitive indices in table order
     const int* short_list;
+    // the snap action (smplgpu_lattice_set_snap): snap = 1 makes word 0 of every expansion the snap, words 1.. the
+    // primitives; 0 = no snap word
+    int snap;
+    double snap_thresh;
+    int ik_max_iterations;
+    double ik_tolerance;
 };
 
 // ManipLattice::stateToCoord (manip_lattice.cpp:1263-1289; every KDL planning variable is continuous or bounded)
@@ -172,7 +180,8 @@ __device__ __forceinline__ bool lattice_is_goal(int dof, const LatticeGoal* __re
     return normalize_angle(2.0 * acos(d)) < g->rpy_tol;
 }
 
-// Round, step 1: the edges of every expansion.  Thread (i, j): j-th active primitive of the state expansion i pops.
+// Round, step 1: the edges of every expansion.  Thread (i, j): j-th active primitive of the state expansion i pops
+// (with snaps enabled word 0 is the snap's, which lattice_snap_kernel fills in, and word j the (j-1)-th primitive).
 // Inactive positions and successors beyond a joint limit become zero-length edges (no waypoint, no work in the
 // edge kernels) and are flagged.
 __global__ void lattice_gen_kernel(const DevModel* __restrict__ M, LatticeBank B, const int* __restrict__ slot,
@@ -195,9 +204,10 @@ __global__ void lattice_gen_kernel(const DevModel* __restrict__ M, LatticeBank B
     const bool near_goal = B.use_short_dist && goal_dist <= B.short_dist_thresh;
     const int cnt = near_goal ? B.n_short : B.n_long;
     double succ[MAX_DOF];
-    bool on = j < cnt;
+    const int w = j - B.snap;
+    bool on = w >= 0 && w < cnt;
     if (on) {
-        const int prim = near_goal ? B.short_list[j] : B.long_list[j];
+        const int prim = near_goal ? B.short_list[w] : B.long_list[w];
         for (int v = 0; v < dof; ++v) {
             succ[v] = B.deltas[(size_t)prim * dof + v] + a[v];
         }

@@ -27,6 +27,7 @@
 #include "validity_warp.cuh"
 #include "expand1.cuh"
 #include "lattice.cuh"
+#include "ik.cuh"
 
 using namespace smplgpu;
 
@@ -148,6 +149,8 @@ struct smplgpu_ctx
     int lat_dof = 0;                               // dof the lattice arrays were sized for
     unsigned long long* lat_resolved = nullptr;   // pinned, mapped: edges the rounds resolved in double (running total)
     bool lat_fused = false;                        // one kernel per round (lattice_round_kernel)
+    int lat_prim_stride = 0;                       // successor words of the primitives (smplgpu_lattice_create)
+    unsigned long long* d_snap_counters = nullptr; // IK solves of the snap actions: run, converged
     size_t lat_round_smem = 0;
     // smplgpu_expand_state: primitive table, page-locked record array + completion flag, arrival counter
     double* d_x1_deltas = nullptr; int x1_prims = -1; int x1_dof = 0;
@@ -397,6 +400,7 @@ void smplgpu_destroy(smplgpu_ctx* ctx)
     free_bfs(ctx);
     free_grid(ctx->bank);
     free_tiles(ctx->bank_tiles);
+    cudaFree(ctx->d_snap_counters);
     cudaFree(ctx->d_model); cudaFree(ctx->d_stats); cudaFree(ctx->d_seed_count); cudaFree(ctx->d_df);
     cudaFree(ctx->d_blob); cudaFree(ctx->d_unc_list); cudaFree(ctx->d_unc_mask); cudaFree(ctx->d_unc_count);
     cudaFree(ctx->d_prim); cudaFree(ctx->d_deltas);
@@ -3076,6 +3080,38 @@ int smplgpu_lattice_max_slots(smplgpu_ctx* ctx, int max_states)
     return (int)std::max<size_t>(1, std::min<size_t>((size_t)(0.4 * (double)have) / per, (size_t)1 << 20));
 }
 
+// round buffers for up to one expansion per slot (lat_max_n) of lat.stride words: every allocation happens here,
+// not while planners run
+static int lattice_round_buffers(smplgpu_ctx* ctx)
+{
+    const int dof = ctx->h_model->dof;
+    const int max_n = ctx->lat_max_n;
+    const size_t ne = (size_t)max_n * ctx->lat.stride;
+    int r;
+    for (int b = 0; b < SMPLGPU_EXPAND_BUFFERS; ++b) {
+        const size_t in_bytes = 2 * (size_t)max_n * sizeof(int) + 64;
+        const size_t out_bytes = (2 * ne + (size_t)max_n + 2) * sizeof(int) + 64;   // succ | h | count | resolved (8 B)
+        const size_t dev_bytes = 2 * ne * dof * sizeof(double) + 2 * ((ne + 63) / 64 * 64) + 256;
+        if (in_bytes > ctx->lat_in_cap[b]) {
+            if (ctx->lat_in[b]) { CU(cudaFreeHost(ctx->lat_in[b])); ctx->lat_in[b] = nullptr; ctx->lat_in_cap[b] = 0; }
+            CU(cudaHostAlloc(&ctx->lat_in[b], in_bytes, cudaHostAllocMapped));
+            ctx->lat_in_cap[b] = in_bytes;
+        }
+        if (out_bytes > ctx->lat_out_cap[b]) {
+            if (ctx->lat_out[b]) { CU(cudaFreeHost(ctx->lat_out[b])); ctx->lat_out[b] = nullptr; ctx->lat_out_cap[b] = 0; }
+            CU(cudaHostAlloc(&ctx->lat_out[b], out_bytes, cudaHostAllocMapped));
+            ctx->lat_out_cap[b] = out_bytes;
+        }
+        if ((r = grow(ctx, &ctx->d_lat[b], &ctx->d_lat_cap[b], dev_bytes))) return r;
+    }
+    if ((r = ensure_unc(ctx, ne))) return r;
+    if (!ctx->lat_resolved) {
+        CU(cudaHostAlloc((void**)&ctx->lat_resolved, 64, cudaHostAllocMapped));
+        *ctx->lat_resolved = 0;
+    }
+    return 0;
+}
+
 int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, int n_slots)
 {
     if (!ctx || !p || n_slots <= 0) return SMPLGPU_ERR_INVALID;
@@ -3099,13 +3135,13 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
     CU(cudaStreamSynchronize(ctx->stream));
     const int cap = p->max_states;
     const int tsize = lattice_table_size(cap);
-    const bool same_shape = ctx->has_lat && ctx->lat.n_slots == n_slots && ctx->lat.cap == cap && ctx->lat.stride == stride &&
+    const bool same_shape = ctx->has_lat && ctx->lat.n_slots == n_slots && ctx->lat.cap == cap && ctx->lat_prim_stride == stride &&
                             ctx->lat_dof == dof;
     if (!same_shape) {
         // the lattices are a scene-level allocation (gigabytes for thousands of queries): kept across calls
         free_lattice(ctx);
         LatticeBank& B = ctx->lat;
-        B.n_slots = n_slots; B.cap = cap; B.table_size = tsize; B.stride = stride;
+        B.n_slots = n_slots; B.cap = cap; B.table_size = tsize;
         ctx->lat_dof = dof;
         CU(cudaMalloc(&B.q, (size_t)n_slots * cap * dof * sizeof(double)));
         CU(cudaMalloc(&B.coord, (size_t)n_slots * cap * dof * sizeof(int)));
@@ -3116,6 +3152,9 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
         CU(cudaMemset(B.count, 0, (size_t)n_slots * sizeof(int)));
     }
     LatticeBank& B = ctx->lat;
+    B.stride = stride;
+    ctx->lat_prim_stride = stride;
+    B.snap = 0;   // smplgpu_lattice_set_snap turns them on
     B.n_long = (int)long_list.size();
     B.n_short = (int)short_list.size();
     B.use_short_dist = p->use_short_dist ? 1 : 0;
@@ -3138,30 +3177,8 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
     B.short_list = (const int*)(aux + db + lb);
     ctx->lat_params = ctx->lattice;
     for (int v = 0; v < MAX_DOF; ++v) ctx->lat_vals.v[v] = ctx->lattice_vals[v];
-    // round buffers for up to one expansion per slot: every allocation happens here, not while planners run
-    const int max_n = n_slots;
-    const size_t ne = (size_t)max_n * stride;
-    for (int b = 0; b < SMPLGPU_EXPAND_BUFFERS; ++b) {
-        const size_t in_bytes = 2 * (size_t)max_n * sizeof(int) + 64;
-        const size_t out_bytes = (2 * ne + (size_t)max_n + 2) * sizeof(int) + 64;   // succ | h | count | resolved (8 B)
-        const size_t dev_bytes = 2 * ne * dof * sizeof(double) + 2 * ((ne + 63) / 64 * 64) + 256;
-        if (in_bytes > ctx->lat_in_cap[b]) {
-            if (ctx->lat_in[b]) { CU(cudaFreeHost(ctx->lat_in[b])); ctx->lat_in[b] = nullptr; ctx->lat_in_cap[b] = 0; }
-            CU(cudaHostAlloc(&ctx->lat_in[b], in_bytes, cudaHostAllocMapped));
-            ctx->lat_in_cap[b] = in_bytes;
-        }
-        if (out_bytes > ctx->lat_out_cap[b]) {
-            if (ctx->lat_out[b]) { CU(cudaFreeHost(ctx->lat_out[b])); ctx->lat_out[b] = nullptr; ctx->lat_out_cap[b] = 0; }
-            CU(cudaHostAlloc(&ctx->lat_out[b], out_bytes, cudaHostAllocMapped));
-            ctx->lat_out_cap[b] = out_bytes;
-        }
-        if ((r = grow(ctx, &ctx->d_lat[b], &ctx->d_lat_cap[b], dev_bytes))) return r;
-    }
-    if ((r = ensure_unc(ctx, ne))) return r;
-    if (!ctx->lat_resolved) {
-        CU(cudaHostAlloc((void**)&ctx->lat_resolved, 64, cudaHostAllocMapped));
-        *ctx->lat_resolved = 0;
-    }
+    ctx->lat_max_n = n_slots;
+    if ((r = lattice_round_buffers(ctx))) return r;
     // SMPLGPU_LATTICE_FUSED=1: one kernel per round (lattice_round_kernel; measured slower at the default number of
     // planner contexts, see lattice.cuh) when the single-precision model is in use and a block's shared memory holds
     // the blob, the per-thread f32 state and one warp's double-precision slots
@@ -3179,7 +3196,6 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
             CU(cudaFuncSetAttribute(lattice_round_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)1024)));
         }
     }
-    ctx->lat_max_n = max_n;
     ctx->has_lat = true;
     return stride;
 }
@@ -3207,6 +3223,18 @@ static void quat_from_rpy(double roll, double pitch, double yaw, double* q)
 static bool bad_tolerance(double t)
 {
     return std::isnan(t) || t < 0.0;
+}
+
+// KDL Rotation::RPY(roll, pitch, yaw) = Rz(yaw) Ry(pitch) Rx(roll), row-major: the IK's goal rotation, with the host's
+// libm and the expression of the oracle (oracle/snap/snap_lattice.cpp rpyMatrix)
+static void rpy_matrix(double roll, double pitch, double yaw, double* R)
+{
+    const double ca1 = std::cos(yaw), sa1 = std::sin(yaw);
+    const double cb1 = std::cos(pitch), sb1 = std::sin(pitch);
+    const double cc1 = std::cos(roll), sc1 = std::sin(roll);
+    R[0] = ca1 * cb1;  R[1] = ca1 * sb1 * sc1 - sa1 * cc1;  R[2] = ca1 * sb1 * cc1 + sa1 * sc1;
+    R[3] = sa1 * cb1;  R[4] = sa1 * sb1 * sc1 + ca1 * cc1;  R[5] = sa1 * sb1 * cc1 - ca1 * sc1;
+    R[6] = -sb1;       R[7] = cb1 * sc1;                    R[8] = cb1 * cc1;
 }
 
 static int lattice_begin_records(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
@@ -3262,6 +3290,7 @@ int smplgpu_lattice_begin(smplgpu_ctx* ctx, const int32_t* slots, const double* 
             g.xyz[a] = goals_xyz[3 * i + a];
             g.xyz_tol[a] = ctx->lat_xyz_tol[a];
         }
+        rpy_matrix(0.0, 0.0, 0.0, g.R);
     }
     return lattice_begin_records(ctx, slots, starts, start_gd, recs, n);
 }
@@ -3284,6 +3313,7 @@ int smplgpu_lattice_begin_goals(smplgpu_ctx* ctx, const int32_t* slots, const do
                 g.xyz[a] = in.pose[a];
                 g.xyz_tol[a] = in.xyz_tolerance[a];
             }
+            rpy_matrix(in.pose[3], in.pose[4], in.pose[5], g.R);   // the snap's IK target: the full pose of the record
             if (in.type == SMPLGPU_GOAL_XYZ_RPY) {
                 if (bad_tolerance(in.rpy_tolerance)) return fail(ctx, SMPLGPU_ERR_INVALID, "goal %d: rpy tolerance is NaN or negative", i);
                 g.rpy_tol = in.rpy_tolerance;
@@ -3337,7 +3367,7 @@ int smplgpu_lattice_expand_submit(smplgpu_ctx* ctx, const int32_t* slot, const i
     int* out_h = out_succ + ne;
     int* out_count = out_h + ne;
     // the kernels read the (slot, state id) pairs from, and write the results to, page-locked host memory directly
-    if (ctx->lat_fused) {
+    if (ctx->lat_fused && !B.snap) {
         lattice_round_kernel<<<n, LROUND_THREADS, ctx->lat_round_smem, ctx->stream>>>(
             ctx->d_blob, ctx->blob_words, ctx->d_model, ctx->d_df, ctx->grid32, ctx->grid, B, ctx->lat_params, ctx->lat_vals,
             ctx->bank.dist, ctx->bank.DX, ctx->bank.DY, ctx->bank_slot_dz, in_slot, in_parent, n, out_succ, out_h, out_count,
@@ -3351,6 +3381,11 @@ int smplgpu_lattice_expand_submit(smplgpu_ctx* ctx, const int32_t* slot, const i
     lattice_gen_kernel<<<(unsigned)((ne + 127) / 128), 128, 0, ctx->stream>>>(ctx->d_model, B, in_slot, in_parent, n, dq0, dq1, dactive,
                                                                               ctx->d_stats);
     ++ctx->launches;
+    if (B.snap) {
+        lattice_snap_kernel<<<(unsigned)((n + IK_WARPS - 1) / IK_WARPS), 32 * IK_WARPS, 0, ctx->stream>>>(
+            ctx->d_model, B, in_slot, in_parent, n, dq1, dactive, ctx->d_snap_counters);
+        ++ctx->launches;
+    }
     int r = launch_edges(ctx, dq0, dq1, (int)ne, dverdict, nullptr);
     if (r) return r;
     lattice_commit_kernel<<<(unsigned)((n * 32 + 127) / 128), 128, 0, ctx->stream>>>(
@@ -3408,6 +3443,96 @@ int smplgpu_lattice_states(smplgpu_ctx* ctx, const int32_t* slot, const int32_t*
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(q_out, d_out, ob, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+///////////////////////////////////////////////////////////////////////////////
+// planning-link IK and the snap action
+///////////////////////////////////////////////////////////////////////////////
+
+static bool bad_ik_params(const smplgpu_ik_params* p)
+{
+    return p->max_iterations < 1 || !(p->tolerance > 0.0);
+}
+
+int smplgpu_planning_link_ik(smplgpu_ctx* ctx, const double* pose6, const double* seeds, int n,
+                             const smplgpu_ik_params* params, double* q_out, uint8_t* ok, int32_t* iterations)
+{
+    if (!ctx || n < 0 || !params) return SMPLGPU_ERR_INVALID;
+    if (bad_ik_params(params)) return fail(ctx, SMPLGPU_ERR_INVALID, "IK: max_iterations < 1, or a tolerance that is not positive");
+    if (!ctx->has_robot) return fail(ctx, SMPLGPU_ERR_STATE, "robot tables not set (smplgpu_set_robot)");
+    if (n == 0) return 0;
+    if (!pose6 || !seeds || !q_out || !ok || !iterations) return fail(ctx, SMPLGPU_ERR_INVALID, "null pointer");
+    const int dof = ctx->h_model->dof;
+    std::vector<IkTarget> tg(n);
+    for (int k = 0; k < n; ++k) {
+        const double* P = pose6 + 6 * (size_t)k;
+        for (int a = 0; a < 3; ++a) tg[k].p[a] = P[a];
+        rpy_matrix(P[3], P[4], P[5], tg[k].R);
+    }
+    const size_t tb = (size_t)n * sizeof(IkTarget), qb = (size_t)n * dof * sizeof(double);
+    const size_t ib = ((size_t)n * sizeof(int) + 7) / 8 * 8, ob = ((size_t)n + 7) / 8 * 8;
+    int r = grow(ctx, &ctx->d_misc, &ctx->misc_cap, tb + 2 * qb + ib + ob + 64);
+    if (r) return r;
+    uint8_t* base = (uint8_t*)ctx->d_misc;
+    IkTarget* d_tg = (IkTarget*)base;
+    double* d_seeds = (double*)(base + tb);
+    double* d_q = (double*)(base + tb + qb);
+    int* d_it = (int*)(base + tb + 2 * qb);
+    uint8_t* d_ok = base + tb + 2 * qb + ib;
+    CU(cudaMemcpyAsync(d_tg, tg.data(), tb, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_seeds, seeds, qb, cudaMemcpyHostToDevice, ctx->stream));
+    planning_link_ik_kernel<<<(unsigned)((n + IK_WARPS - 1) / IK_WARPS), 32 * IK_WARPS, 0, ctx->stream>>>(
+        ctx->d_model, d_tg, d_seeds, n, params->max_iterations, params->tolerance, d_q, d_ok, d_it);
+    ++ctx->launches;
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(q_out, d_q, qb, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(ok, d_ok, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(iterations, d_it, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    int n_ok = 0;
+    for (int k = 0; k < n; ++k) n_ok += ok[k] ? 1 : 0;
+    return n_ok;
+}
+
+int smplgpu_lattice_set_snap(smplgpu_ctx* ctx, const smplgpu_snap_params* p)
+{
+    if (!ctx || !p) return SMPLGPU_ERR_INVALID;
+    if (std::isnan(p->dist_thresh) || p->dist_thresh < 0.0) return fail(ctx, SMPLGPU_ERR_INVALID, "snap threshold is NaN or negative");
+    if (bad_ik_params(&p->ik)) return fail(ctx, SMPLGPU_ERR_INVALID, "IK: max_iterations < 1, or a tolerance that is not positive");
+    if (!ctx->has_lat) return fail(ctx, SMPLGPU_ERR_STATE, "lattices not created (smplgpu_lattice_create)");
+    for (int b = 0; b < SMPLGPU_EXPAND_BUFFERS; ++b) {
+        if (ctx->lat_n[b] >= 0) return fail(ctx, SMPLGPU_ERR_STATE, "lattice buffer %d is in flight", b);
+    }
+    const int snap = p->enabled ? 1 : 0;
+    const int stride = ctx->lat_prim_stride + snap;
+    if (stride > LATTICE_MAX_STRIDE)
+        return fail(ctx, SMPLGPU_ERR_LIMIT, "%d successors per expansion with the snap (limit %d)", stride, LATTICE_MAX_STRIDE);
+    if (snap && !ctx->d_snap_counters) {
+        CU(cudaMalloc(&ctx->d_snap_counters, 2 * sizeof(unsigned long long)));
+        CU(cudaMemset(ctx->d_snap_counters, 0, 2 * sizeof(unsigned long long)));
+    }
+    CU(cudaStreamSynchronize(ctx->stream));
+    LatticeBank& B = ctx->lat;
+    B.snap = snap;
+    B.stride = stride;
+    B.snap_thresh = p->dist_thresh;
+    B.ik_max_iterations = p->ik.max_iterations;
+    B.ik_tolerance = p->ik.tolerance;
+    const int r = lattice_round_buffers(ctx);
+    return r ? r : stride;
+}
+
+int smplgpu_lattice_snap_counters(smplgpu_ctx* ctx, int64_t counters[2])
+{
+    if (!ctx || !counters) return SMPLGPU_ERR_INVALID;
+    counters[0] = counters[1] = 0;
+    if (!ctx->d_snap_counters) return 0;
+    unsigned long long c[2];
+    CU(cudaMemcpyAsync(c, ctx->d_snap_counters, sizeof(c), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    counters[0] = (int64_t)c[0];
+    counters[1] = (int64_t)c[1];
     return 0;
 }
 

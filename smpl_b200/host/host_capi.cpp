@@ -1,6 +1,7 @@
 // Flat C entry points over the host-side C++ (model builder + adapters) so the
 // Python plumbing (tests, bench.py) can drive it with ctypes.  Declared in
 // include/smplhost.h.
+#include <array>
 #include <chrono>
 #include <cmath>
 #include <cstring>
@@ -234,7 +235,8 @@ int smplhost_tables_pairs(smplhost_tables* h, int32_t* out, int max_pairs)
 
 static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const double* starts,
                           const smplgpu_goal* goals, int nq, int max_concurrent, int32_t* summary, int32_t* path_ids,
-                          int max_path, double* stats, double* path_states)
+                          int max_path, double* stats, double* path_states, const smplhost_snap_params* snap = nullptr,
+                          int64_t* counters = nullptr)
 {
     if (!ctx || !p || nq < 0 || (nq > 0 && (!starts || !goals || !summary))) {
         g_err = "smplhost_plan_batch: null argument";
@@ -267,6 +269,12 @@ static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const
         cfg.xyz_tolerance[a] = p->xyz_tolerance[a];
         cfg.origin[a] = p->origin[a];
         cfg.dims[a] = p->dims[a];
+    }
+    if (snap && snap->enabled) {
+        cfg.snap = true;
+        cfg.snap_dist_thresh = snap->dist_thresh;
+        cfg.snap_weight = snap->weight;
+        cfg.ik = snap->ik;
     }
     smplhost::BatchPlanner planner(ctx, cfg, max_concurrent);
     std::vector<smplhost::QueryResult> out;
@@ -307,18 +315,27 @@ static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const
         stats[8] = s.setup_seconds;
         stats[9] = s.max_wait_seconds;
     }
+    if (counters) {
+        counters[0] = planner.stats().ik_attempted;
+        counters[1] = planner.stats().ik_converged;
+    }
     return 0;
 }
 
 // one planner thread per context, queries dealt round-robin
 static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
                                const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
-                               int32_t* path_ids, int max_path, double* stats, double* path_states)
+                               int32_t* path_ids, int max_path, double* stats, double* path_states,
+                               const smplhost_snap_params* snap = nullptr, int64_t* counters = nullptr)
 {
+    if (counters) {
+        counters[0] = counters[1] = 0;
+    }
     if (n_ctx == 1) {
         return plan_batch_one(ctxs[0], p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path, stats,
-                              path_states);
+                              path_states, snap, counters);
     }
+    std::vector<std::array<int64_t, 2>> ik(n_ctx, std::array<int64_t, 2>{ { 0, 0 } });
     const int dof = p->dof;
     std::vector<int> rc(n_ctx, 0);
     std::vector<std::string> errs(n_ctx);
@@ -351,7 +368,7 @@ static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplho
             pt.n_threads = 1;
             rc[t] = plan_batch_one(ctxs[t], &pt, s.data(), g.data(), m, max_concurrent_per_ctx, sum.data(),
                                    path_ids ? paths.data() : nullptr, max_path, st[t].data(),
-                                   path_states ? pstates.data() : nullptr);
+                                   path_states ? pstates.data() : nullptr, snap, ik[t].data());
             if (rc[t] != 0) {
                 errs[t] = g_err;   // thread-local: copy it out
                 return;
@@ -376,6 +393,12 @@ static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplho
         if (rc[t] != 0) {
             g_err = errs[t];
             return rc[t];
+        }
+    }
+    if (counters) {
+        for (int t = 0; t < n_ctx; ++t) {
+            counters[0] += ik[t][0];
+            counters[1] += ik[t][1];
         }
     }
     if (stats) {
@@ -436,9 +459,10 @@ static bool bad_tolerance(double t)
     return std::isnan(t) || t < 0.0;
 }
 
-int smplhost_plan_batch_goals(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
-                              const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
-                              int32_t* path_ids, int max_path, double* stats, double* path_states)
+// the argument and goal-record checks of smplhost_plan_batch_goals (those of smplgpu_lattice_begin_goals), before
+// any query starts
+static int check_goal_args(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const smplgpu_goal* goals,
+                           int nq)
 {
     if (!ctxs || n_ctx <= 0 || !p || nq < 0 || (nq > 0 && !goals)) {
         g_err = "smplhost_plan_batch_goals: bad argument";
@@ -472,8 +496,42 @@ int smplhost_plan_batch_goals(smplgpu_ctx* const* ctxs, int n_ctx, const smplhos
             return SMPLGPU_ERR_INVALID;
         }
     }
+    return 0;
+}
+
+int smplhost_plan_batch_goals(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
+                              const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
+                              int32_t* path_ids, int max_path, double* stats, double* path_states)
+{
+    const int r = check_goal_args(ctxs, n_ctx, p, goals, nq);
+    if (r) return r;
     return plan_batch_contexts(ctxs, n_ctx, p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path,
                                stats, path_states);
+}
+
+int smplhost_plan_batch_snap(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
+                             const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
+                             int32_t* path_ids, int max_path, double* stats, double* path_states,
+                             const smplhost_snap_params* snap, int64_t* counters)
+{
+    const int r = check_goal_args(ctxs, n_ctx, p, goals, nq);
+    if (r) return r;
+    if (!snap) {
+        g_err = "smplhost_plan_batch_snap: null snap parameters";
+        return SMPLGPU_ERR_INVALID;
+    }
+    // the checks of smplgpu_lattice_set_snap, and the cost weight, before any query starts
+    if (std::isnan(snap->dist_thresh) || snap->dist_thresh < 0.0 || std::isnan(snap->weight) || snap->weight < 0.0 ||
+        snap->weight > 1e6) {
+        g_err = "smplhost_plan_batch_snap: snap threshold or weight is NaN, negative or too large";
+        return SMPLGPU_ERR_INVALID;
+    }
+    if (snap->ik.max_iterations < 1 || !(snap->ik.tolerance > 0.0)) {
+        g_err = "smplhost_plan_batch_snap: IK max_iterations < 1, or a tolerance that is not positive";
+        return SMPLGPU_ERR_INVALID;
+    }
+    return plan_batch_contexts(ctxs, n_ctx, p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path,
+                               stats, path_states, snap, counters);
 }
 
 struct smplhost_adapters

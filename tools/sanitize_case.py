@@ -41,6 +41,10 @@ pp = scenes.PlanParams(7); pp.max_expansions = 60
 st, g = scenes.tabletop_queries(6, seed=13)
 res, stats = api.plan_batch(pctx, ps, pt, pp, st, g, max_concurrent=4, n_threads=2)
 pctx.probe_df_lookup_rate()
+# the planning-link IK kernel and a round chain with the snap action
+ik_seeds = st + 0.05
+pctx.planning_link_ik(pctx.planning_frame_fk(st), ik_seeds)
+api.plan_batch(pctx, ps, pt, pp, st, g, max_concurrent=4, snap=api.SnapParams(dist_thresh=0.2))
 # scene ingest (voxeliser + EDT) and the indexed-edge batch of path shortcutting
 ictx, it = api.setup_context(scenes.pr2_shelf_objects_scene())
 paths = [q[:12].copy(), q[20:40].copy()]
