@@ -344,6 +344,14 @@ int smplgpu_bfs_bank_run_slots(smplgpu_ctx* ctx, const int32_t* slots, const int
  * (smplgpu_expand_batch*, smplgpu_bfs_bank_distances) before smplgpu_bfs_bank_run_done returns 1 or
  * smplgpu_bfs_bank_run_wait returns.  smplgpu_bfs_bank_run_done: 1 finished / nothing in flight, 0 still running. */
 int smplgpu_bfs_bank_run_slots_async(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, int n);
+/* The two above with any number of seeds per slot (BFS_3D::run(begin, end), bfs3d.h:157-211, every seed of the list
+ * committed): slot slots[i] is seeded at seeds_xyz[seed_offsets[i] .. seed_offsets[i + 1] - 1][3].  seed_offsets[n + 1]
+ * is non-decreasing from 0.  Seeds outside the grid are dropped; a slot with none has no goal cell.  Returns the
+ * number of seeds inside the grid (the synchronous form) or n (the asynchronous one). */
+int smplgpu_bfs_bank_run_slots_multi(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz,
+                                     const int32_t* seed_offsets, int n);
+int smplgpu_bfs_bank_run_slots_multi_async(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz,
+                                           const int32_t* seed_offsets, int n);
 int smplgpu_bfs_bank_run_done(smplgpu_ctx* ctx);
 int smplgpu_bfs_bank_run_wait(smplgpu_ctx* ctx);
 /* BFS_3D::getDistance(cell) of slot[i] */
@@ -432,6 +440,19 @@ typedef struct smplgpu_goal {
  * computed here, on the host.  An unknown type, or a NaN or negative tolerance the type reads, is SMPLGPU_ERR_INVALID. */
 int smplgpu_lattice_begin_goals(smplgpu_ctx* ctx, const int32_t* slots, const double* starts,
                                 const int32_t* start_goal_dist_cells, const smplgpu_goal* goals, int n);
+/* Goal sets: query i accepts any record of goals[goal_offsets[i] .. goal_offsets[i + 1] - 1] (1 to
+ * SMPLGPU_MAX_GOAL_SET records, types may be mixed; goal_offsets[n + 1] non-decreasing from 0).  A successor is tested
+ * against the records in set order, and the first one it satisfies is its reached index: the h word of a successor
+ * flagged SMPLGPU_LATTICE_GOAL_FLAG carries that index instead of a heuristic.  The slot's BFS must have been seeded at
+ * the goal positions of all records (smplgpu_bfs_bank_run_slots_multi*).  The snap action (smplgpu_lattice_set_snap)
+ * targets the record whose goal position is nearest to the expanded state's target-offset position (squared
+ * Euclidean distance, the lower index on a tie).  smplgpu_lattice_begin_goals is this call with sets of one.  Each
+ * record is checked as smplgpu_lattice_begin_goals checks it; a set that is empty or larger than the bound is
+ * SMPLGPU_ERR_INVALID too. */
+#define SMPLGPU_MAX_GOAL_SET 64
+int smplgpu_lattice_begin_goal_sets(smplgpu_ctx* ctx, const int32_t* slots, const double* starts,
+                                    const int32_t* start_goal_dist_cells, const smplgpu_goal* goals,
+                                    const int32_t* goal_offsets, int n);
 /* One round: expansion i expands state parent_id[i] of the query in slot[i] (at most one expansion per slot and
  * round).  submit queues the work and returns; wait blocks and hands out pointers into page-locked memory valid
  * until the next submit on `buffer` (0 .. SMPLGPU_EXPAND_BUFFERS - 1):

@@ -134,6 +134,18 @@ int smplhost_plan_batch_snap(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost
                              const double* starts, const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx,
                              int32_t* summary, int32_t* path_ids, int max_path, double* stats, double* path_states,
                              const smplhost_snap_params* snap, int64_t* counters);
+/* Goal sets: query i succeeds at a state that satisfies any record of goals[goal_offsets[i] .. goal_offsets[i + 1] - 1]
+ * (1 to SMPLGPU_MAX_GOAL_SET records, types may be mixed; goal_offsets[nq + 1] non-decreasing from 0).  Its BFS
+ * heuristic is seeded at the goal positions of all records; the snap action (snap nullable = off) targets the record
+ * nearest to the expanded state (smplgpu_lattice_begin_goal_sets).  reached_goal[nq]: the index in the set of the
+ * first record that the path's goal-reaching action satisfies, -1 when the query is unsolved.  The other outputs are
+ * those of smplhost_plan_batch_snap; a set of one plans as smplhost_plan_batch_goals / _snap.  Bad sets, offsets,
+ * records or snap parameters are SMPLGPU_ERR_INVALID before anything is planned. */
+int smplhost_plan_batch_goal_sets(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* params,
+                                  const double* starts, const smplgpu_goal* goals, const int32_t* goal_offsets, int nq,
+                                  int max_concurrent_per_ctx, int32_t* summary, int32_t* path_ids, int max_path,
+                                  double* stats, double* path_states, const smplhost_snap_params* snap,
+                                  int64_t* counters, int32_t* reached_goal);
 
 /* ---- drop-in adapters (smpl_b200/host/gpu_adapters.h): the reference's CollisionChecker / RobotModel /
  * RobotHeuristic virtuals implemented over the C ABI.  These shims drive the C++ objects one virtual call at

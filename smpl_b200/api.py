@@ -73,6 +73,26 @@ def pose_goals(poses, xyz_tolerance=(0.015, 0.015, 0.015), rpy_tolerance=None):
     return out
 
 
+MAX_GOAL_SET = 64   # SMPLGPU_MAX_GOAL_SET: records in one query's goal set
+
+
+def goal_sets(sets):
+    """A goal set per query, for plan_batch(goals=...): sets is a list of GOAL_DTYPE record arrays (1 to MAX_GOAL_SET
+    records each, types may be mixed).  A query succeeds at a state that satisfies any record of its set.
+    Returns (records, offsets): the records concatenated, and offsets (nq + 1,) int32 with query i's records at
+    records[offsets[i]:offsets[i + 1]]."""
+    sets = [np.asarray(g).reshape(-1) for g in sets]
+    for i, g in enumerate(sets):
+        if g.dtype != GOAL_DTYPE:
+            raise ValueError("goal set %d: records must be GOAL_DTYPE" % i)
+        if not 1 <= len(g) <= MAX_GOAL_SET:
+            raise ValueError("goal set %d has %d records (1 to %d)" % (i, len(g), MAX_GOAL_SET))
+    offsets = np.zeros(len(sets) + 1, np.int32)
+    offsets[1:] = np.cumsum([len(g) for g in sets])
+    records = np.concatenate(sets) if sets else np.zeros(0, GOAL_DTYPE)
+    return np.ascontiguousarray(records), offsets
+
+
 def joint_goals(angles, angle_tolerances):
     """Goal records for joint configurations: angles (n, dof); angle_tolerances (dof,) or (n, dof).  The state is a
     goal when every planning variable is within its tolerance (no angle wrapping)."""
@@ -186,6 +206,8 @@ def gpu_lib():
         L.smplgpu_bfs_bank_run.argtypes = [vp, ip]
         L.smplgpu_bfs_bank_run_slots.argtypes = [vp, ip, ip, i]
         L.smplgpu_bfs_bank_run_slots_async.argtypes = [vp, ip, ip, i]
+        L.smplgpu_bfs_bank_run_slots_multi.argtypes = [vp, ip, ip, ip, i]
+        L.smplgpu_bfs_bank_run_slots_multi_async.argtypes = [vp, ip, ip, ip, i]
         L.smplgpu_bfs_bank_run_done.argtypes = [vp]
         L.smplgpu_bfs_bank_run_wait.argtypes = [vp]
         L.smplgpu_bfs_bank_distances.argtypes = [vp, ip, ip, i, ip]
@@ -240,6 +262,10 @@ def host_lib():
         H.smplhost_plan_batch_snap.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PlanParamsC), c_double_p,
                                                C.POINTER(GoalC), C.c_int, C.c_int, c_int32_p, c_int32_p, C.c_int,
                                                c_double_p, c_double_p, C.POINTER(SnapParamsC), C.POINTER(C.c_int64)]
+        H.smplhost_plan_batch_goal_sets.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PlanParamsC), c_double_p,
+                                                    C.POINTER(GoalC), c_int32_p, C.c_int, C.c_int, c_int32_p, c_int32_p,
+                                                    C.c_int, c_double_p, c_double_p, C.POINTER(SnapParamsC),
+                                                    C.POINTER(C.c_int64), c_int32_p]
         H.smplhost_shortcut_paths.argtypes = [vp, C.c_int, c_uint8_p, c_double_p, c_int32_p, C.c_int, C.c_int, c_int32_p,
                                               c_int32_p, c_double_p]
         H.smplhost_interpolate_paths.argtypes = [vp, vp, c_double_p, c_int32_p, C.c_int, c_double_p, C.c_int, c_int32_p,
@@ -676,6 +702,18 @@ class GpuContext:
         s = np.ascontiguousarray(seeds, dtype=np.int32).reshape(-1, 3)
         return self._ck(self.L.smplgpu_bfs_bank_run_slots(self.h, _ip(sl), _ip(s), len(sl)), "bfs_bank_run_slots")
 
+    def bfs_bank_run_slots_multi(self, slots, seed_sets, wait=True):
+        """smplgpu_bfs_bank_run_slots_multi (_async when wait is False): slot slots[i] seeded at every cell of
+        seed_sets[i] ((k, 3) ints, k >= 0).  Returns the seeds in bounds (synchronous) or the slot count."""
+        sl = np.ascontiguousarray(slots, dtype=np.int32)
+        cells = [np.asarray(c, np.int32).reshape(-1, 3) for c in seed_sets]
+        off = np.zeros(len(cells) + 1, np.int32)
+        off[1:] = np.cumsum([len(c) for c in cells])
+        s = np.ascontiguousarray(np.concatenate(cells) if cells else np.zeros((0, 3), np.int32), dtype=np.int32)
+        s = s if s.size else np.zeros(3, np.int32)
+        f = self.L.smplgpu_bfs_bank_run_slots_multi if wait else self.L.smplgpu_bfs_bank_run_slots_multi_async
+        return self._ck(f(self.h, _ip(sl), _ip(s), _ip(off), len(sl)), "bfs_bank_run_slots_multi")
+
     def bfs_bank_run_slots_async(self, slots, seeds):
         """Queues the BFS of the listed slots and returns; poll bfs_bank_run_done() or call bfs_bank_run_wait()."""
         sl = np.ascontiguousarray(slots, dtype=np.int32)
@@ -865,7 +903,9 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
     """smplhost_plan_batch: many ARA* queries in lock step, one device call per round.
     params: smpl_b200.scenes.PlanParams.  Returns (list of dict per query, stats dict).
     goals: (nq, 3) positions (XYZ goals with params.xyz_tolerance), or goal records of GOAL_DTYPE (pose_goals,
-    joint_goals; types may be mixed), which go through smplhost_plan_batch_goals.
+    joint_goals; types may be mixed), which go through smplhost_plan_batch_goals, or a goal set per query, the
+    (records, offsets) pair of goal_sets(), through smplhost_plan_batch_goal_sets: each result then also holds
+    reached_goal, the index in the query's set of the record its path reaches (-1 when unsolved).
     `ctx` may be a list of contexts (same GPU, same scene): one planner thread per context
     (smplhost_plan_batch_multi), max_concurrent is then per context.
     snap: SnapParams -- the snap-to-goal action, through smplhost_plan_batch_snap (position goals become XYZ goal
@@ -873,6 +913,12 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
     H = host_lib()
     dof = tables.dof
     starts = np.ascontiguousarray(starts, dtype=np.float64).reshape(-1, dof)
+    offsets = None
+    if isinstance(goals, tuple):
+        goals, offsets = goals
+        offsets = np.ascontiguousarray(offsets, dtype=np.int32).reshape(-1)
+        if len(offsets) != len(starts) + 1:
+            raise ValueError("%d starts, %d goal sets" % (len(starts), len(offsets) - 1))
     records = isinstance(goals, np.ndarray) and goals.dtype == GOAL_DTYPE
     if snap is not None and not records:
         goals = pose_goals(np.asarray(goals, np.float64).reshape(-1, 3), params.xyz_tolerance)
@@ -881,7 +927,7 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
         goals = np.ascontiguousarray(goals.reshape(-1))
     else:
         goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(-1, 3)
-    if len(goals) != len(starts):
+    if offsets is None and len(goals) != len(starts):
         raise ValueError("%d starts, %d goals" % (len(starts), len(goals)))
     nq = len(starts)
     lo, hi, cont = tables.limits()
@@ -912,7 +958,17 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
     pstates = np.zeros((nq, max_path, dof), np.float64) if want_states else None
     ps_ptr = _dp(pstates) if want_states else None
     counters = np.zeros(2, np.int64)
-    if snap is not None:
+    reached = np.full(nq, -1, np.int32)
+    if offsets is not None:
+        ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
+        arr = (C.c_void_p * len(ctxs))(*[c.h for c in ctxs])
+        sp = snap.c() if snap is not None else None
+        r = H.smplhost_plan_batch_goal_sets(arr, len(ctxs), C.byref(P), _dp(starts),
+                                            goals.ctypes.data_as(C.POINTER(GoalC)), _ip(offsets), nq,
+                                            int(max_concurrent), _ip(summary), _ip(paths), int(max_path), _dp(stats),
+                                            ps_ptr, C.byref(sp) if sp is not None else None,
+                                            counters.ctypes.data_as(C.POINTER(C.c_int64)), _ip(reached))
+    elif snap is not None:
         ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
         arr = (C.c_void_p * len(ctxs))(*[c.h for c in ctxs])
         sp = snap.c()
@@ -940,6 +996,8 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
                         path_ids=paths[i, :min(n, max_path)].copy(), num_states=int(summary[i, 4])))
         if want_states:   # ManipLattice::extractPath: joint values of the path states
             out[-1]["path_states"] = pstates[i, :min(n, max_path)].copy()
+        if offsets is not None:
+            out[-1]["reached_goal"] = int(reached[i])
     st = dict(rounds=int(stats[0]), edges_submitted=int(stats[1]), device_calls=int(stats[2]),
               device_seconds=float(stats[3]), host_seconds=float(stats[4]), total_seconds=float(stats[5]),
               bfs_runs=int(stats[6]), edges_resolved_f64=int(stats[7]), setup_seconds=float(stats[8]),

@@ -250,10 +250,29 @@ planning_link_ik_kernel(const DevModel* __restrict__ M, const IkTarget* __restri
     }
 }
 
+// The snap's target in a goal set: the record whose goal position is nearest to p (squared Euclidean distance, the
+// lower index on a tie).  The oracle (oracle/goal_sets/goal_set_lattice.cpp nearestRecord) uses the same expression.
+__device__ __forceinline__ int nearest_goal_record(const LatticeGoal* __restrict__ set, int n, const double* p)
+{
+    int best = 0;
+    double best_d = 0.0;
+    for (int r = 0; r < n; ++r) {
+        const double dx = set[r].pos[0] - p[0], dy = set[r].pos[1] - p[1], dz = set[r].pos[2] - p[2];
+        const double d = (dx * dx + dy * dy) + dz * dz;
+        if (r == 0 || d < best_d) {
+            best = r;
+            best_d = d;
+        }
+    }
+    return best;
+}
+
 // Round, step 1b with snaps enabled (between lattice_gen_kernel and the edge kernels): a warp per expansion.  The snap
 // is active when the parent's metric goal distance (the quantity of the short-distance switch) is within the
-// threshold; its action -- an IK solution for the goal pose seeded at the parent (XYZ and XYZ_RPY goals), or the
-// angles of a JOINT_STATE goal -- becomes word 0's edge when it exists and is within the joint limits.
+// threshold; its target is the record of the slot's goal set nearest to the parent's target-offset position
+// (nearest_goal_record), and its action -- an IK solution for that record's pose seeded at the parent (XYZ and XYZ_RPY
+// records), or the angles of a JOINT_STATE record -- becomes word 0's edge when it exists and is within the joint
+// limits.
 // lattice_gen_kernel left word 0 an inactive zero-length edge.  counters[0] / [1]: IK solves run / converged.
 __global__ void __launch_bounds__(32 * IK_WARPS)
 lattice_snap_kernel(const DevModel* __restrict__ M, LatticeBank B, const int* __restrict__ slot,
@@ -273,7 +292,15 @@ lattice_snap_kernel(const DevModel* __restrict__ M, LatticeBank B, const int* __
     }
     IkScratch& S = sS[warp];
     const int dof = M->dof;
-    const LatticeGoal* g = B.goal + s;
+    const LatticeGoal* set = B.goal + (size_t)s * SMPLGPU_MAX_GOAL_SET;
+    const int n_goals = B.n_goals[s];
+    int target = 0;
+    if (n_goals > 1) {
+        double pose[6];
+        planning_frame_fk(M, B.q + ((size_t)s * B.cap + p) * dof, pose);   // the same in every lane
+        target = nearest_goal_record(set, n_goals, pose);
+    }
+    const LatticeGoal* g = set + target;
     bool found = true;
     if (g->type == SMPLGPU_GOAL_JOINT_STATE) {
         if (lane < dof) {

@@ -122,7 +122,7 @@ struct smplgpu_ctx
     long long bank_level_cap = 0;
     int bank_step_tiles = 0;              // the stepwise run in flight: 0 = one level per launch, else the tile kernel's TILE_RPT
     int bank_step_blocks = 0;
-    std::vector<int32_t> staged_slots, staged_seeds;
+    std::vector<int32_t> staged_slots, staged_seeds, staged_offsets;
     unsigned long long* d_stats = nullptr;
     unsigned long long h_stats[4] = { 0, 0, 0, 0 };
     // bumped whenever an answer of the validity / heuristic entry points may change (robot, field, walls, BFS run):
@@ -371,7 +371,7 @@ static int finish_bank_run(smplgpu_ctx* ctx);   // waits for an asynchronous ban
 static void free_lattice(smplgpu_ctx* ctx)
 {
     cudaFree(ctx->lat.q); cudaFree(ctx->lat.coord); cudaFree(ctx->lat.gdist); cudaFree(ctx->lat.table);
-    cudaFree(ctx->lat.count); cudaFree(ctx->lat.goal); cudaFree(ctx->d_lat_aux);
+    cudaFree(ctx->lat.count); cudaFree(ctx->lat.goal); cudaFree(ctx->lat.n_goals); cudaFree(ctx->d_lat_aux);
     if (ctx->lat_resolved) cudaFreeHost(ctx->lat_resolved);
     ctx->lat_resolved = nullptr;
     memset(&ctx->lat, 0, sizeof(ctx->lat));
@@ -2630,6 +2630,21 @@ int smplgpu_bfs_bank_max_slots(smplgpu_ctx* ctx)
     return (int)std::max(1LL, std::min(by_index, 1LL << 20));
 }
 
+// the staging of a bank run of n_seeds seeds: seeds | slot mask, on the device and in page-locked memory
+static int reserve_bank_stage(smplgpu_ctx* ctx, size_t n_seeds, size_t* seed_cap)
+{
+    *seed_cap = (n_seeds * 3 * sizeof(int) + 15) / 16 * 16;
+    const size_t need = *seed_cap + (size_t)ctx->bank_slots + 64;
+    int r = grow(ctx, &ctx->d_bank_stage, &ctx->bank_stage_cap, need);
+    if (r) return r;
+    if (need > ctx->h_bank_stage_cap) {
+        if (ctx->h_bank_stage) { CU(cudaFreeHost(ctx->h_bank_stage)); ctx->h_bank_stage = nullptr; ctx->h_bank_stage_cap = 0; }
+        CU(cudaMallocHost(&ctx->h_bank_stage, need));
+        ctx->h_bank_stage_cap = need;
+    }
+    return 0;
+}
+
 int smplgpu_bfs_bank_create(smplgpu_ctx* ctx, int n_slots, double inflation_radius)
 {
     if (!ctx || n_slots <= 0) return SMPLGPU_ERR_INVALID;
@@ -2654,6 +2669,12 @@ int smplgpu_bfs_bank_create(smplgpu_ctx* ctx, int n_slots, double inflation_radi
     }
     ctx->bank_slots = n_slots;
     ctx->bank_slot_dz = nz + 2;
+    {
+        // room for a full goal set in every slot: runs queued while planners work never allocate
+        size_t seed_cap = 0;
+        const int r = reserve_bank_stage(ctx, (size_t)n_slots * SMPLGPU_MAX_GOAL_SET, &seed_cap);
+        if (r) return r;
+    }
     const int kmax = wall_threshold(ctx, inflation_radius);
     ctx->bank_kmax = kmax;
     unsigned int* d_count = (unsigned int*)ctx->d_seed_count;
@@ -2670,21 +2691,16 @@ int smplgpu_bfs_bank_create(smplgpu_ctx* ctx, int n_slots, double inflation_radi
 }
 
 // queues one bank run (walls of the listed slots from the field, reset, wavefront) on `stream`; the seeds and the
-// slot mask are staged in page-locked memory owned by the context, so nothing of the caller is read afterwards
-static int launch_bank_run(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, int n, cudaStream_t stream,
-                           int* d_seed_count, int* n_seeds_out)
+// slot mask are staged in page-locked memory owned by the context, so nothing of the caller is read afterwards.
+// Slot slots[i] is seeded at seeds_xyz[seed_offsets[i] .. seed_offsets[i + 1] - 1] (seed_offsets null: seed i alone).
+static int launch_bank_run(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, const int32_t* seed_offsets,
+                           int n, cudaStream_t stream, int* d_seed_count, int* n_seeds_out)
 {
     const int nx = ctx->grid.nx, ny = ctx->grid.ny, nz = ctx->grid.nz;
     ctx->bank_next_level = 0;   // set again by run_grid when this run goes level by level
-    const size_t seed_cap = ((size_t)n * 3 * sizeof(int) + 15) / 16 * 16;
-    const size_t need = seed_cap + (size_t)ctx->bank_slots + 64;
-    int r = grow(ctx, &ctx->d_bank_stage, &ctx->bank_stage_cap, need);
+    size_t seed_cap = 0;
+    int r = reserve_bank_stage(ctx, seed_offsets ? (size_t)seed_offsets[n] : (size_t)n, &seed_cap);
     if (r) return r;
-    if (need > ctx->h_bank_stage_cap) {
-        if (ctx->h_bank_stage) { CU(cudaFreeHost(ctx->h_bank_stage)); ctx->h_bank_stage = nullptr; ctx->h_bank_stage_cap = 0; }
-        CU(cudaMallocHost(&ctx->h_bank_stage, need));
-        ctx->h_bank_stage_cap = need;
-    }
     int* h_seeds = (int*)ctx->h_bank_stage;
     uint8_t* h_mask = (uint8_t*)ctx->h_bank_stage + seed_cap;
     memset(h_mask, 0, (size_t)ctx->bank_slots);
@@ -2694,10 +2710,13 @@ static int launch_bank_run(smplgpu_ctx* ctx, const int32_t* slots, const int32_t
         if (s < 0 || s >= ctx->bank_slots) return fail(ctx, SMPLGPU_ERR_INVALID, "slot %d out of range", s);
         if (h_mask[s]) return fail(ctx, SMPLGPU_ERR_INVALID, "slot %d listed twice", s);
         h_mask[s] = 1;
-        const int x = seeds_xyz[3 * i], y = seeds_xyz[3 * i + 1], z = seeds_xyz[3 * i + 2];
-        if (x >= 0 && y >= 0 && z >= 0 && x < nx && y < ny && z < nz) {
-            h_seeds[3 * n_in] = x; h_seeds[3 * n_in + 1] = y; h_seeds[3 * n_in + 2] = s * ctx->bank_slot_dz + z;
-            ++n_in;
+        const int e0 = seed_offsets ? seed_offsets[i] : i, e1 = seed_offsets ? seed_offsets[i + 1] : i + 1;
+        for (int e = e0; e < e1; ++e) {
+            const int x = seeds_xyz[3 * e], y = seeds_xyz[3 * e + 1], z = seeds_xyz[3 * e + 2];
+            if (x >= 0 && y >= 0 && z >= 0 && x < nx && y < ny && z < nz) {
+                h_seeds[3 * n_in] = x; h_seeds[3 * n_in + 1] = y; h_seeds[3 * n_in + 2] = s * ctx->bank_slot_dz + z;
+                ++n_in;
+            }
         }
     }
     uint8_t* d_mask = (uint8_t*)ctx->d_bank_stage + seed_cap;
@@ -2731,8 +2750,8 @@ static int launch_staged_bank_run(smplgpu_ctx* ctx)
     CU(cudaEventRecord(ctx->ev_bfs, ctx->stream));
     CU(cudaStreamWaitEvent(ctx->bfs_stream, ctx->ev_bfs, 0));
     int n_in = 0;
-    int r = launch_bank_run(ctx, ctx->staged_slots.data(), ctx->staged_seeds.data(), (int)ctx->staged_slots.size(),
-                            ctx->bfs_stream, ctx->d_bank_seed_count, &n_in);
+    int r = launch_bank_run(ctx, ctx->staged_slots.data(), ctx->staged_seeds.data(), ctx->staged_offsets.data(),
+                            (int)ctx->staged_slots.size(), ctx->bfs_stream, ctx->d_bank_seed_count, &n_in);
     if (r) return r;
     CU(cudaEventRecord(ctx->ev_bfs, ctx->bfs_stream));
     ctx->bank_run_state = 2;
@@ -2804,31 +2823,64 @@ static int finish_bank_run(smplgpu_ctx* ctx)
     return 0;
 }
 
-int smplgpu_bfs_bank_run_slots(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, int n)
+// seed_offsets[n + 1] non-decreasing from 0 (null: one seed per slot)
+static int check_seed_offsets(smplgpu_ctx* ctx, const int32_t* seed_offsets, int n)
 {
-    if (!ctx || n < 0 || (n > 0 && (!slots || !seeds_xyz))) return SMPLGPU_ERR_INVALID;
+    if (!seed_offsets) return 0;
+    if (seed_offsets[0] != 0) return fail(ctx, SMPLGPU_ERR_INVALID, "seed_offsets[0] is %d, not 0", seed_offsets[0]);
+    for (int i = 0; i < n; ++i) {
+        if (seed_offsets[i + 1] < seed_offsets[i]) return fail(ctx, SMPLGPU_ERR_INVALID, "seed_offsets decrease at %d", i + 1);
+    }
+    return 0;
+}
+
+static int bank_run_slots(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, const int32_t* seed_offsets, int n)
+{
     if (!ctx->has_bank) return fail(ctx, SMPLGPU_ERR_STATE, "BFS bank not created");
     if (n == 0) return 0;
-    int r = finish_bank_run(ctx);   // one run at a time: the staging buffers and the wavefront state are shared
+    int r = check_seed_offsets(ctx, seed_offsets, n);
+    if (r) return r;
+    r = finish_bank_run(ctx);   // one run at a time: the staging buffers and the wavefront state are shared
     if (r) return r;
     int n_in = 0;
-    r = launch_bank_run(ctx, slots, seeds_xyz, n, ctx->stream, ctx->d_seed_count, &n_in);
+    r = launch_bank_run(ctx, slots, seeds_xyz, seed_offsets, n, ctx->stream, ctx->d_seed_count, &n_in);
     if (r) return r;
     CU(cudaStreamSynchronize(ctx->stream));
     return n_in;
 }
 
-int smplgpu_bfs_bank_run_slots_async(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, int n)
+int smplgpu_bfs_bank_run_slots(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, int n)
 {
     if (!ctx || n < 0 || (n > 0 && (!slots || !seeds_xyz))) return SMPLGPU_ERR_INVALID;
+    return bank_run_slots(ctx, slots, seeds_xyz, nullptr, n);
+}
+
+int smplgpu_bfs_bank_run_slots_multi(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz,
+                                     const int32_t* seed_offsets, int n)
+{
+    if (!ctx || n < 0 || (n > 0 && (!slots || !seed_offsets || (!seeds_xyz && seed_offsets[n] > 0)))) return SMPLGPU_ERR_INVALID;
+    return bank_run_slots(ctx, slots, seeds_xyz, seed_offsets, n);
+}
+
+static int bank_run_slots_async(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, const int32_t* seed_offsets,
+                                int n)
+{
     if (!ctx->has_bank) return fail(ctx, SMPLGPU_ERR_STATE, "BFS bank not created");
     if (ctx->bank_run_state != 0) return fail(ctx, SMPLGPU_ERR_STATE, "a bank run is already in flight");
     if (n == 0) return 0;
     for (int i = 0; i < n; ++i) {
         if (slots[i] < 0 || slots[i] >= ctx->bank_slots) return fail(ctx, SMPLGPU_ERR_INVALID, "slot %d out of range", slots[i]);
     }
+    const int r = check_seed_offsets(ctx, seed_offsets, n);
+    if (r) return r;
     ctx->staged_slots.assign(slots, slots + n);
-    ctx->staged_seeds.assign(seeds_xyz, seeds_xyz + 3 * (size_t)n);
+    if (seed_offsets) {
+        ctx->staged_offsets.assign(seed_offsets, seed_offsets + n + 1);
+    } else {
+        ctx->staged_offsets.resize(n + 1);
+        for (int i = 0; i <= n; ++i) ctx->staged_offsets[i] = i;
+    }
+    ctx->staged_seeds.assign(seeds_xyz, seeds_xyz + 3 * (size_t)ctx->staged_offsets[n]);
     ctx->bank_run_state = 1;
     if (take_bank_turn(ctx)) {
         const int r = launch_staged_bank_run(ctx);
@@ -2839,6 +2891,19 @@ int smplgpu_bfs_bank_run_slots_async(smplgpu_ctx* ctx, const int32_t* slots, con
         }
     }
     return n;
+}
+
+int smplgpu_bfs_bank_run_slots_async(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz, int n)
+{
+    if (!ctx || n < 0 || (n > 0 && (!slots || !seeds_xyz))) return SMPLGPU_ERR_INVALID;
+    return bank_run_slots_async(ctx, slots, seeds_xyz, nullptr, n);
+}
+
+int smplgpu_bfs_bank_run_slots_multi_async(smplgpu_ctx* ctx, const int32_t* slots, const int32_t* seeds_xyz,
+                                           const int32_t* seed_offsets, int n)
+{
+    if (!ctx || n < 0 || (n > 0 && (!slots || !seed_offsets || (!seeds_xyz && seed_offsets[n] > 0)))) return SMPLGPU_ERR_INVALID;
+    return bank_run_slots_async(ctx, slots, seeds_xyz, seed_offsets, n);
 }
 
 int smplgpu_bfs_bank_run_done(smplgpu_ctx* ctx)
@@ -3053,10 +3118,20 @@ int smplgpu_expand_batch(smplgpu_ctx* ctx, const double* q0, const double* q1, c
 // device-resident lattices
 ///////////////////////////////////////////////////////////////////////////////
 
+// the staging of smplgpu_lattice_begin_goal_sets for n queries of n_rec goal records: starts | goal records |
+// slots | start distances | goal offsets | record -> query
+static size_t lattice_begin_bytes(int dof, size_t n, size_t n_rec)
+{
+    const size_t sb = (n * sizeof(int) + 7) / 8 * 8, ob = ((n + 1) * sizeof(int) + 7) / 8 * 8;
+    return n * dof * sizeof(double) + n_rec * sizeof(LatticeGoal) + 2 * sb + ob + (n_rec * sizeof(int) + 7) / 8 * 8 + 64;
+}
+
+// the slot's lattice, its goal set, and its share of the begin staging for a full goal set (reserved when the
+// lattices are created, so that no query admission allocates)
 static size_t lattice_bytes_per_slot(int dof, int cap, int table_size)
 {
     return (size_t)cap * dof * (sizeof(double) + sizeof(int)) + (size_t)cap * sizeof(int) + (size_t)table_size * sizeof(int) +
-           sizeof(int) + sizeof(LatticeGoal);
+           2 * sizeof(int) + SMPLGPU_MAX_GOAL_SET * sizeof(LatticeGoal) + lattice_begin_bytes(dof, 1, SMPLGPU_MAX_GOAL_SET);
 }
 
 static int lattice_table_size(int cap)
@@ -3148,9 +3223,13 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
         CU(cudaMalloc(&B.gdist, (size_t)n_slots * cap * sizeof(int)));
         CU(cudaMalloc(&B.table, (size_t)n_slots * tsize * sizeof(int)));
         CU(cudaMalloc(&B.count, (size_t)n_slots * sizeof(int)));
-        CU(cudaMalloc(&B.goal, (size_t)n_slots * sizeof(LatticeGoal)));
+        CU(cudaMalloc(&B.goal, (size_t)n_slots * SMPLGPU_MAX_GOAL_SET * sizeof(LatticeGoal)));
+        CU(cudaMalloc(&B.n_goals, (size_t)n_slots * sizeof(int)));
         CU(cudaMemset(B.count, 0, (size_t)n_slots * sizeof(int)));
+        CU(cudaMemset(B.n_goals, 0, (size_t)n_slots * sizeof(int)));
     }
+    r = grow(ctx, &ctx->d_misc, &ctx->misc_cap, lattice_begin_bytes(dof, n_slots, (size_t)n_slots * SMPLGPU_MAX_GOAL_SET));
+    if (r) return r;
     LatticeBank& B = ctx->lat;
     B.stride = stride;
     ctx->lat_prim_stride = stride;
@@ -3237,27 +3316,39 @@ static void rpy_matrix(double roll, double pitch, double yaw, double* R)
     R[6] = -sb1;       R[7] = cb1 * sc1;                    R[8] = cb1 * cc1;
 }
 
+// goals[goal_offsets[k] .. goal_offsets[k + 1] - 1] = the goal set of query k (offsets checked by the caller)
 static int lattice_begin_records(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
-                                 const std::vector<LatticeGoal>& goals, int n)
+                                 const std::vector<LatticeGoal>& goals, const int32_t* goal_offsets, int n)
 {
     const int dof = ctx->h_model->dof;
-    const size_t sb = ((size_t)n * sizeof(int) + 7) / 8 * 8, qb = (size_t)n * dof * sizeof(double),
-                 gb = (size_t)n * sizeof(LatticeGoal);
-    int r = grow(ctx, &ctx->d_misc, &ctx->misc_cap, 2 * sb + qb + gb + 64);
+    const size_t n_rec = goals.size();
+    const size_t sb = ((size_t)n * sizeof(int) + 7) / 8 * 8, ob = ((size_t)(n + 1) * sizeof(int) + 7) / 8 * 8,
+                 qb = (size_t)n * dof * sizeof(double), gb = n_rec * sizeof(LatticeGoal);
+    int r = grow(ctx, &ctx->d_misc, &ctx->misc_cap, lattice_begin_bytes(dof, n, n_rec));   // reserved by smplgpu_lattice_create
     if (r) return r;
+    std::vector<int32_t> goal_set(n_rec);
+    for (int k = 0; k < n; ++k) {
+        std::fill(goal_set.begin() + goal_offsets[k], goal_set.begin() + goal_offsets[k + 1], k);
+    }
     uint8_t* base = (uint8_t*)ctx->d_misc;
     double* d_starts = (double*)base;
     LatticeGoal* d_goals = (LatticeGoal*)(base + qb);
     int* d_slots = (int*)(base + qb + gb);
     int* d_gd = (int*)(base + qb + gb + sb);
+    int* d_offsets = (int*)(base + qb + gb + 2 * sb);
+    int* d_goal_set = (int*)(base + qb + gb + 2 * sb + ob);
     CU(cudaMemcpyAsync(d_starts, starts, qb, cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaMemcpyAsync(d_goals, goals.data(), gb, cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaMemcpyAsync(d_slots, slots, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaMemcpyAsync(d_gd, start_gd, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_offsets, goal_offsets, (size_t)(n + 1) * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_goal_set, goal_set.data(), n_rec * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     const size_t total = (size_t)n * ctx->lat.table_size;
+    const int threads = (int)std::max<size_t>((size_t)n, n_rec);
     lattice_clear_kernel<<<(unsigned)std::min<size_t>((total + 255) / 256, (size_t)ctx->sm_count * 16), 256, 0, ctx->stream>>>(ctx->lat, d_slots, n);
-    lattice_begin_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_model, ctx->lat, ctx->lat_params, ctx->lat_vals, d_slots,
-                                                                  d_starts, d_gd, d_goals, n);
+    lattice_begin_kernel<<<(threads + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_model, ctx->lat, ctx->lat_params, ctx->lat_vals,
+                                                                        d_slots, d_starts, d_gd, d_goals, d_goal_set,
+                                                                        d_offsets, n, (int)n_rec);
     ctx->launches += 2;
     CU(cudaGetLastError());
     CU(cudaStreamSynchronize(ctx->stream));   // the inputs may be pageable
@@ -3292,18 +3383,36 @@ int smplgpu_lattice_begin(smplgpu_ctx* ctx, const int32_t* slots, const double* 
         }
         rpy_matrix(0.0, 0.0, 0.0, g.R);
     }
-    return lattice_begin_records(ctx, slots, starts, start_gd, recs, n);
+    std::vector<int32_t> offsets(n + 1);
+    for (int i = 0; i <= n; ++i) offsets[i] = i;
+    return lattice_begin_records(ctx, slots, starts, start_gd, recs, offsets.data(), n);
 }
 
 int smplgpu_lattice_begin_goals(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
                                 const smplgpu_goal* goals, int n)
 {
     if (!ctx || n < 0) return SMPLGPU_ERR_INVALID;
+    std::vector<int32_t> offsets(n + 1);
+    for (int i = 0; i <= n; ++i) offsets[i] = i;
+    return smplgpu_lattice_begin_goal_sets(ctx, slots, starts, start_gd, goals, offsets.data(), n);
+}
+
+int smplgpu_lattice_begin_goal_sets(smplgpu_ctx* ctx, const int32_t* slots, const double* starts, const int32_t* start_gd,
+                                    const smplgpu_goal* goals, const int32_t* goal_offsets, int n)
+{
+    if (!ctx || n < 0) return SMPLGPU_ERR_INVALID;
     int r = lattice_begin_check(ctx, slots, starts, start_gd, goals, n);
     if (r || n == 0) return r;
+    if (!goal_offsets) return fail(ctx, SMPLGPU_ERR_INVALID, "null pointer");
+    if (goal_offsets[0] != 0) return fail(ctx, SMPLGPU_ERR_INVALID, "goal_offsets[0] is %d, not 0", goal_offsets[0]);
+    for (int k = 0; k < n; ++k) {
+        const long long m = (long long)goal_offsets[k + 1] - goal_offsets[k];
+        if (m < 1 || m > SMPLGPU_MAX_GOAL_SET)
+            return fail(ctx, SMPLGPU_ERR_INVALID, "query %d: goal set of %lld records (1 to %d)", k, m, SMPLGPU_MAX_GOAL_SET);
+    }
     const int dof = ctx->h_model->dof;
-    std::vector<LatticeGoal> recs(n);   // zero-filled
-    for (int i = 0; i < n; ++i) {
+    std::vector<LatticeGoal> recs(goal_offsets[n]);   // zero-filled
+    for (int i = 0; i < goal_offsets[n]; ++i) {
         const smplgpu_goal& in = goals[i];
         LatticeGoal& g = recs[i];
         g.type = in.type;
@@ -3329,7 +3438,7 @@ int smplgpu_lattice_begin_goals(smplgpu_ctx* ctx, const int32_t* slots, const do
             return fail(ctx, SMPLGPU_ERR_INVALID, "goal %d: unknown goal type %d", i, in.type);
         }
     }
-    return lattice_begin_records(ctx, slots, starts, start_gd, recs, n);
+    return lattice_begin_records(ctx, slots, starts, start_gd, recs, goal_offsets, n);
 }
 
 int smplgpu_lattice_expand_submit(smplgpu_ctx* ctx, const int32_t* slot, const int32_t* parent_id, int n, int buffer)

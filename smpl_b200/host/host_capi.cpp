@@ -233,10 +233,12 @@ int smplhost_tables_pairs(smplhost_tables* h, int32_t* out, int max_pairs)
     return d->n_pairs;
 }
 
+// goal_offsets (nullable: one goal record per query) gives each query's goal set; reached (nullable) gets each query's
+// reached_goal
 static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const double* starts,
                           const smplgpu_goal* goals, int nq, int max_concurrent, int32_t* summary, int32_t* path_ids,
                           int max_path, double* stats, double* path_states, const smplhost_snap_params* snap = nullptr,
-                          int64_t* counters = nullptr)
+                          int64_t* counters = nullptr, const int32_t* goal_offsets = nullptr, int32_t* reached = nullptr)
 {
     if (!ctx || !p || nq < 0 || (nq > 0 && (!starts || !goals || !summary))) {
         g_err = "smplhost_plan_batch: null argument";
@@ -280,7 +282,7 @@ static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const
     std::vector<smplhost::QueryResult> out;
     std::string err;
     const auto t0 = std::chrono::steady_clock::now();
-    if (!planner.plan(starts, goals, nq, out, &err)) {
+    if (!planner.plan(starts, goals, goal_offsets, nq, out, &err)) {
         g_err = err;
         return SMPLGPU_ERR_CUDA;
     }
@@ -292,6 +294,9 @@ static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const
         summary[5 * i + 2] = r.cost;
         summary[5 * i + 3] = (int)r.path_ids.size();
         summary[5 * i + 4] = r.num_states;
+        if (reached) {
+            reached[i] = r.reached_goal;
+        }
         if (path_ids) {
             for (int k = 0; k < max_path; ++k) {
                 path_ids[(size_t)i * max_path + k] = k < (int)r.path_ids.size() ? r.path_ids[k] : -1;
@@ -326,15 +331,17 @@ static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const
 static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
                                const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
                                int32_t* path_ids, int max_path, double* stats, double* path_states,
-                               const smplhost_snap_params* snap = nullptr, int64_t* counters = nullptr)
+                               const smplhost_snap_params* snap = nullptr, int64_t* counters = nullptr,
+                               const int32_t* goal_offsets = nullptr, int32_t* reached = nullptr)
 {
     if (counters) {
         counters[0] = counters[1] = 0;
     }
     if (n_ctx == 1) {
         return plan_batch_one(ctxs[0], p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path, stats,
-                              path_states, snap, counters);
+                              path_states, snap, counters, goal_offsets, reached);
     }
+    auto set_begin = [&](int i) { return goal_offsets ? goal_offsets[i] : i; };
     std::vector<std::array<int64_t, 2>> ik(n_ctx, std::array<int64_t, 2>{ { 0, 0 } });
     const int dof = p->dof;
     std::vector<int> rc(n_ctx, 0);
@@ -356,10 +363,12 @@ static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplho
                 return;
             }
             std::vector<double> s((size_t)m * dof);
-            std::vector<smplgpu_goal> g(m);
+            std::vector<smplgpu_goal> g;
+            std::vector<int32_t> off(1, 0), got(m, -1);
             for (int k = 0; k < m; ++k) {
                 std::copy(starts + (size_t)mine[k] * dof, starts + (size_t)(mine[k] + 1) * dof, s.begin() + (size_t)k * dof);
-                g[k] = goals[mine[k]];
+                g.insert(g.end(), goals + set_begin(mine[k]), goals + set_begin(mine[k] + 1));
+                off.push_back((int32_t)g.size());
             }
             std::vector<int32_t> sum((size_t)m * 5), paths(path_ids ? (size_t)m * max_path : 0);
             const size_t ps = (size_t)max_path * dof;
@@ -368,13 +377,16 @@ static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplho
             pt.n_threads = 1;
             rc[t] = plan_batch_one(ctxs[t], &pt, s.data(), g.data(), m, max_concurrent_per_ctx, sum.data(),
                                    path_ids ? paths.data() : nullptr, max_path, st[t].data(),
-                                   path_states ? pstates.data() : nullptr, snap, ik[t].data());
+                                   path_states ? pstates.data() : nullptr, snap, ik[t].data(), off.data(), got.data());
             if (rc[t] != 0) {
                 errs[t] = g_err;   // thread-local: copy it out
                 return;
             }
             for (int k = 0; k < m; ++k) {
                 std::copy(sum.begin() + (size_t)k * 5, sum.begin() + (size_t)(k + 1) * 5, summary + (size_t)mine[k] * 5);
+                if (reached) {
+                    reached[mine[k]] = got[k];
+                }
                 if (path_ids) {
                     std::copy(paths.begin() + (size_t)k * max_path, paths.begin() + (size_t)(k + 1) * max_path,
                               path_ids + (size_t)mine[k] * max_path);
@@ -459,8 +471,8 @@ static bool bad_tolerance(double t)
     return std::isnan(t) || t < 0.0;
 }
 
-// the argument and goal-record checks of smplhost_plan_batch_goals (those of smplgpu_lattice_begin_goals), before
-// any query starts
+// the argument and goal-record checks of smplhost_plan_batch_goals (those of smplgpu_lattice_begin_goals) of nq goal
+// records, before any query starts
 static int check_goal_args(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const smplgpu_goal* goals,
                            int nq)
 {
@@ -509,17 +521,9 @@ int smplhost_plan_batch_goals(smplgpu_ctx* const* ctxs, int n_ctx, const smplhos
                                stats, path_states);
 }
 
-int smplhost_plan_batch_snap(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
-                             const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
-                             int32_t* path_ids, int max_path, double* stats, double* path_states,
-                             const smplhost_snap_params* snap, int64_t* counters)
+// the checks of smplgpu_lattice_set_snap and the snap's cost weight
+static int check_snap_args(const smplhost_snap_params* snap)
 {
-    const int r = check_goal_args(ctxs, n_ctx, p, goals, nq);
-    if (r) return r;
-    if (!snap) {
-        g_err = "smplhost_plan_batch_snap: null snap parameters";
-        return SMPLGPU_ERR_INVALID;
-    }
     // the checks of smplgpu_lattice_set_snap, and the cost weight, before any query starts
     if (std::isnan(snap->dist_thresh) || snap->dist_thresh < 0.0 || std::isnan(snap->weight) || snap->weight < 0.0 ||
         snap->weight > 1e6) {
@@ -530,8 +534,60 @@ int smplhost_plan_batch_snap(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost
         g_err = "smplhost_plan_batch_snap: IK max_iterations < 1, or a tolerance that is not positive";
         return SMPLGPU_ERR_INVALID;
     }
+    return 0;
+}
+
+int smplhost_plan_batch_snap(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
+                             const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
+                             int32_t* path_ids, int max_path, double* stats, double* path_states,
+                             const smplhost_snap_params* snap, int64_t* counters)
+{
+    int r = check_goal_args(ctxs, n_ctx, p, goals, nq);
+    if (r) return r;
+    if (!snap) {
+        g_err = "smplhost_plan_batch_snap: null snap parameters";
+        return SMPLGPU_ERR_INVALID;
+    }
+    r = check_snap_args(snap);
+    if (r) return r;
     return plan_batch_contexts(ctxs, n_ctx, p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path,
                                stats, path_states, snap, counters);
+}
+
+int smplhost_plan_batch_goal_sets(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p,
+                                  const double* starts, const smplgpu_goal* goals, const int32_t* goal_offsets, int nq,
+                                  int max_concurrent_per_ctx, int32_t* summary, int32_t* path_ids, int max_path,
+                                  double* stats, double* path_states, const smplhost_snap_params* snap,
+                                  int64_t* counters, int32_t* reached_goal)
+{
+    if (nq < 0 || (nq > 0 && (!goal_offsets || !reached_goal))) {
+        g_err = "smplhost_plan_batch_goal_sets: bad argument";
+        return SMPLGPU_ERR_INVALID;
+    }
+    // the set checks of smplgpu_lattice_begin_goal_sets, before any query starts
+    if (nq > 0 && goal_offsets[0] != 0) {
+        g_err = "smplhost_plan_batch_goal_sets: goal_offsets[0] is not 0";
+        return SMPLGPU_ERR_INVALID;
+    }
+    for (int i = 0; i < nq; ++i) {
+        const long long m = (long long)goal_offsets[i + 1] - goal_offsets[i];
+        if (m < 1 || m > SMPLGPU_MAX_GOAL_SET) {
+            g_err = "smplhost_plan_batch_goal_sets: query " + std::to_string(i) + " has a goal set of " + std::to_string(m) +
+                    " records (1 to " + std::to_string(SMPLGPU_MAX_GOAL_SET) + ")";
+            return SMPLGPU_ERR_INVALID;
+        }
+    }
+    int r = check_goal_args(ctxs, n_ctx, p, goals, nq > 0 ? goal_offsets[nq] : 0);
+    if (r) return r;
+    if (snap) {
+        r = check_snap_args(snap);
+        if (r) return r;
+    }
+    if (counters) {
+        counters[0] = counters[1] = 0;
+    }
+    return plan_batch_contexts(ctxs, n_ctx, p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path,
+                               stats, path_states, snap, counters, goal_offsets, reached_goal);
 }
 
 struct smplhost_adapters
