@@ -498,8 +498,42 @@ typedef struct smplgpu_snap_params {
     smplgpu_ik_params ik;
 } smplgpu_snap_params;
 int smplgpu_lattice_set_snap(smplgpu_ctx* ctx, const smplgpu_snap_params* params);
-/* IK solves the snap actions of this context's rounds ran so far, and how many converged (running totals) */
+/* IK solves the snap actions of this context's rounds ran so far, and how many converged (running totals over the
+ * snap kinds) */
 int smplgpu_lattice_snap_counters(smplgpu_ctx* ctx, int64_t counters[2]);
+
+/* The three adaptive actions of ManipLatticeActionSpace, each enabled on its own and with its own threshold (metres
+ * of metric goal distance, as for smplgpu_snap_params).  Enabled kinds take successor words 0 .. k-1 in the order of
+ * their indices below, before the primitives'.  Every kind of an expansion aims at the same record, the one
+ * smplgpu_lattice_begin_goal_sets names, seeds its IK at the expanded state and produces nothing for a record type it
+ * does not apply to:
+ *   SMPLGPU_SNAP_RPY      XYZ_RPY records: the full-pose IK for the expanded state's own target-offset position (as
+ *                         smplgpu_planning_frame_fk reports it) and the record's orientation -- a turn in place
+ *   SMPLGPU_SNAP_XYZ      XYZ and XYZ_RPY records: the position-only IK (smplgpu_planning_link_ik_position) for the
+ *                         record's position, the orientation free
+ *   SMPLGPU_SNAP_XYZ_RPY  every record: smplgpu_lattice_set_snap's action (the full pose, or a joint record's angles)
+ * The IK parameters are shared. */
+#define SMPLGPU_SNAP_RPY      0
+#define SMPLGPU_SNAP_XYZ      1
+#define SMPLGPU_SNAP_XYZ_RPY  2
+typedef struct smplgpu_snap_kinds {
+    int32_t enabled[3];       /* by SMPLGPU_SNAP_* */
+    double  dist_thresh[3];   /* metres, >= 0 (checked for disabled kinds too) */
+    smplgpu_ik_params ik;
+} smplgpu_snap_kinds;
+/* smplgpu_lattice_set_snap for any set of kinds; smplgpu_lattice_set_snap is this call with SMPLGPU_SNAP_XYZ_RPY alone.
+ * Returns the stride, the number of enabled kinds + the primitives'; SMPLGPU_ERR_LIMIT above the stride limit,
+ * SMPLGPU_ERR_INVALID for a NaN or negative threshold of any kind or bad IK parameters. */
+int smplgpu_lattice_set_snaps(smplgpu_ctx* ctx, const smplgpu_snap_kinds* kinds);
+/* counters[2 k] / [2 k + 1]: IK solves the snap kind k (SMPLGPU_SNAP_*) ran so far, and how many converged */
+int smplgpu_lattice_snap_counters_by_kind(smplgpu_ctx* ctx, int64_t counters[6]);
+/* The position-only IK of the planning link: smplgpu_planning_link_ik with only the position rows -- e = the target
+ * position - the target-offset position, J its 3 x dof block, q += J^T (J J^T + 1e-6 I)^-1 e by a 3 x 3 Cholesky,
+ * converged when the three |e_i| <= tolerance; the orientation is free.  xyz[n][3] target positions, seeds[n][dof];
+ * outputs and return value as smplgpu_planning_link_ik. */
+int smplgpu_planning_link_ik_position(smplgpu_ctx* ctx, const double* xyz, const double* seeds, int n,
+                                      const smplgpu_ik_params* params, double* q_out, uint8_t* ok,
+                                      int32_t* iterations);
 
 /* ---- lattice states on the wire as 16-bit coordinates ---- */
 /* The real caller of the validity path, ManipLattice, holds a state as dof small integers (RobotCoord) and forms the

@@ -146,6 +146,23 @@ int smplhost_plan_batch_goal_sets(smplgpu_ctx* const* ctxs, int n_ctx, const smp
                                   int max_concurrent_per_ctx, int32_t* summary, int32_t* path_ids, int max_path,
                                   double* stats, double* path_states, const smplhost_snap_params* snap,
                                   int64_t* counters, int32_t* reached_goal);
+/* The snap actions SNAP_TO_RPY, SNAP_TO_XYZ and SNAP_TO_XYZ_RPY (smplgpu_lattice_set_snaps), each enabled on its own
+ * with its own threshold, at one cost of (int)(1000 * weight) (weight >= 0) and with one set of IK parameters. */
+typedef struct smplhost_snaps_params {
+    smplgpu_snap_kinds kinds;
+    double weight;
+} smplhost_snaps_params;
+/* smplhost_plan_batch_goal_sets with any set of snap kinds (snaps nullable = off).  counters[6] (nullable): by
+ * SMPLGPU_SNAP_* kind k, counters[2 k] the IK solves that kind ran and counters[2 k + 1] how many converged (summed
+ * over the contexts).  The goal action extractPath takes from an expansion is the first valid goal-reaching word (the
+ * snaps in kind order, then the primitives).  smplhost_plan_batch_snap and smplhost_plan_batch_goal_sets are this call
+ * with SMPLGPU_SNAP_XYZ_RPY alone.  Bad sets, offsets, records, thresholds (NaN or negative, of any kind) or IK
+ * parameters are SMPLGPU_ERR_INVALID before anything is planned. */
+int smplhost_plan_batch_snaps(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* params,
+                              const double* starts, const smplgpu_goal* goals, const int32_t* goal_offsets, int nq,
+                              int max_concurrent_per_ctx, int32_t* summary, int32_t* path_ids, int max_path,
+                              double* stats, double* path_states, const smplhost_snaps_params* snaps,
+                              int64_t* counters, int32_t* reached_goal);
 
 /* ---- drop-in adapters (smpl_b200/host/gpu_adapters.h): the reference's CollisionChecker / RobotModel /
  * RobotHeuristic virtuals implemented over the C ABI.  These shims drive the C++ objects one virtual call at

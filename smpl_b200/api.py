@@ -128,21 +128,61 @@ class SnapParamsC(C.Structure):
     _fields_ = [("enabled", C.c_int32), ("dist_thresh", C.c_double), ("weight", C.c_double), ("ik", IkParamsC)]
 
 
-class SnapParams:
-    """The snap-to-goal action of the batched planner (smplhost_snap_params): an expansion whose metric goal distance
-    is within dist_thresh metres first tries to jump straight to the goal -- to an IK solution for a pose goal, to the
-    angles of a joint goal -- at a cost of int(1000 * weight).  dist_thresh = 0.0 is the reference demo's setting."""
+SNAP_RPY, SNAP_XYZ, SNAP_XYZ_RPY = 0, 1, 2   # SMPLGPU_SNAP_*: the snap kinds, in successor-word order
+SNAP_KIND_NAMES = ("rpy", "xyz", "xyz_rpy")
 
-    def __init__(self, enabled=True, dist_thresh=0.0, weight=0.5, max_iterations=100, tolerance=1e-6):
+
+class SnapKindsC(C.Structure):
+    """smplgpu_snap_kinds (include/smplgpu.h)."""
+    _fields_ = [("enabled", C.c_int32 * 3), ("dist_thresh", C.c_double * 3), ("ik", IkParamsC)]
+
+
+class SnapsParamsC(C.Structure):
+    """smplhost_snaps_params (include/smplhost.h)."""
+    _fields_ = [("kinds", SnapKindsC), ("weight", C.c_double)]
+
+
+class SnapParams:
+    """The snap-to-goal actions of the batched planner.  enabled / dist_thresh: SNAP_TO_XYZ_RPY -- an expansion whose
+    metric goal distance is within dist_thresh metres first tries to jump straight to the goal: to an IK solution for a
+    pose goal's full pose, to the angles of a joint goal.  xyz_dist_thresh: SNAP_TO_XYZ (None = off), a position-only
+    IK solution for a pose goal's position, the orientation free.  rpy_dist_thresh: SNAP_TO_RPY (None = off), for an
+    XYZ_RPY goal an IK solution that keeps the expanded state's position and turns it to the goal's orientation.  Every
+    snap costs int(1000 * weight).  dist_thresh = 0.0 is the reference demo's setting."""
+
+    def __init__(self, enabled=True, dist_thresh=0.0, weight=0.5, max_iterations=100, tolerance=1e-6,
+                 xyz_dist_thresh=None, rpy_dist_thresh=None):
         self.enabled = enabled
         self.dist_thresh = dist_thresh
         self.weight = weight
         self.max_iterations = max_iterations
         self.tolerance = tolerance
+        self.xyz_dist_thresh = xyz_dist_thresh
+        self.rpy_dist_thresh = rpy_dist_thresh
 
     def c(self):
         return SnapParamsC(int(bool(self.enabled)), float(self.dist_thresh), float(self.weight),
                            IkParamsC(int(self.max_iterations), float(self.tolerance)))
+
+    def new_kinds(self):
+        """whether SNAP_TO_XYZ or SNAP_TO_RPY is on"""
+        return self.xyz_dist_thresh is not None or self.rpy_dist_thresh is not None
+
+    def kinds(self):
+        """(enabled (3,), dist_thresh (3,)) by SNAP_* kind"""
+        en = [self.rpy_dist_thresh is not None, self.xyz_dist_thresh is not None, bool(self.enabled)]
+        th = [0.0 if self.rpy_dist_thresh is None else float(self.rpy_dist_thresh),
+              0.0 if self.xyz_dist_thresh is None else float(self.xyz_dist_thresh), float(self.dist_thresh)]
+        return en, th
+
+    def c_kinds(self):
+        en, th = self.kinds()
+        k = SnapKindsC()
+        for i in range(3):
+            k.enabled[i] = int(en[i])
+            k.dist_thresh[i] = th[i]
+        k.ik = IkParamsC(int(self.max_iterations), float(self.tolerance))
+        return SnapsParamsC(k, float(self.weight))
 
 
 def gpu_lib():
@@ -191,6 +231,7 @@ def gpu_lib():
         L.smplgpu_goal_heuristics_dev.argtypes = [vp, vp, i, i, vp]
         L.smplgpu_planning_frame_fk.argtypes = [vp, dp, i, dp]
         L.smplgpu_planning_link_ik.argtypes = [vp, dp, dp, i, C.POINTER(IkParamsC), dp, bp, ip]
+        L.smplgpu_planning_link_ik_position.argtypes = [vp, dp, dp, i, C.POINTER(IkParamsC), dp, bp, ip]
         L.smplgpu_is_mprim_edges_valid.argtypes = [vp, dp, ip, i, dp, i, bp, ip]
         L.smplgpu_is_indexed_edges_valid.argtypes = [vp, dp, i, ip, ip, i, bp, ip]
         L.smplgpu_set_precision_mode.argtypes = [vp, i]
@@ -266,6 +307,10 @@ def host_lib():
                                                     C.POINTER(GoalC), c_int32_p, C.c_int, C.c_int, c_int32_p, c_int32_p,
                                                     C.c_int, c_double_p, c_double_p, C.POINTER(SnapParamsC),
                                                     C.POINTER(C.c_int64), c_int32_p]
+        H.smplhost_plan_batch_snaps.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(PlanParamsC), c_double_p,
+                                                C.POINTER(GoalC), c_int32_p, C.c_int, C.c_int, c_int32_p, c_int32_p,
+                                                C.c_int, c_double_p, c_double_p, C.POINTER(SnapsParamsC),
+                                                C.POINTER(C.c_int64), c_int32_p]
         H.smplhost_shortcut_paths.argtypes = [vp, C.c_int, c_uint8_p, c_double_p, c_int32_p, C.c_int, C.c_int, c_int32_p,
                                               c_int32_p, c_double_p]
         H.smplhost_interpolate_paths.argtypes = [vp, vp, c_double_p, c_int32_p, C.c_int, c_double_p, C.c_int, c_int32_p,
@@ -675,8 +720,12 @@ class GpuContext:
 
     def planning_link_ik(self, poses, seeds, max_iterations=100, tolerance=1e-6):
         """smplgpu_planning_link_ik: the planning link's IK for target-offset poses (n, 6) x y z roll pitch yaw,
-        seeded at seeds (n, dof).  Returns (q (n, dof), ok (n,) bool, iterations (n,))."""
-        poses = np.ascontiguousarray(poses, dtype=np.float64).reshape(-1, 6)
+        seeded at seeds (n, dof).  Targets of shape (n, 3) (positions) take the position-only IK,
+        smplgpu_planning_link_ik_position, whose answers leave the orientation free.
+        Returns (q (n, dof), ok (n,) bool, iterations (n,))."""
+        poses = np.ascontiguousarray(poses, dtype=np.float64)
+        width = 3 if poses.shape[-1] == 3 else 6
+        poses = poses.reshape(-1, width)
         seeds = self._q(seeds)
         if len(seeds) != len(poses):
             raise ValueError("%d poses, %d seeds" % (len(poses), len(seeds)))
@@ -685,8 +734,8 @@ class GpuContext:
         ok = np.zeros(n, np.uint8)
         it = np.zeros(n, np.int32)
         prm = IkParamsC(int(max_iterations), float(tolerance))
-        self._ck(self.L.smplgpu_planning_link_ik(self.h, _dp(poses), _dp(seeds), n, C.byref(prm), _dp(q), _bp(ok),
-                                                 _ip(it)), "planning_link_ik")
+        f = self.L.smplgpu_planning_link_ik if width == 6 else self.L.smplgpu_planning_link_ik_position
+        self._ck(f(self.h, _dp(poses), _dp(seeds), n, C.byref(prm), _dp(q), _bp(ok), _ip(it)), "planning_link_ik")
         return q, ok.astype(bool), it
 
 
@@ -908,8 +957,10 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
     reached_goal, the index in the query's set of the record its path reaches (-1 when unsolved).
     `ctx` may be a list of contexts (same GPU, same scene): one planner thread per context
     (smplhost_plan_batch_multi), max_concurrent is then per context.
-    snap: SnapParams -- the snap-to-goal action, through smplhost_plan_batch_snap (position goals become XYZ goal
-    records); the stats then also hold ik_attempted / ik_converged."""
+    snap: SnapParams -- the snap-to-goal actions, through smplhost_plan_batch_snap (position goals become XYZ goal
+    records), or smplhost_plan_batch_snaps when SNAP_TO_XYZ or SNAP_TO_RPY is on; the stats then also hold
+    ik_attempted / ik_converged (totals over the kinds) and, per kind name of SNAP_KIND_NAMES, ik_attempted_<kind> /
+    ik_converged_<kind>."""
     H = host_lib()
     dof = tables.dof
     starts = np.ascontiguousarray(starts, dtype=np.float64).reshape(-1, dof)
@@ -957,9 +1008,18 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
     stats = np.zeros(12)
     pstates = np.zeros((nq, max_path, dof), np.float64) if want_states else None
     ps_ptr = _dp(pstates) if want_states else None
-    counters = np.zeros(2, np.int64)
+    counters = np.zeros(6, np.int64)
     reached = np.full(nq, -1, np.int32)
-    if offsets is not None:
+    if snap is not None and snap.new_kinds():
+        ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
+        arr = (C.c_void_p * len(ctxs))(*[c.h for c in ctxs])
+        sp = snap.c_kinds()
+        off = offsets if offsets is not None else np.arange(nq + 1, dtype=np.int32)
+        r = H.smplhost_plan_batch_snaps(arr, len(ctxs), C.byref(P), _dp(starts), goals.ctypes.data_as(C.POINTER(GoalC)),
+                                        _ip(off), nq, int(max_concurrent), _ip(summary), _ip(paths), int(max_path),
+                                        _dp(stats), ps_ptr, C.byref(sp), counters.ctypes.data_as(C.POINTER(C.c_int64)),
+                                        _ip(reached))
+    elif offsets is not None:
         ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
         arr = (C.c_void_p * len(ctxs))(*[c.h for c in ctxs])
         sp = snap.c() if snap is not None else None
@@ -1003,7 +1063,12 @@ def plan_batch(ctx, scene, tables, params, starts, goals, max_concurrent=64, max
               bfs_runs=int(stats[6]), edges_resolved_f64=int(stats[7]), setup_seconds=float(stats[8]),
               max_wait_seconds=float(stats[9]), n_threads=int(n_threads))
     if snap is not None:
-        st.update(ik_attempted=int(counters[0]), ik_converged=int(counters[1]))
+        if not snap.new_kinds():   # the two-counter entry points: every solve is SNAP_TO_XYZ_RPY's
+            counters[2 * SNAP_XYZ_RPY:2 * SNAP_XYZ_RPY + 2] = counters[:2]
+            counters[:2] = 0
+        st.update(ik_attempted=int(counters[0::2].sum()), ik_converged=int(counters[1::2].sum()))
+        for k, name in enumerate(SNAP_KIND_NAMES):
+            st.update({"ik_attempted_" + name: int(counters[2 * k]), "ik_converged_" + name: int(counters[2 * k + 1])})
     return out, st
 
 

@@ -39,6 +39,7 @@ struct IkScratch
     double A[21];                    // lower triangle of J J^T + lambda^2 I, row by row
     double x[6];
     double q[MAX_DOF];
+    double tp[3];                    // lattice_snap_kernel's SNAP_TO_RPY target position
 };
 
 // The rotation vector (axis * angle, angle in [0, pi]) of the rotation matrix E.  v = (E21 - E12, E02 - E20,
@@ -81,10 +82,16 @@ __device__ __forceinline__ void rotation_vector(const double* E, double* w)
 }
 
 // The IK of one problem by one warp, seeded at S.q (set and __syncwarp'ed by the caller); the answer is left in S.q.
+// ROWS = 6: the full pose (tp, tR).  ROWS = 3: the position alone (SNAP_TO_XYZ; oracle/snap_kinds/snap_kinds_lattice.cpp
+// planningLinkIkPosition): e = tp - pt, the 3 x dof position block of J, a 3 x 3 Cholesky, converged when the three
+// position rows are within the tolerance; tR is not read and the orientation is free.
 // Returns converged (warp-uniform); *iterations = steps taken.
+template <int ROWS>
 __device__ bool ik_warp(const DevModel* __restrict__ M, const double* tp, const double* tR, int max_iterations,
                         double tolerance, IkScratch& S, int lane, int* iterations)
 {
+    static_assert(ROWS == 6 || ROWS == 3, "full pose or position only");
+    constexpr int NA = ROWS * (ROWS + 1) / 2;   // entries of the lower triangle of J J^T
     const int dof = M->dof, nseg = M->n_segments;
     for (int k = lane; k < 6 * MAX_DOF; k += 32) {
         (&S.J[0][0])[k] = 0.0;   // variables beyond the chain keep zero columns
@@ -113,19 +120,22 @@ __device__ bool ik_warp(const DevModel* __restrict__ M, const double* tp, const 
         // error (every lane, the same values)
         KFrame f;
         kframe_mul(Tk, S.pre[nseg], f);
-        double pt[3], e[6], E[9];
+        double pt[3], e[6];
         for (int i = 0; i < 3; ++i) {
             pt[i] = (f.M[3 * i] * M->xyz_offset[0] + f.M[3 * i + 1] * M->xyz_offset[1] + f.M[3 * i + 2] * M->xyz_offset[2]) + f.p[i];
             e[i] = tp[i] - pt[i];
         }
-        for (int i = 0; i < 3; ++i) {
-            for (int j = 0; j < 3; ++j) {
-                E[3 * i + j] = (tR[3 * i] * f.M[3 * j] + tR[3 * i + 1] * f.M[3 * j + 1]) + tR[3 * i + 2] * f.M[3 * j + 2];
+        if (ROWS == 6) {
+            double E[9];
+            for (int i = 0; i < 3; ++i) {
+                for (int j = 0; j < 3; ++j) {
+                    E[3 * i + j] = (tR[3 * i] * f.M[3 * j] + tR[3 * i + 1] * f.M[3 * j + 1]) + tR[3 * i + 2] * f.M[3 * j + 2];
+                }
             }
+            rotation_vector(E, e + 3);
         }
-        rotation_vector(E, e + 3);
         bool conv = true;
-        for (int i = 0; i < 6; ++i) {
+        for (int i = 0; i < ROWS; ++i) {
             conv = conv && fabs(e[i]) <= tolerance;
         }
         if (conv || it == max_iterations) {
@@ -159,7 +169,7 @@ __device__ bool ik_warp(const DevModel* __restrict__ M, const double* tp, const 
         }
         __syncwarp();
         // J J^T + lambda^2 I: entry (r, c), c <= r, by lane r (r + 1) / 2 + c
-        if (lane < 21) {
+        if (lane < NA) {
             int r = 0;
             while ((r + 1) * (r + 2) / 2 <= lane) ++r;
             const int c = lane - r * (r + 1) / 2;
@@ -172,14 +182,14 @@ __device__ bool ik_warp(const DevModel* __restrict__ M, const double* tp, const 
         __syncwarp();
         // Cholesky and the two triangular solves
         if (lane == 0) {
-            double L[6][6], y[6];
-            for (int j = 0; j < 6; ++j) {
+            double L[ROWS][ROWS], y[ROWS];
+            for (int j = 0; j < ROWS; ++j) {
                 double d = S.A[j * (j + 1) / 2 + j];
                 for (int k = 0; k < j; ++k) {
                     d = d - L[j][k] * L[j][k];
                 }
                 L[j][j] = sqrt(d);
-                for (int i = j + 1; i < 6; ++i) {
+                for (int i = j + 1; i < ROWS; ++i) {
                     double t = S.A[i * (i + 1) / 2 + j];
                     for (int k = 0; k < j; ++k) {
                         t = t - L[i][k] * L[j][k];
@@ -187,16 +197,16 @@ __device__ bool ik_warp(const DevModel* __restrict__ M, const double* tp, const 
                     L[i][j] = t / L[j][j];
                 }
             }
-            for (int i = 0; i < 6; ++i) {
+            for (int i = 0; i < ROWS; ++i) {
                 double t = e[i];
                 for (int k = 0; k < i; ++k) {
                     t = t - L[i][k] * y[k];
                 }
                 y[i] = t / L[i][i];
             }
-            for (int i = 5; i >= 0; --i) {
+            for (int i = ROWS - 1; i >= 0; --i) {
                 double t = y[i];
-                for (int k = i + 1; k < 6; ++k) {
+                for (int k = i + 1; k < ROWS; ++k) {
                     t = t - L[k][i] * S.x[k];
                 }
                 S.x[i] = t / L[i][i];
@@ -206,7 +216,7 @@ __device__ bool ik_warp(const DevModel* __restrict__ M, const double* tp, const 
         // the step, variable `lane`
         if (lane < dof) {
             double dq = 0.0;
-            for (int r = 0; r < 6; ++r) {
+            for (int r = 0; r < ROWS; ++r) {
                 dq = dq + S.J[r][lane] * S.x[r];
             }
             double nq = S.q[lane] + dq;
@@ -221,7 +231,8 @@ __device__ bool ik_warp(const DevModel* __restrict__ M, const double* tp, const 
     }
 }
 
-// smplgpu_planning_link_ik: problem k = warp k
+// smplgpu_planning_link_ik (ROWS = 6) and smplgpu_planning_link_ik_position (ROWS = 3): problem k = warp k
+template <int ROWS>
 __global__ void __launch_bounds__(32 * IK_WARPS)
 planning_link_ik_kernel(const DevModel* __restrict__ M, const IkTarget* __restrict__ targets,
                         const double* __restrict__ seeds, int n, int max_iterations, double tolerance,
@@ -240,7 +251,7 @@ planning_link_ik_kernel(const DevModel* __restrict__ M, const IkTarget* __restri
     }
     __syncwarp();
     int it = 0;
-    const bool conv = ik_warp(M, targets[k].p, targets[k].R, max_iterations, tolerance, S, lane, &it);
+    const bool conv = ik_warp<ROWS>(M, targets[k].p, targets[k].R, max_iterations, tolerance, S, lane, &it);
     if (lane < dof) {
         q_out[(size_t)k * dof + lane] = S.q[lane];
     }
@@ -267,40 +278,60 @@ __device__ __forceinline__ int nearest_goal_record(const LatticeGoal* __restrict
     return best;
 }
 
-// Round, step 1b with snaps enabled (between lattice_gen_kernel and the edge kernels): a warp per expansion.  The snap
-// is active when the parent's metric goal distance (the quantity of the short-distance switch) is within the
-// threshold; its target is the record of the slot's goal set nearest to the parent's target-offset position
-// (nearest_goal_record), and its action -- an IK solution for that record's pose seeded at the parent (XYZ and XYZ_RPY
-// records), or the angles of a JOINT_STATE record -- becomes word 0's edge when it exists and is within the joint
-// limits.
-// lattice_gen_kernel left word 0 an inactive zero-length edge.  counters[0] / [1]: IK solves run / converged.
-__global__ void __launch_bounds__(32 * IK_WARPS)
+// Round, step 1b with snaps enabled (between lattice_gen_kernel and the edge kernels): a warp per (expansion, enabled
+// snap kind); kind index k fills successor word k (B.snap_kind[k]: SMPLGPU_SNAP_RPY, _XYZ, _XYZ_RPY in that order).  A
+// kind is active when the parent's metric goal distance (the quantity of the short-distance switch) is within its
+// threshold.  Every kind of an expansion aims at the same record: the one of the slot's goal set nearest to the
+// parent's target-offset position (nearest_goal_record).  Its action, seeded at the parent:
+//   SNAP_TO_XYZ_RPY  (XYZ, XYZ_RPY, JOINT_STATE records) an IK solution for the record's full pose, or a joint
+//                    record's angles
+//   SNAP_TO_XYZ      (XYZ, XYZ_RPY records) a position-only IK solution for the record's goal position
+//   SNAP_TO_RPY      (XYZ_RPY records) an IK solution for the parent's own target-offset position and the record's
+//                    rotation: the orientation turned in place
+// A kind that does not apply to the record's type produces nothing.  The action becomes the word's edge when it exists
+// and is within the joint limits.  lattice_gen_kernel left the snap words inactive zero-length edges.
+// counters[2 kind] / [2 kind + 1]: IK solves of that kind run / converged.
+// With both IK forms inlined the kernel spills under ptxas's default cap of 128 registers; a minimum of one block per
+// SM lifts the cap (152 registers, no spills; DESIGN.md section 4).
+__global__ void __launch_bounds__(32 * IK_WARPS, 1)
 lattice_snap_kernel(const DevModel* __restrict__ M, LatticeBank B, const int* __restrict__ slot,
                     const int* __restrict__ parent, int n, double* __restrict__ q1, uint8_t* __restrict__ active,
                     unsigned long long* counters)
 {
     __shared__ IkScratch sS[IK_WARPS];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int i = (int)blockIdx.x * IK_WARPS + warp;
+    const int w = (int)blockIdx.x * IK_WARPS + warp;
+    const int i = w / B.snap, word = w - i * B.snap;
     if (i >= n) {
         return;
     }
+    const int kind = B.snap_kind[word];
     const int s = slot[i], p = parent[i];
     const double goal_dist = (double)B.gdist[(size_t)s * B.cap + p] * B.res;
-    if (!(goal_dist <= B.snap_thresh)) {
+    if (!(goal_dist <= B.snap_thresh[kind])) {
         return;
     }
     IkScratch& S = sS[warp];
     const int dof = M->dof;
+    const double* a = B.q + ((size_t)s * B.cap + p) * dof;
     const LatticeGoal* set = B.goal + (size_t)s * SMPLGPU_MAX_GOAL_SET;
     const int n_goals = B.n_goals[s];
     int target = 0;
-    if (n_goals > 1) {
+    if (n_goals > 1 || kind == SMPLGPU_SNAP_RPY) {
         double pose[6];
-        planning_frame_fk(M, B.q + ((size_t)s * B.cap + p) * dof, pose);   // the same in every lane
-        target = nearest_goal_record(set, n_goals, pose);
+        planning_frame_fk(M, a, pose);   // the same in every lane
+        if (n_goals > 1) {
+            target = nearest_goal_record(set, n_goals, pose);
+        }
+        if (lane < 3) {
+            S.tp[lane] = pose[lane];
+        }
     }
     const LatticeGoal* g = set + target;
+    if ((kind == SMPLGPU_SNAP_XYZ && g->type == SMPLGPU_GOAL_JOINT_STATE) ||
+        (kind == SMPLGPU_SNAP_RPY && g->type != SMPLGPU_GOAL_XYZ_RPY)) {
+        return;
+    }
     bool found = true;
     if (g->type == SMPLGPU_GOAL_JOINT_STATE) {
         if (lane < dof) {
@@ -309,21 +340,26 @@ lattice_snap_kernel(const DevModel* __restrict__ M, LatticeBank B, const int* __
         __syncwarp();
     } else {
         if (lane < dof) {
-            S.q[lane] = B.q[((size_t)s * B.cap + p) * dof + lane];
+            S.q[lane] = a[lane];
         }
         __syncwarp();
         int it = 0;
-        found = ik_warp(M, g->xyz, g->R, B.ik_max_iterations, B.ik_tolerance, S, lane, &it);
+        if (kind == SMPLGPU_SNAP_XYZ) {
+            found = ik_warp<3>(M, g->xyz, g->R, B.ik_max_iterations, B.ik_tolerance, S, lane, &it);
+        } else {
+            found = ik_warp<6>(M, kind == SMPLGPU_SNAP_RPY ? S.tp : g->xyz, g->R, B.ik_max_iterations, B.ik_tolerance,
+                               S, lane, &it);
+        }
         if (lane == 0) {
-            atomicAdd(&counters[0], 1ull);
+            atomicAdd(&counters[2 * kind], 1ull);
             if (found) {
-                atomicAdd(&counters[1], 1ull);
+                atomicAdd(&counters[2 * kind + 1], 1ull);
             }
         }
     }
     // checkAction: joint limits first (the edge kernels that follow check the motion)
     const bool on = found && joint_limits_ok(M, S.q);
-    const size_t t = (size_t)i * B.stride;
+    const size_t t = (size_t)i * B.stride + word;
     if (on && lane < dof) {
         q1[t * dof + lane] = S.q[lane];
     }

@@ -61,10 +61,11 @@ struct LatticeBank
     const double* deltas;     // [n_prims][dof]
     const int* long_list;     // primitive indices in table order
     const int* short_list;
-    // the snap action (smplgpu_lattice_set_snap): snap = 1 makes word 0 of every expansion the snap, words 1.. the
-    // primitives; 0 = no snap word
+    // the snap actions (smplgpu_lattice_set_snaps): snap = the number of enabled kinds, which take words 0 .. snap-1
+    // of every expansion (word k is kind snap_kind[k]), the primitives the words after them; 0 = no snap word
     int snap;
-    double snap_thresh;
+    int snap_kind[3];          // SMPLGPU_SNAP_* of word k, in the order RPY, XYZ, XYZ_RPY
+    double snap_thresh[3];     // by SMPLGPU_SNAP_* kind
     int ik_max_iterations;
     double ik_tolerance;
 };
@@ -209,7 +210,8 @@ __device__ __forceinline__ bool lattice_is_goal(int dof, const LatticeGoal* __re
 }
 
 // Round, step 1: the edges of every expansion.  Thread (i, j): j-th active primitive of the state expansion i pops
-// (with snaps enabled word 0 is the snap's, which lattice_snap_kernel fills in, and word j the (j-1)-th primitive).
+// (with k snap kinds enabled words 0 .. k-1 are the snaps', which lattice_snap_kernel fills in, and word j the
+// (j-k)-th primitive).
 // Inactive positions and successors beyond a joint limit become zero-length edges (no waypoint, no work in the
 // edge kernels) and are flagged.
 __global__ void lattice_gen_kernel(const DevModel* __restrict__ M, LatticeBank B, const int* __restrict__ slot,

@@ -150,7 +150,7 @@ struct smplgpu_ctx
     unsigned long long* lat_resolved = nullptr;   // pinned, mapped: edges the rounds resolved in double (running total)
     bool lat_fused = false;                        // one kernel per round (lattice_round_kernel)
     int lat_prim_stride = 0;                       // successor words of the primitives (smplgpu_lattice_create)
-    unsigned long long* d_snap_counters = nullptr; // IK solves of the snap actions: run, converged
+    unsigned long long* d_snap_counters = nullptr; // IK solves of the snap actions: run, converged, per SMPLGPU_SNAP_* kind
     size_t lat_round_smem = 0;
     // smplgpu_expand_state: primitive table, page-locked record array + completion flag, arrival counter
     double* d_x1_deltas = nullptr; int x1_prims = -1; int x1_dof = 0;
@@ -3233,7 +3233,7 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
     LatticeBank& B = ctx->lat;
     B.stride = stride;
     ctx->lat_prim_stride = stride;
-    B.snap = 0;   // smplgpu_lattice_set_snap turns them on
+    B.snap = 0;   // smplgpu_lattice_set_snaps turns them on
     B.n_long = (int)long_list.size();
     B.n_short = (int)short_list.size();
     B.use_short_dist = p->use_short_dist ? 1 : 0;
@@ -3491,7 +3491,7 @@ int smplgpu_lattice_expand_submit(smplgpu_ctx* ctx, const int32_t* slot, const i
                                                                               ctx->d_stats);
     ++ctx->launches;
     if (B.snap) {
-        lattice_snap_kernel<<<(unsigned)((n + IK_WARPS - 1) / IK_WARPS), 32 * IK_WARPS, 0, ctx->stream>>>(
+        lattice_snap_kernel<<<(unsigned)(((size_t)n * B.snap + IK_WARPS - 1) / IK_WARPS), 32 * IK_WARPS, 0, ctx->stream>>>(
             ctx->d_model, B, in_slot, in_parent, n, dq1, dactive, ctx->d_snap_counters);
         ++ctx->launches;
     }
@@ -3564,20 +3564,22 @@ static bool bad_ik_params(const smplgpu_ik_params* p)
     return p->max_iterations < 1 || !(p->tolerance > 0.0);
 }
 
-int smplgpu_planning_link_ik(smplgpu_ctx* ctx, const double* pose6, const double* seeds, int n,
-                             const smplgpu_ik_params* params, double* q_out, uint8_t* ok, int32_t* iterations)
+// the batched IK of smplgpu_planning_link_ik (width 6: x y z roll pitch yaw) and smplgpu_planning_link_ik_position
+// (width 3: x y z); ROWS = the width
+static int planning_link_ik(smplgpu_ctx* ctx, int ROWS, const double* targets, const double* seeds, int n,
+                            const smplgpu_ik_params* params, double* q_out, uint8_t* ok, int32_t* iterations)
 {
     if (!ctx || n < 0 || !params) return SMPLGPU_ERR_INVALID;
     if (bad_ik_params(params)) return fail(ctx, SMPLGPU_ERR_INVALID, "IK: max_iterations < 1, or a tolerance that is not positive");
     if (!ctx->has_robot) return fail(ctx, SMPLGPU_ERR_STATE, "robot tables not set (smplgpu_set_robot)");
     if (n == 0) return 0;
-    if (!pose6 || !seeds || !q_out || !ok || !iterations) return fail(ctx, SMPLGPU_ERR_INVALID, "null pointer");
+    if (!targets || !seeds || !q_out || !ok || !iterations) return fail(ctx, SMPLGPU_ERR_INVALID, "null pointer");
     const int dof = ctx->h_model->dof;
-    std::vector<IkTarget> tg(n);
+    std::vector<IkTarget> tg(n);   // zero-filled: the position-only IK reads no rotation
     for (int k = 0; k < n; ++k) {
-        const double* P = pose6 + 6 * (size_t)k;
+        const double* P = targets + (size_t)ROWS * k;
         for (int a = 0; a < 3; ++a) tg[k].p[a] = P[a];
-        rpy_matrix(P[3], P[4], P[5], tg[k].R);
+        if (ROWS == 6) rpy_matrix(P[3], P[4], P[5], tg[k].R);
     }
     const size_t tb = (size_t)n * sizeof(IkTarget), qb = (size_t)n * dof * sizeof(double);
     const size_t ib = ((size_t)n * sizeof(int) + 7) / 8 * 8, ob = ((size_t)n + 7) / 8 * 8;
@@ -3591,7 +3593,8 @@ int smplgpu_planning_link_ik(smplgpu_ctx* ctx, const double* pose6, const double
     uint8_t* d_ok = base + tb + 2 * qb + ib;
     CU(cudaMemcpyAsync(d_tg, tg.data(), tb, cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaMemcpyAsync(d_seeds, seeds, qb, cudaMemcpyHostToDevice, ctx->stream));
-    planning_link_ik_kernel<<<(unsigned)((n + IK_WARPS - 1) / IK_WARPS), 32 * IK_WARPS, 0, ctx->stream>>>(
+    auto* kernel = ROWS == 6 ? planning_link_ik_kernel<6> : planning_link_ik_kernel<3>;
+    kernel<<<(unsigned)((n + IK_WARPS - 1) / IK_WARPS), 32 * IK_WARPS, 0, ctx->stream>>>(
         ctx->d_model, d_tg, d_seeds, n, params->max_iterations, params->tolerance, d_q, d_ok, d_it);
     ++ctx->launches;
     CU(cudaGetLastError());
@@ -3604,47 +3607,87 @@ int smplgpu_planning_link_ik(smplgpu_ctx* ctx, const double* pose6, const double
     return n_ok;
 }
 
+int smplgpu_planning_link_ik(smplgpu_ctx* ctx, const double* pose6, const double* seeds, int n,
+                             const smplgpu_ik_params* params, double* q_out, uint8_t* ok, int32_t* iterations)
+{
+    return planning_link_ik(ctx, 6, pose6, seeds, n, params, q_out, ok, iterations);
+}
+
+int smplgpu_planning_link_ik_position(smplgpu_ctx* ctx, const double* xyz, const double* seeds, int n,
+                                      const smplgpu_ik_params* params, double* q_out, uint8_t* ok, int32_t* iterations)
+{
+    return planning_link_ik(ctx, 3, xyz, seeds, n, params, q_out, ok, iterations);
+}
+
 int smplgpu_lattice_set_snap(smplgpu_ctx* ctx, const smplgpu_snap_params* p)
 {
     if (!ctx || !p) return SMPLGPU_ERR_INVALID;
-    if (std::isnan(p->dist_thresh) || p->dist_thresh < 0.0) return fail(ctx, SMPLGPU_ERR_INVALID, "snap threshold is NaN or negative");
+    smplgpu_snap_kinds k = {};
+    k.enabled[SMPLGPU_SNAP_XYZ_RPY] = p->enabled;
+    k.dist_thresh[SMPLGPU_SNAP_XYZ_RPY] = p->dist_thresh;
+    k.ik = p->ik;
+    return smplgpu_lattice_set_snaps(ctx, &k);
+}
+
+int smplgpu_lattice_set_snaps(smplgpu_ctx* ctx, const smplgpu_snap_kinds* p)
+{
+    if (!ctx || !p) return SMPLGPU_ERR_INVALID;
+    for (int k = 0; k < 3; ++k) {
+        if (std::isnan(p->dist_thresh[k]) || p->dist_thresh[k] < 0.0)
+            return fail(ctx, SMPLGPU_ERR_INVALID, "snap kind %d: threshold is NaN or negative", k);
+    }
     if (bad_ik_params(&p->ik)) return fail(ctx, SMPLGPU_ERR_INVALID, "IK: max_iterations < 1, or a tolerance that is not positive");
     if (!ctx->has_lat) return fail(ctx, SMPLGPU_ERR_STATE, "lattices not created (smplgpu_lattice_create)");
     for (int b = 0; b < SMPLGPU_EXPAND_BUFFERS; ++b) {
         if (ctx->lat_n[b] >= 0) return fail(ctx, SMPLGPU_ERR_STATE, "lattice buffer %d is in flight", b);
     }
-    const int snap = p->enabled ? 1 : 0;
+    int snap = 0, kind_of_word[3] = { 0, 0, 0 };
+    for (int k = 0; k < 3; ++k) {
+        if (p->enabled[k]) kind_of_word[snap++] = k;
+    }
     const int stride = ctx->lat_prim_stride + snap;
     if (stride > LATTICE_MAX_STRIDE)
-        return fail(ctx, SMPLGPU_ERR_LIMIT, "%d successors per expansion with the snap (limit %d)", stride, LATTICE_MAX_STRIDE);
+        return fail(ctx, SMPLGPU_ERR_LIMIT, "%d successors per expansion with %d snap kinds (limit %d)", stride, snap, LATTICE_MAX_STRIDE);
     if (snap && !ctx->d_snap_counters) {
-        CU(cudaMalloc(&ctx->d_snap_counters, 2 * sizeof(unsigned long long)));
-        CU(cudaMemset(ctx->d_snap_counters, 0, 2 * sizeof(unsigned long long)));
+        CU(cudaMalloc(&ctx->d_snap_counters, 6 * sizeof(unsigned long long)));
+        CU(cudaMemset(ctx->d_snap_counters, 0, 6 * sizeof(unsigned long long)));
     }
     CU(cudaStreamSynchronize(ctx->stream));
     LatticeBank& B = ctx->lat;
     B.snap = snap;
     B.stride = stride;
-    B.snap_thresh = p->dist_thresh;
+    for (int k = 0; k < 3; ++k) {
+        B.snap_kind[k] = kind_of_word[k];
+        B.snap_thresh[k] = p->dist_thresh[k];
+    }
     B.ik_max_iterations = p->ik.max_iterations;
     B.ik_tolerance = p->ik.tolerance;
     const int r = lattice_round_buffers(ctx);
     return r ? r : stride;
 }
 
-int smplgpu_lattice_snap_counters(smplgpu_ctx* ctx, int64_t counters[2])
+int smplgpu_lattice_snap_counters_by_kind(smplgpu_ctx* ctx, int64_t counters[6])
 {
     if (!ctx || !counters) return SMPLGPU_ERR_INVALID;
-    counters[0] = counters[1] = 0;
+    for (int k = 0; k < 6; ++k) counters[k] = 0;
     if (!ctx->d_snap_counters) return 0;
-    unsigned long long c[2];
+    unsigned long long c[6];
     CU(cudaMemcpyAsync(c, ctx->d_snap_counters, sizeof(c), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
-    counters[0] = (int64_t)c[0];
-    counters[1] = (int64_t)c[1];
+    for (int k = 0; k < 6; ++k) counters[k] = (int64_t)c[k];
     return 0;
 }
 
+int smplgpu_lattice_snap_counters(smplgpu_ctx* ctx, int64_t counters[2])
+{
+    if (!ctx || !counters) return SMPLGPU_ERR_INVALID;
+    int64_t c[6];
+    const int r = smplgpu_lattice_snap_counters_by_kind(ctx, c);
+    if (r) return r;
+    counters[0] = c[0] + c[2] + c[4];
+    counters[1] = c[1] + c[3] + c[5];
+    return 0;
+}
 ///////////////////////////////////////////////////////////////////////////////
 // lattice states: 16-bit coordinates on the wire
 ///////////////////////////////////////////////////////////////////////////////

@@ -61,7 +61,7 @@ BatchPlanner::BatchPlanner(smplgpu_ctx* ctx, const PlannerConfig& cfg, int max_c
             (cfg.short_flags[p] != 0 ? m_cost_short : m_cost_long).push_back((int)(1000 * w));
         }
     }
-    m_snap_words = cfg.snap ? 1 : 0;
+    m_snap_words = (cfg.snap[0] ? 1 : 0) + (cfg.snap[1] ? 1 : 0) + (cfg.snap[2] ? 1 : 0);
     m_snap_cost = (int)(1000 * cfg.snap_weight);
     m_stride = m_snap_words + std::max(n_long, cfg.use_short_dist ? n_short : 0);
 }
@@ -393,7 +393,7 @@ void BatchPlanner::expandOne(Query& Q)
 }
 
 // ARAStar::expand relaxations (arastar.cpp:531-568) over the successors the device returned for this query's
-// expansion, in primitive order (the snap first, when enabled): succ[j] = lattice id | goal flag, or -1 (inactive
+// expansion, in primitive order (the snaps first, when enabled): succ[j] = lattice id | goal flag, or -1 (inactive
 // action, joint limit, collision)
 void BatchPlanner::absorbOne(Query& Q, const int32_t* succ, const int32_t* h, int count)
 {
@@ -426,7 +426,7 @@ void BatchPlanner::absorbOne(Query& Q, const int32_t* succ, const int32_t* h, in
         sstate(Q, target);
         touch(Q, target, h[e]);
         SState& ss = Q.search[target];
-        const int k = e - m_snap_words;   // primitive index; -1 = the snap
+        const int k = e - m_snap_words;   // primitive index; negative = a snap
         const int edge_cost = k < 0 ? m_snap_cost : ((size_t)k < edge_costs.size() ? edge_costs[k] : 1000);
         const int new_cost = Q.search[Q.expanding].eg + edge_cost;
         if ((unsigned int)new_cost < ss.g) {   // int vs unsigned, compared as unsigned (arastar.cpp:545-548)
@@ -513,8 +513,8 @@ bool BatchPlanner::plan(const double* starts, const smplgpu_goal* goals, const i
         }
     }
     const long long resolved0 = smplgpu_expand_batch_resolved(m_ctx);
-    int64_t ik0[2] = { 0, 0 };
-    if (m_cfg.snap && smplgpu_lattice_snap_counters(m_ctx, ik0) < 0) return fail_dev();
+    int64_t ik0[6] = { 0, 0, 0, 0, 0, 0 };
+    if (m_snap_words && smplgpu_lattice_snap_counters_by_kind(m_ctx, ik0) < 0) return fail_dev();
     // a query creates at most (its expansions) x (successors per expansion) states besides the goal and the start
     const long long want_states = 2 + (long long)std::max(0, m_cfg.max_expansions) * std::max(1, m_stride);
     const int max_states = (int)std::min<long long>(want_states, 1LL << 26);
@@ -540,12 +540,14 @@ bool BatchPlanner::plan(const double* starts, const smplgpu_goal* goals, const i
         lp.max_states = max_states;
         int stride = smplgpu_lattice_create(m_ctx, &lp, n_slots);
         if (stride < 0) return fail_dev();
-        if (m_cfg.snap) {
-            smplgpu_snap_params sp;
-            sp.enabled = 1;
-            sp.dist_thresh = m_cfg.snap_dist_thresh;
-            sp.ik = m_cfg.ik;
-            stride = smplgpu_lattice_set_snap(m_ctx, &sp);
+        if (m_snap_words) {
+            smplgpu_snap_kinds sk;
+            for (int k = 0; k < 3; ++k) {
+                sk.enabled[k] = m_cfg.snap[k] ? 1 : 0;
+                sk.dist_thresh[k] = m_cfg.snap_dist_thresh[k];
+            }
+            sk.ik = m_cfg.ik;
+            stride = smplgpu_lattice_set_snaps(m_ctx, &sk);
             if (stride < 0) return fail_dev();
         }
         if (stride != m_stride) {
@@ -824,11 +826,13 @@ bool BatchPlanner::plan(const double* starts, const smplgpu_goal* goals, const i
                 m_stats.host_seconds);
     }
     m_stats.edges_resolved_f64 = smplgpu_expand_batch_resolved(m_ctx) - resolved0;
-    if (m_cfg.snap) {
-        int64_t ik1[2];
-        if (smplgpu_lattice_snap_counters(m_ctx, ik1) < 0) return fail_dev();
-        m_stats.ik_attempted = ik1[0] - ik0[0];
-        m_stats.ik_converged = ik1[1] - ik0[1];
+    if (m_snap_words) {
+        int64_t ik1[6];
+        if (smplgpu_lattice_snap_counters_by_kind(m_ctx, ik1) < 0) return fail_dev();
+        for (int k = 0; k < 3; ++k) {
+            m_stats.ik_attempted[k] = ik1[2 * k] - ik0[2 * k];
+            m_stats.ik_converged[k] = ik1[2 * k + 1] - ik0[2 * k + 1];
+        }
     }
     // nothing can be in flight here: a group's queries finish in absorb or expand, and a round is only submitted for
     // queries that are not done; drain defensively anyway

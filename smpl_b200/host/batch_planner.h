@@ -60,10 +60,11 @@ struct PlannerConfig
     int n_threads = 1;
     // fetch the joint values along every found path from the device (ManipLattice::extractPath)
     bool want_path_states = true;
-    // the SNAP_TO_XYZ_RPY action (smplgpu_lattice_set_snap): active within snap_dist_thresh metres of metric goal
-    // distance; it costs (int)(1000 * snap_weight) (the fork registers it with weight 0.5)
-    bool snap = false;
-    double snap_dist_thresh = 0.0;
+    // the snap actions SNAP_TO_RPY, SNAP_TO_XYZ and SNAP_TO_XYZ_RPY (smplgpu_lattice_set_snaps), by SMPLGPU_SNAP_*
+    // kind: each active within its own snap_dist_thresh metres of metric goal distance; every kind costs
+    // (int)(1000 * snap_weight) (the fork registers them with weight 0.5) and solves with the same IK parameters
+    bool snap[3] = { false, false, false };
+    double snap_dist_thresh[3] = { 0.0, 0.0, 0.0 };
     double snap_weight = 0.5;
     smplgpu_ik_params ik = { 100, 1e-6 };
 };
@@ -94,8 +95,8 @@ struct BatchStats
     double host_seconds = 0.0;     // everything else
     double setup_seconds = 0.0;    // of device_seconds: bank creation, BFS bank runs, setStart (per refill)
     double max_wait_seconds = 0.0; // longest single wait for an expansion batch
-    long long ik_attempted = 0;    // IK solves of the snap actions, and how many converged
-    long long ik_converged = 0;
+    long long ik_attempted[3] = { 0, 0, 0 };   // IK solves of the snap actions by SMPLGPU_SNAP_* kind, and how many
+    long long ik_converged[3] = { 0, 0, 0 };   // converged
 };
 
 class BatchPlanner
@@ -172,8 +173,8 @@ private:
     std::vector<double> m_prim_deltas;     // [n_prims][dof], converses included
     std::vector<uint8_t> m_prim_short;
     std::vector<int> m_cost_long, m_cost_short;   // edge cost of the j-th active long / short primitive (converses included)
-    int m_stride = 0;                      // successor words per expansion (the snap's first when enabled)
-    int m_snap_words = 0;                  // 1 with the snap action, else 0
+    int m_stride = 0;                      // successor words per expansion (the snaps' first when enabled)
+    int m_snap_words = 0;                  // the number of enabled snap kinds
     int m_snap_cost = 0;
     BatchStats m_stats;
 

@@ -1,6 +1,7 @@
 // Flat C entry points over the host-side C++ (model builder + adapters) so the
 // Python plumbing (tests, bench.py) can drive it with ctypes.  Declared in
 // include/smplhost.h.
+#include <algorithm>
 #include <array>
 #include <chrono>
 #include <cmath>
@@ -237,7 +238,7 @@ int smplhost_tables_pairs(smplhost_tables* h, int32_t* out, int max_pairs)
 // reached_goal
 static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const double* starts,
                           const smplgpu_goal* goals, int nq, int max_concurrent, int32_t* summary, int32_t* path_ids,
-                          int max_path, double* stats, double* path_states, const smplhost_snap_params* snap = nullptr,
+                          int max_path, double* stats, double* path_states, const smplhost_snaps_params* snaps = nullptr,
                           int64_t* counters = nullptr, const int32_t* goal_offsets = nullptr, int32_t* reached = nullptr)
 {
     if (!ctx || !p || nq < 0 || (nq > 0 && (!starts || !goals || !summary))) {
@@ -272,11 +273,13 @@ static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const
         cfg.origin[a] = p->origin[a];
         cfg.dims[a] = p->dims[a];
     }
-    if (snap && snap->enabled) {
-        cfg.snap = true;
-        cfg.snap_dist_thresh = snap->dist_thresh;
-        cfg.snap_weight = snap->weight;
-        cfg.ik = snap->ik;
+    if (snaps) {
+        for (int k = 0; k < 3; ++k) {
+            cfg.snap[k] = snaps->kinds.enabled[k] != 0;
+            cfg.snap_dist_thresh[k] = snaps->kinds.dist_thresh[k];
+        }
+        cfg.snap_weight = snaps->weight;
+        cfg.ik = snaps->kinds.ik;
     }
     smplhost::BatchPlanner planner(ctx, cfg, max_concurrent);
     std::vector<smplhost::QueryResult> out;
@@ -321,8 +324,10 @@ static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const
         stats[9] = s.max_wait_seconds;
     }
     if (counters) {
-        counters[0] = planner.stats().ik_attempted;
-        counters[1] = planner.stats().ik_converged;
+        for (int k = 0; k < 3; ++k) {
+            counters[2 * k] = planner.stats().ik_attempted[k];
+            counters[2 * k + 1] = planner.stats().ik_converged[k];
+        }
     }
     return 0;
 }
@@ -331,18 +336,18 @@ static int plan_batch_one(smplgpu_ctx* ctx, const smplhost_plan_params* p, const
 static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
                                const smplgpu_goal* goals, int nq, int max_concurrent_per_ctx, int32_t* summary,
                                int32_t* path_ids, int max_path, double* stats, double* path_states,
-                               const smplhost_snap_params* snap = nullptr, int64_t* counters = nullptr,
+                               const smplhost_snaps_params* snaps = nullptr, int64_t* counters = nullptr,
                                const int32_t* goal_offsets = nullptr, int32_t* reached = nullptr)
 {
     if (counters) {
-        counters[0] = counters[1] = 0;
+        std::fill(counters, counters + 6, 0);
     }
     if (n_ctx == 1) {
         return plan_batch_one(ctxs[0], p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path, stats,
-                              path_states, snap, counters, goal_offsets, reached);
+                              path_states, snaps, counters, goal_offsets, reached);
     }
     auto set_begin = [&](int i) { return goal_offsets ? goal_offsets[i] : i; };
-    std::vector<std::array<int64_t, 2>> ik(n_ctx, std::array<int64_t, 2>{ { 0, 0 } });
+    std::vector<std::array<int64_t, 6>> ik(n_ctx, std::array<int64_t, 6>{ { 0, 0, 0, 0, 0, 0 } });
     const int dof = p->dof;
     std::vector<int> rc(n_ctx, 0);
     std::vector<std::string> errs(n_ctx);
@@ -377,7 +382,7 @@ static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplho
             pt.n_threads = 1;
             rc[t] = plan_batch_one(ctxs[t], &pt, s.data(), g.data(), m, max_concurrent_per_ctx, sum.data(),
                                    path_ids ? paths.data() : nullptr, max_path, st[t].data(),
-                                   path_states ? pstates.data() : nullptr, snap, ik[t].data(), off.data(), got.data());
+                                   path_states ? pstates.data() : nullptr, snaps, ik[t].data(), off.data(), got.data());
             if (rc[t] != 0) {
                 errs[t] = g_err;   // thread-local: copy it out
                 return;
@@ -409,8 +414,7 @@ static int plan_batch_contexts(smplgpu_ctx* const* ctxs, int n_ctx, const smplho
     }
     if (counters) {
         for (int t = 0; t < n_ctx; ++t) {
-            counters[0] += ik[t][0];
-            counters[1] += ik[t][1];
+            for (int k = 0; k < 6; ++k) counters[k] += ik[t][k];
         }
     }
     if (stats) {
@@ -521,20 +525,44 @@ int smplhost_plan_batch_goals(smplgpu_ctx* const* ctxs, int n_ctx, const smplhos
                                stats, path_states);
 }
 
-// the checks of smplgpu_lattice_set_snap and the snap's cost weight
-static int check_snap_args(const smplhost_snap_params* snap)
+// the checks of smplgpu_lattice_set_snaps and the snaps' cost weight, before any query starts
+static int check_snaps_args(const smplhost_snaps_params* snaps)
 {
-    // the checks of smplgpu_lattice_set_snap, and the cost weight, before any query starts
-    if (std::isnan(snap->dist_thresh) || snap->dist_thresh < 0.0 || std::isnan(snap->weight) || snap->weight < 0.0 ||
-        snap->weight > 1e6) {
-        g_err = "smplhost_plan_batch_snap: snap threshold or weight is NaN, negative or too large";
+    if (std::isnan(snaps->weight) || snaps->weight < 0.0 || snaps->weight > 1e6) {
+        g_err = "smplhost_plan_batch_snaps: snap weight is NaN, negative or too large";
         return SMPLGPU_ERR_INVALID;
     }
-    if (snap->ik.max_iterations < 1 || !(snap->ik.tolerance > 0.0)) {
-        g_err = "smplhost_plan_batch_snap: IK max_iterations < 1, or a tolerance that is not positive";
+    for (int k = 0; k < 3; ++k) {
+        if (std::isnan(snaps->kinds.dist_thresh[k]) || snaps->kinds.dist_thresh[k] < 0.0) {
+            g_err = "smplhost_plan_batch_snaps: the threshold of snap kind " + std::to_string(k) + " is NaN or negative";
+            return SMPLGPU_ERR_INVALID;
+        }
+    }
+    if (snaps->kinds.ik.max_iterations < 1 || !(snaps->kinds.ik.tolerance > 0.0)) {
+        g_err = "smplhost_plan_batch_snaps: IK max_iterations < 1, or a tolerance that is not positive";
         return SMPLGPU_ERR_INVALID;
     }
     return 0;
+}
+
+// smplhost_snap_params as the SNAP_TO_XYZ_RPY kind alone
+static smplhost_snaps_params xyz_rpy_alone(const smplhost_snap_params* snap)
+{
+    smplhost_snaps_params s = {};
+    s.kinds.enabled[SMPLGPU_SNAP_XYZ_RPY] = snap->enabled;
+    s.kinds.dist_thresh[SMPLGPU_SNAP_XYZ_RPY] = snap->dist_thresh;
+    s.kinds.ik = snap->ik;
+    s.weight = snap->weight;
+    return s;
+}
+
+// counters[6] by kind -> counters[2] summed over the kinds
+static void counter_totals(const int64_t* by_kind, int64_t* counters)
+{
+    if (counters) {
+        counters[0] = by_kind[0] + by_kind[2] + by_kind[4];
+        counters[1] = by_kind[1] + by_kind[3] + by_kind[5];
+    }
 }
 
 int smplhost_plan_batch_snap(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
@@ -548,10 +576,14 @@ int smplhost_plan_batch_snap(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost
         g_err = "smplhost_plan_batch_snap: null snap parameters";
         return SMPLGPU_ERR_INVALID;
     }
-    r = check_snap_args(snap);
+    const smplhost_snaps_params snaps = xyz_rpy_alone(snap);
+    r = check_snaps_args(&snaps);
     if (r) return r;
-    return plan_batch_contexts(ctxs, n_ctx, p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path,
-                               stats, path_states, snap, counters);
+    int64_t by_kind[6] = { 0, 0, 0, 0, 0, 0 };
+    r = plan_batch_contexts(ctxs, n_ctx, p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path,
+                            stats, path_states, &snaps, by_kind);
+    counter_totals(by_kind, counters);
+    return r;
 }
 
 int smplhost_plan_batch_goal_sets(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p,
@@ -559,6 +591,24 @@ int smplhost_plan_batch_goal_sets(smplgpu_ctx* const* ctxs, int n_ctx, const smp
                                   int max_concurrent_per_ctx, int32_t* summary, int32_t* path_ids, int max_path,
                                   double* stats, double* path_states, const smplhost_snap_params* snap,
                                   int64_t* counters, int32_t* reached_goal)
+{
+    smplhost_snaps_params snaps;
+    if (snap) {
+        snaps = xyz_rpy_alone(snap);
+    }
+    int64_t by_kind[6] = { 0, 0, 0, 0, 0, 0 };
+    const int r = smplhost_plan_batch_snaps(ctxs, n_ctx, p, starts, goals, goal_offsets, nq, max_concurrent_per_ctx,
+                                            summary, path_ids, max_path, stats, path_states, snap ? &snaps : nullptr,
+                                            by_kind, reached_goal);
+    counter_totals(by_kind, counters);
+    return r;
+}
+
+int smplhost_plan_batch_snaps(smplgpu_ctx* const* ctxs, int n_ctx, const smplhost_plan_params* p, const double* starts,
+                              const smplgpu_goal* goals, const int32_t* goal_offsets, int nq,
+                              int max_concurrent_per_ctx, int32_t* summary, int32_t* path_ids, int max_path,
+                              double* stats, double* path_states, const smplhost_snaps_params* snaps,
+                              int64_t* counters, int32_t* reached_goal)
 {
     if (nq < 0 || (nq > 0 && (!goal_offsets || !reached_goal))) {
         g_err = "smplhost_plan_batch_goal_sets: bad argument";
@@ -579,15 +629,15 @@ int smplhost_plan_batch_goal_sets(smplgpu_ctx* const* ctxs, int n_ctx, const smp
     }
     int r = check_goal_args(ctxs, n_ctx, p, goals, nq > 0 ? goal_offsets[nq] : 0);
     if (r) return r;
-    if (snap) {
-        r = check_snap_args(snap);
+    if (snaps) {
+        r = check_snaps_args(snaps);
         if (r) return r;
     }
     if (counters) {
-        counters[0] = counters[1] = 0;
+        std::fill(counters, counters + 6, 0);
     }
     return plan_batch_contexts(ctxs, n_ctx, p, starts, goals, nq, max_concurrent_per_ctx, summary, path_ids, max_path,
-                               stats, path_states, snap, counters, goal_offsets, reached_goal);
+                               stats, path_states, snaps, counters, goal_offsets, reached_goal);
 }
 
 struct smplhost_adapters

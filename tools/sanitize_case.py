@@ -45,6 +45,11 @@ pctx.probe_df_lookup_rate()
 ik_seeds = st + 0.05
 pctx.planning_link_ik(pctx.planning_frame_fk(st), ik_seeds)
 api.plan_batch(pctx, ps, pt, pp, st, g, max_concurrent=4, snap=api.SnapParams(dist_thresh=0.2))
+# the position-only IK kernel and a round chain with all three snap kinds
+pctx.planning_link_ik(pctx.planning_frame_fk(st)[:, :3], ik_seeds)
+rg = api.pose_goals(np.concatenate([g, np.zeros((len(g), 3))], axis=1), pp.xyz_tolerance, rpy_tolerance=0.05)
+api.plan_batch(pctx, ps, pt, pp, st, rg, max_concurrent=4,
+               snap=api.SnapParams(dist_thresh=0.2, xyz_dist_thresh=0.2, rpy_dist_thresh=0.2))
 # scene ingest (voxeliser + EDT) and the indexed-edge batch of path shortcutting
 ictx, it = api.setup_context(scenes.pr2_shelf_objects_scene())
 paths = [q[:12].copy(), q[20:40].copy()]
