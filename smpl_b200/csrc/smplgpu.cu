@@ -60,6 +60,7 @@ struct smplgpu_ctx
     int v32_slots = 0, v32_ptrees = 0;
     double e_pos = 0.0, eps_cells = 0.0;
     Grid32 grid32{};
+    double fk32_origin[3] = { 0.0, 0.0, 0.0 };   // metres of the model's coordinate 0 (fk_centers32_kernel)
     int* d_prim = nullptr; size_t prim_cap = 0;     // bytes; primitive ids of two chunks in flight
     double* d_deltas = nullptr; size_t deltas_cap = 0;
     int* d_unc_list = nullptr; size_t unc_cap = 0;  // ints
@@ -615,15 +616,32 @@ static void fold_constant_links(const DevModel& m, DevModel& F)
 
 // Builds the shared-memory blob of validity32.cuh and the error bounds that certify it.
 //
-// Error model (u = 2^-24, all norms Euclidean; R = rotation part, t = translation part of a link transform):
+// The blob is in GRID UNITS: with s = inv_res and o the grid's (ox, oy, oz), every link-origin translation, sphere
+// centre and radius is scaled by s, the rotation blocks are left as they are, and the base transform of a root link
+// (world <- root, [R_b | t_b]) becomes [R_b | s (t_b - o) - 1 - K], K the whole cell of the first root link's origin.
+// The chain then yields c - K, where c = s (x - o) - 1 for a centre x in metres is the grid coordinate whose
+// round-to-nearest is the reference's cell; the lookup adds K back in its integer index step (validity32.cuh:
+// lookup32).  With K taken out, the chain's translations are lengths along the robot, not distances from the grid
+// origin, which keeps the rounding terms 7u tn below small.  A
+// moving prismatic joint keeps q in joint units: its axis slot holds s times the third origin column.
+//
+// Error model (u = 2^-24, all norms Euclidean, all lengths in cells; R = rotation part, t = translation part of a
+// link transform):
 //   joint transform J(q):  ||dR_J||_F <= 3.5u (constant), 40u (axis-aligned revolute: sincosf <= 2 ulp, hi/lo
-//                          angle split, 2 roundings per entry), 80u (general axis); ||dt_J|| <= u ||t_J|| (+ 4u |q|max
+//                          angle split, 2 roundings per entry), 80u (general axis); ||dt_J|| <= u ||t_J|| (+ 4u s |q|max
 //                          for a prismatic joint, whose low part of q is dropped)
+//   base transform:        ||dR_B||_F <= 3.5u, ||dt_B|| <= u ||t_B||, t_B = s (t_b - o) - 1 - K (formed in double, rounded
+//                          once to float): the world -> grid map's own rounding is this one term
 //   product T = P J:       ||dR_T||_F <= ||dR_P||_F + ||dR_J||_F + 12u                  (||R|| = 1)
 //                          ||dt_T||   <= ||dt_P|| + ||dR_P||_F ||t_J|| + ||dt_J|| + 7u tn,   tn >= ||t_T||
-//   centre  x = T c:       ||dx||     <= ||dt_T|| + ||dR_T||_F ||c|| + 7u (tn + ||c||) + u ||c||
-// E_pos = 1.5 * max over nodes.  Grid coordinate g = inv_res (x - o) + 1/2 evaluated in float:
-//   |dg| <= inv_res E_pos + u (inv_res max|o| + 4 (max_dim + 4)) + 1e-7.
+//   centre  c = T y:       ||dc||     <= ||dt_T|| + ||dR_T||_F ||y|| + 7u (tn + ||y||) + u ||y||
+// E = 1.5 * max over nodes bounds |c_f32 - c_f64| (the factor covers the double chain's own rounding).  The lookup
+// forms its cell and remainder exactly (lookup32) and compares the remainder against 1/2 - eps in float, which rounds
+// by at most 2^-26; the reference rounds its double grid coordinate by ~2^-53 |c|.  Both sit in the 1e-7 of
+// eps_cells = E + 1e-7.  Since E >= 10.5u (tn + ||y||) >= 10.5u |c - K|, eps_cells < 0.125 also means |c - K| < 2^21
+// for every centre the kernels evaluate (joints beyond V32_MAX_ANGLE or q_lin_max go to the double path first), where
+// lookup32's rounding is exact; the check of that below only restates it.  |K| < 2^21 keeps the index in int range.  The pair tests compare squared
+// distances in cells, which scale with s^2 on both sides, with the tolerance 2.5 E (d + r) + 2e-6 (d^2 + r^2).
 static int build_model32(smplgpu_ctx* ctx)
 {
     ctx->has_model32 = false;
@@ -675,7 +693,18 @@ static int build_model32(smplgpu_ctx* ctx)
         }
     }
 
-    // ---- error bounds ----
+    // ---- error bounds (cells) ----
+    const double sc = ctx->grid.inv_res;
+    const double go[3] = { ctx->grid.ox, ctx->grid.oy, ctx->grid.oz };
+    // whole-cell offset K: the grid cell of the first root link's origin (validity32.cuh: Grid32)
+    double K[3] = { 0.0, 0.0, 0.0 };
+    for (int l = 0; l < nl; ++l) {
+        if (m.link_parent[l] < 0) {
+            for (int i = 0; i < 3; ++i) K[i] = std::nearbyint(sc * (m.link_base[l][4 * i + 3] - go[i]) - 1.0);
+            break;
+        }
+    }
+    auto base_t = [&](int l, int i) { return sc * (m.link_base[l][4 * i + 3] - go[i]) - 1.0 - K[i]; };
     std::vector<double> EF(nl), Et(nl), tn(nl);
     double q_lin_max = 0.0;
     for (int v = 0; v < m.dof; ++v) {
@@ -685,29 +714,29 @@ static int build_model32(smplgpu_ctx* ctx)
             q_lin_max = std::max(q_lin_max, lim + 1.0);
         }
     }
-    double e_max = 0.0;
+    const double q_lin_cells = sc * q_lin_max;
+    double e_max = 0.0, c_max = 0.0;
     for (int l = 0; l < nl; ++l) {
         const int fn = m.link_joint[l];
         const bool moving = m.link_var[l] >= 0;
         const double* o = m.link_origin[l];
-        const double to[3] = { o[3], o[7], o[11] };
+        const double to[3] = { sc * o[3], sc * o[7], sc * o[11] };
         double EF_J, Et_J, tJ;
         if (!moving || fn == 0) {
             EF_J = 3.5 * u;
-            tJ = norm3(to) + ((fn == 5) ? std::fabs(m.link_const[l]) : 0.0);
+            tJ = norm3(to) + ((fn == 5) ? sc * std::fabs(m.link_const[l]) : 0.0);
             Et_J = u * tJ;
         } else if (fn <= 3) {
             EF_J = 40.0 * u; tJ = norm3(to); Et_J = u * tJ;
         } else if (fn == 4) {
             EF_J = 80.0 * u; tJ = norm3(to); Et_J = u * tJ;
         } else {
-            EF_J = 3.5 * u; tJ = norm3(to) + q_lin_max; Et_J = u * tJ + 4.0 * u * q_lin_max;
+            EF_J = 3.5 * u; tJ = norm3(to) + q_lin_cells; Et_J = u * tJ + 4.0 * u * q_lin_cells;
         }
         double EF_P, Et_P, tn_P;
         const int p = m.link_parent[l];
         if (p < 0) {
-            const double* b = m.link_base[l];
-            const double tb[3] = { b[3], b[7], b[11] };
+            const double tb[3] = { base_t(l, 0), base_t(l, 1), base_t(l, 2) };
             EF_P = 3.5 * u; tn_P = norm3(tb); Et_P = u * tn_P;
         } else {
             EF_P = EF[p]; Et_P = Et[p]; tn_P = tn[p];
@@ -716,18 +745,17 @@ static int build_model32(smplgpu_ctx* ctx)
         tn[l] = tn_P + tJ;
         Et[l] = Et_P + EF_P * tJ + Et_J + 7.0 * u * tn[l];
         for (int i = link_nbeg[l]; i < link_nend[l]; ++i) {
-            const double cn = norm3(m.node_center[orig_of[i]]);
+            const double cn = sc * norm3(m.node_center[orig_of[i]]);
             e_max = std::max(e_max, Et[l] + EF[l] * cn + 7.0 * u * (tn[l] + cn) + u * cn);
+            c_max = std::max(c_max, tn[l] + cn);
         }
     }
-    const double e_pos = 1.5 * e_max;
-    const double inv_res = ctx->grid.inv_res;
-    const int max_dim = std::max(ctx->grid.nx, std::max(ctx->grid.ny, ctx->grid.nz));
-    const double o_max = std::max(std::fabs(ctx->grid.ox), std::max(std::fabs(ctx->grid.oy), std::fabs(ctx->grid.oz)));
-    const double eps_cells = inv_res * e_pos + u * (inv_res * o_max + 4.0 * (max_dim + 4)) + 1e-7;
-    ctx->e_pos = e_pos;
+    const double e_cells = 1.5 * e_max;
+    const double eps_cells = e_cells + 1e-7;
+    ctx->e_pos = e_cells / sc;   // metres
     ctx->eps_cells = eps_cells;
-    if (!(eps_cells < 0.125)) {
+    const double k_max = std::max(std::fabs(K[0]), std::max(std::fabs(K[1]), std::fabs(K[2])));
+    if (!(eps_cells < 0.125) || !(c_max < 0x1p21) || !(k_max < 0x1p21)) {
         return 0; // bound too loose for this resolution: the double path handles everything
     }
 
@@ -787,9 +815,9 @@ static int build_model32(smplgpu_ctx* ctx)
     h.off_pair = w; w = align4(w + 4 * m.n_pairs);
     h.off_allowed = w; w = align4(w + 2 * m.n_allowed);
     h.words = w;
-    h.e_pos = (float)e_pos;
+    h.e_cells = (float)e_cells;
     h.eps_cells = (float)(eps_cells * 1.0000002);
-    h.pair_k = (float)(2.5 * e_pos);
+    h.pair_k = (float)(2.5 * e_cells);
     h.q_lin_max = (float)q_lin_max;
     std::vector<float>& B = ctx->h_blob;
     B.assign(w, 0.0f);
@@ -811,15 +839,18 @@ static int build_model32(smplgpu_ctx* ctx)
         BI[h.off_link_n + 2 * l] = link_nbeg[l];
         BI[h.off_link_n + 2 * l + 1] = link_nend[l];
         for (int k = 0; k < 12; ++k) {
-            B[h.off_origin + 12 * l + k] = (float)J[k];
-            B[h.off_base + 12 * l + k] = (float)m.link_base[l][k];
+            const bool t = k % 4 == 3;
+            B[h.off_origin + 12 * l + k] = (float)(t ? sc * J[k] : J[k]);
+            B[h.off_base + 12 * l + k] = (float)(t ? base_t(l, k / 4) : m.link_base[l][k]);
         }
-        for (int k = 0; k < 3; ++k) B[h.off_axis + 4 * l + k] = (float)m.link_axis[l][k];
+        for (int k = 0; k < 3; ++k) {
+            B[h.off_axis + 4 * l + k] = (float)(fn == 5 ? sc * J[4 * k + 2] : m.link_axis[l][k]);
+        }
     }
     for (int i = 0; i < n32; ++i) {
         const int node = orig_of[i];
-        for (int k = 0; k < 3; ++k) B[h.off_node_c + 4 * i + k] = (float)m.node_center[node][k];
-        B[h.off_node_c + 4 * i + 3] = (float)m.node_radius[node];
+        for (int k = 0; k < 3; ++k) B[h.off_node_c + 4 * i + k] = (float)(sc * m.node_center[node][k]);
+        B[h.off_node_c + 4 * i + 3] = (float)(sc * m.node_radius[node]);
         BI[h.off_node_i + 4 * i] = skip[i];
         BI[h.off_node_i + 4 * i + 1] = m.node_thresh[node];
         BI[h.off_node_i + 4 * i + 2] = roots_only ? ptree_of_root[node] : m.link_slot[m.node_link[node]];
@@ -886,8 +917,12 @@ static int build_model32(smplgpu_ctx* ctx)
     CU(cudaMemcpyAsync(ctx->d_blob, B.data(), (size_t)w * 4, cudaMemcpyHostToDevice, ctx->stream));
     ctx->blob_words = w;
     ctx->grid32.nx = ctx->grid.nx; ctx->grid32.ny = ctx->grid.ny; ctx->grid32.nz = ctx->grid.nz;
-    ctx->grid32.inv_res = (float)ctx->grid.inv_res;
-    ctx->grid32.ox = (float)ctx->grid.ox; ctx->grid32.oy = (float)ctx->grid.oy; ctx->grid32.oz = (float)ctx->grid.oz;
+    {
+        int magic;
+        memcpy(&magic, &ROUND_MAGIC, sizeof(magic));
+        ctx->grid32.kx = magic - (int)K[0]; ctx->grid32.ky = magic - (int)K[1]; ctx->grid32.kz = magic - (int)K[2];
+        for (int i = 0; i < 3; ++i) ctx->fk32_origin[i] = (&ctx->grid.ox)[i] + (K[i] + 1.0) * ctx->res;
+    }
     ctx->has_model32 = true;
     return 0;
 }
@@ -1118,10 +1153,17 @@ int smplgpu_set_robot(smplgpu_ctx* ctx, const smplgpu_robot_desc* d)
 // distance field
 ///////////////////////////////////////////////////////////////////////////////
 
+// the single-precision kernels index the field with 32-bit ints
+static bool field_cells_ok(int nx, int ny, int nz)
+{
+    return (unsigned long long)nx * ny * nz < (1ull << 31);
+}
+
 static int set_df_common(smplgpu_ctx* ctx, int nx, int ny, int nz, const double origin[3], double res, int dmax_sq, double padding)
 {
     if (nx <= 0 || ny <= 0 || nz <= 0 || !(res > 0.0) || dmax_sq < 0 || dmax_sq > 65534)
         return fail(ctx, SMPLGPU_ERR_INVALID, "bad distance field parameters");
+    if (!field_cells_ok(nx, ny, nz)) return fail(ctx, SMPLGPU_ERR_INVALID, "distance field of 2^31 cells or more");
     // a bank run queued behind the caller's back still reads the field; a bank (and the walls derived from the
     // field) of another shape would be indexed with the wrong strides
     {
@@ -1435,6 +1477,7 @@ int smplgpu_reserve_distance_field(smplgpu_ctx* ctx, int nx, int ny, int nz, voi
 {
     if (!ctx || !ptr || !bytes) return SMPLGPU_ERR_INVALID;
     if (nx <= 0 || ny <= 0 || nz <= 0) return fail(ctx, SMPLGPU_ERR_INVALID, "bad distance field dimensions");
+    if (!field_cells_ok(nx, ny, nz)) return fail(ctx, SMPLGPU_ERR_INVALID, "distance field of 2^31 cells or more");
     {
         const int fr = finish_bank_run(ctx);
         if (fr) return fr;
@@ -2070,7 +2113,8 @@ int smplgpu_fk_sphere_centers_f32(smplgpu_ctx* ctx, const double* q, int n, floa
     CU(cudaMemcpyAsync(dq, q, qb, cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaMemsetAsync(dout, 0, ob, ctx->stream));
     const int t32 = ctx->v32_threads;
-    fk_centers32_kernel<<<(n + t32 - 1) / t32, t32, v32_smem(ctx), ctx->stream>>>(ctx->d_blob, ctx->blob_words, dq, n, dout);
+    fk_centers32_kernel<<<(n + t32 - 1) / t32, t32, v32_smem(ctx), ctx->stream>>>(
+        ctx->d_blob, ctx->blob_words, dq, n, ctx->res, ctx->fk32_origin[0], ctx->fk32_origin[1], ctx->fk32_origin[2], dout);
     ++ctx->launches;
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(out, dout, ob, cudaMemcpyDeviceToHost, ctx->stream));

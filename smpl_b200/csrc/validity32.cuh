@@ -7,12 +7,15 @@
 // the single-precision error bound of a decision boundary:
 //
 //   * forward kinematics runs in float with FMA (joint angle split hi + lo so the
-//     sin/cos argument keeps double accuracy); the host derives a rigorous bound
-//     E_pos on |centre_f32 - centre_f64| from the chain (smplgpu.cu: build_model32);
+//     sin/cos argument keeps double accuracy), in GRID UNITS: the host folds the
+//     world -> grid map into the model (translations, centres and radii in cells, the
+//     base transforms map to grid coordinates c = inv_res (x - o) - 1, whose
+//     round-to-nearest is the cell), and derives a rigorous bound E on
+//     |c_f32 - c_f64| from the chain (smplgpu.cu: build_model32);
 //   * a sphere/field test whose grid coordinate lies within eps_cells of a cell
 //     boundary evaluates EVERY cell the double value could fall in; if all of them
 //     give the same outcome the decision is certain, otherwise it is ambiguous;
-//   * a sphere-pair test with |d - (r1+r2)| within 2.5 E_pos is ambiguous.
+//   * a sphere-pair test with |d - (r1+r2)| within 2.5 E is ambiguous.
 //
 // A state with a certain collision is invalid; a state with no collision and no
 // ambiguous decision is valid; anything else is appended to a list that the
@@ -53,28 +56,31 @@ struct Model32Header
     int n_links, n_nodes, n_pairs, n_allowed, n_slots, dof;   // n_slots: transforms kept for branching parents
     int off_link_i;       // int4 per link: parent, fn, var, slot
     int off_link_n;       // int2 per link: first node, end node (pre-order ids of the trees riding on the link)
-    int off_origin;       // float[12] per link (joint origin; constant joints pre-multiplied)
-    int off_axis;         // float4 per link
-    int off_base;         // float[12] per link (used when parent < 0)
-    int off_node_c;       // float4 per node: centre xyz, radius
+    int off_origin;       // float[12] per link (joint origin; constant joints pre-multiplied; translation in cells)
+    int off_axis;         // float4 per link: joint axis (general revolute); prismatic: inv_res * third origin column
+    int off_base;         // float[12] per link (used when parent < 0): world -> grid coordinates less K (Grid32)
+    int off_node_c;       // float4 per node: centre xyz, radius (cells)
     int off_node_i;       // int4 per node: skip, threshold, z, rank of the (double) radius; z = pair-tree index of a
                           // paired tree's root (else -1) in roots-only mode, slot of the node's link in full mode
     int off_node_orig;    // int per node: index in the caller's node table
     int off_pair;         // int4 per pair: pair-tree index a, b; root node a, b (pre-order ids)
     int off_allowed;      // int2 per allowed leaf pair (pre-order ids)
-    float e_pos;          // bound on |centre_f32 - centre_f64| (metres)
-    float eps_cells;      // bound on the grid-coordinate error (cells)
-    float pair_k;         // 2.5 * e_pos
-    float q_lin_max;      // largest |q| of a prismatic variable the bound covers
+    float e_cells;        // bound on |centre_f32 - centre_f64| (cells)
+    float eps_cells;      // e_cells + the rounding of the decision itself (cells)
+    float pair_k;         // 2.5 * e_cells
+    float q_lin_max;      // largest |q| of a prismatic variable the bound covers (joint units)
     int n_ptrees;         // roots-only pair mode: trees in pair tests (one saved root centre each); 0 = full descent mode
     int pad[2];
 };
 static_assert(sizeof(Model32Header) % 16 == 0, "header must keep 16-byte alignment of the arrays");
 
+// The world -> grid map itself is folded into the model's base transforms, less a whole number of cells K per axis
+// (the robot base's cell) that keeps the chain's magnitudes, and so its rounding, small: the model yields c - K and
+// the cell index is round(c - K) + K.  kx, ky, kz = bits(ROUND_MAGIC) - K, the integer round_cell subtracts.
 struct Grid32
 {
     int nx, ny, nz;
-    float inv_res, ox, oy, oz;
+    int kx, ky, kz;
 };
 
 struct Xf32 { float m[12]; };
@@ -122,42 +128,65 @@ __device__ __forceinline__ void slot32_load(const float* slots, int slot, Xf32& 
     for (int e = 0; e < 12; ++e) t.m[e] = p[e * blockDim.x];
 }
 
+// Cell and remainder of a grid coordinate c, on the FMA pipe.  For |c| < 2^22, c + 1.5 * 2^23 lies in (2^23, 2^24),
+// where floats are spaced 1 apart, so this one add rounds c to the nearest integer (ties to even) and leaves it in
+// the low mantissa bits: the integer difference of the two bit patterns is round(c).  (c + M) - M is round(c)
+// exactly (Sterbenz), and so is rem = c - round(c) in [-1/2, 1/2] (both are multiples of ulp(c), or round(c) = 0).
+// k = bits(M) - K adds the model's whole-cell offset K in the same integer subtract.
+constexpr float ROUND_MAGIC = 12582912.0f;   // 1.5 * 2^23
+__device__ __forceinline__ int round_cell(float c, int k, float& rem)
+{
+    const float t = __fadd_rn(c, ROUND_MAGIC);
+    rem = __fsub_rn(c, __fsub_rn(t, ROUND_MAGIC));
+    return __float_as_int(t) - k;
+}
+
 // Sphere vs field with certification.  Returns 1 = passes, 0 = fails, 2 = ambiguous.
-__device__ __forceinline__ int lookup32(const uint16_t* __restrict__ df, const Grid32& G, float eps,
+//   (x, y, z): the centre in grid coordinates c = inv_res (p - o) - 1, less K, so the reference's cell
+//   (int)(inv_res (p - o) + 0.5) - 1 is round(c) and the cell boundaries are the half-integers (for c < -1/2 both
+//   are outside the grid); K is whole, so rem and the boundaries are the same for c - K.  c is within eps of a
+//   boundary iff |rem| > lim = 1/2 - eps; an exact tie (|rem| = 1/2, rounded to either side) is one of those, and the
+//   near branch then evaluates the cells on both sides of it.  build_model32 admits a model only if |K| < 2^21 and
+//   every centre the kernels evaluate has |c - K| < 2^21, so round_cell is exact for all of them, the index does not
+//   overflow, and an out-of-grid centre keeps its out-of-grid index and reads d2 = 0 as in the reference.
+__device__ __forceinline__ int lookup32(const uint16_t* __restrict__ df, const Grid32& G, float lim,
                                         float x, float y, float z, int thresh)
 {
-    const float gx = fmaf(G.inv_res, x - G.ox, 0.5f);
-    const float gy = fmaf(G.inv_res, y - G.oy, 0.5f);
-    const float gz = fmaf(G.inv_res, z - G.oz, 0.5f);
-    const float fx = floorf(gx), fy = floorf(gy), fz = floorf(gz);
-    const float rx = gx - fx, ry = gy - fy, rz = gz - fz;
-    const int ix = (int)fx - 1, iy = (int)fy - 1, iz = (int)fz - 1;
-    const float hi = 1.0f - eps;
-    const bool near = (rx < eps) | (rx > hi) | (ry < eps) | (ry > hi) | (rz < eps) | (rz > hi);
+    float rx, ry, rz;
+    const int ix = round_cell(x, G.kx, rx), iy = round_cell(y, G.ky, ry), iz = round_cell(z, G.kz, rz);
+    const bool near = (fabsf(rx) > lim) | (fabsf(ry) > lim) | (fabsf(rz) > lim);
     if (!near) {
         int d2 = 0;
         if ((unsigned)ix < (unsigned)G.nx && (unsigned)iy < (unsigned)G.ny && (unsigned)iz < (unsigned)G.nz) {
-            d2 = (int)__ldg(&df[((size_t)ix * G.ny + iy) * G.nz + iz]);
+            d2 = (int)__ldg(&df[(ix * G.ny + iy) * G.nz + iz]);   // fields have fewer than 2^31 cells
         }
         return d2 >= thresh ? 1 : 0;
     }
-    // every cell the double-precision coordinate could truncate to
-    const int x0 = ix - (rx < eps ? 1 : 0), x1 = ix + (rx > hi ? 1 : 0);
-    const int y0 = iy - (ry < eps ? 1 : 0), y1 = iy + (ry > hi ? 1 : 0);
-    const int z0 = iz - (rz < eps ? 1 : 0), z1 = iz + (rz > hi ? 1 : 0);
+    // every cell the double-precision coordinate could fall in
+    const int x0 = ix - (rx < -lim ? 1 : 0), x1 = ix + (rx > lim ? 1 : 0);
+    const int y0 = iy - (ry < -lim ? 1 : 0), y1 = iy + (ry > lim ? 1 : 0);
+    const int z0 = iz - (rz < -lim ? 1 : 0), z1 = iz + (rz > lim ? 1 : 0);
     bool any_pass = false, any_fail = false;
     for (int cx = x0; cx <= x1; ++cx) {
         for (int cy = y0; cy <= y1; ++cy) {
             for (int cz = z0; cz <= z1; ++cz) {
                 int d2 = 0;
                 if ((unsigned)cx < (unsigned)G.nx && (unsigned)cy < (unsigned)G.ny && (unsigned)cz < (unsigned)G.nz) {
-                    d2 = (int)__ldg(&df[((size_t)cx * G.ny + cy) * G.nz + cz]);
+                    d2 = (int)__ldg(&df[(cx * G.ny + cy) * G.nz + cz]);
                 }
                 if (d2 >= thresh) any_pass = true; else any_fail = true;
             }
         }
     }
     return (any_pass && any_fail) ? 2 : (any_pass ? 1 : 0);
+}
+
+// val with its low 29 mantissa bits cleared: 24 significant bits, so exact in float (below 2^-126 float drops less than
+// 2^-149 of it), and val minus it is exact in double, so hi = (float)hi_part(val), lo = (float)(val - hi_part(val))
+// keep the angle to ~2^-47 with one DADD and two conversions (|lo| < 2^-23 |val|; a prismatic joint drops lo)
+__device__ __forceinline__ double hi_part(double val)
+{
+    return __hiloint2double(__double2hiint(val), __double2loint(val) & (int)0xE0000000u);
 }
 
 // shared-memory view of the blob
@@ -213,7 +242,7 @@ __device__ __forceinline__ int link_step32(const S32& S, const int* __restrict__
                                            double alpha, float* slots, int l, Xf32& T, bool& amb, Counters& cnt)
 {
     const Model32Header* H = S.h;
-    const float eps = H->eps_cells;
+    const float lim = 0.5f - H->eps_cells;
     {
         const int4 li = S.link_i[l];   // parent, fn, var, slot
         const int fn = li.y;
@@ -226,7 +255,8 @@ __device__ __forceinline__ int link_step32(const S32& S, const int* __restrict__
                 const double diff = (var_type[li.z] == 1) ? normalize_angle(b - a) : (b - a);
                 val = a + alpha * diff;
             }
-            const float hi = (float)val;
+            const double h = hi_part(val);
+            const float hi = (float)h;
             if (fn == 5) {
                 if (!(fabsf(hi) <= H->q_lin_max)) {
                     return 2;
@@ -236,7 +266,7 @@ __device__ __forceinline__ int link_step32(const S32& S, const int* __restrict__
                 if (!(fabsf(hi) <= V32_MAX_ANGLE)) {
                     return 2;   // also catches NaN / inf
                 }
-                const float lo = (float)(val - (double)hi);
+                const float lo = (float)(val - h);
                 float s0, c0;
                 sincosf(hi, &s0, &c0);
                 sn = fmaf(lo, c0, s0);
@@ -277,10 +307,11 @@ __device__ __forceinline__ int link_step32(const S32& S, const int* __restrict__
             A.m[8] = fmaf(cx, ax.z, -sn * ax.y); A.m[9] = fmaf(cy, ax.z, sn * ax.x); A.m[10] = fmaf(cz, ax.z, cs);        A.m[11] = 0.0f;
             xf32_mul(O, A, J);
         } else {
-            J = O;   // origin * Translate(0, 0, q): translation += third column * q
-            J.m[3] = fmaf(O.m[2], lin, O.m[3]);
-            J.m[7] = fmaf(O.m[6], lin, O.m[7]);
-            J.m[11] = fmaf(O.m[10], lin, O.m[11]);
+            const float4 ax = S.axis[l];   // inv_res * third column of the origin
+            J = O;   // origin * Translate(0, 0, q): translation += third column * q, in cells
+            J.m[3] = fmaf(ax.x, lin, O.m[3]);
+            J.m[7] = fmaf(ax.y, lin, O.m[7]);
+            J.m[11] = fmaf(ax.z, lin, O.m[11]);
         }
         Xf32 P;
         if (li.x < 0) {
@@ -309,7 +340,7 @@ __device__ __forceinline__ int link_step32(const S32& S, const int* __restrict__
                 o[0] = x; o[blockDim.x] = y; o[2 * blockDim.x] = z;
             }
             ++cnt.lookups;
-            const int r = lookup32(df, G, eps, x, y, z, ni.y);
+            const int r = lookup32(df, G, lim, x, y, z, ni.y);
             if (r == 1) {
                 node = ni.x;
             } else if (r == 2) {
@@ -1146,10 +1177,12 @@ edges_valid32p_kernel(const float* __restrict__ blob_g, int blob_words, const De
     flush_counters(cnt, stats);
 }
 
-// sphere centres as the single-precision path computes them (original node order), for the error-bound test
+// sphere centres as the single-precision path computes them (original node order), for the error-bound test; the
+// model's coordinates c - K are mapped back to metres in double (x = (c - K) res + o', o' = o + (K + 1) res), so the
+// error is the model's, times res
 __global__ void __launch_bounds__(V32_THREADS)
 fk_centers32_kernel(const float* __restrict__ blob_g, int blob_words, const double* __restrict__ q, int n,
-                    float* __restrict__ out)
+                    double res, double ox, double oy, double oz, float* __restrict__ out)
 {
     extern __shared__ float4 smem4[];
     float* blob = reinterpret_cast<float*>(smem4);
@@ -1170,11 +1203,12 @@ fk_centers32_kernel(const float* __restrict__ blob_g, int blob_words, const doub
         float sn = 0.0f, cs = 1.0f, lin = 0.0f;
         if (li.z >= 0) {
             const double val = qa[li.z];
-            const float hi = (float)val;
+            const double h = hi_part(val);
+            const float hi = (float)h;
             if (fn == 5) {
                 lin = hi;
             } else {
-                const float lo = (float)(val - (double)hi);
+                const float lo = (float)(val - h);
                 float s0, c0;
                 sincosf(hi, &s0, &c0);
                 sn = fmaf(lo, c0, s0);
@@ -1208,10 +1242,11 @@ fk_centers32_kernel(const float* __restrict__ blob_g, int blob_words, const doub
             A.m[8] = fmaf(cx, ax.z, -sn * ax.y); A.m[9] = fmaf(cy, ax.z, sn * ax.x); A.m[10] = fmaf(cz, ax.z, cs);        A.m[11] = 0.0f;
             xf32_mul(O, A, J);
         } else {
+            const float4 ax = S.axis[l];
             J = O;
-            J.m[3] = fmaf(O.m[2], lin, O.m[3]);
-            J.m[7] = fmaf(O.m[6], lin, O.m[7]);
-            J.m[11] = fmaf(O.m[10], lin, O.m[11]);
+            J.m[3] = fmaf(ax.x, lin, O.m[3]);
+            J.m[7] = fmaf(ax.y, lin, O.m[7]);
+            J.m[11] = fmaf(ax.z, lin, O.m[11]);
         }
         Xf32 P;
         if (li.x < 0) {
@@ -1231,7 +1266,9 @@ fk_centers32_kernel(const float* __restrict__ blob_g, int blob_words, const doub
             float x, y, z;
             xf32_point(T, c.x, c.y, c.z, x, y, z);
             float* o = out + ((size_t)i * H->n_nodes + S.node_orig[node]) * 3;
-            o[0] = x; o[1] = y; o[2] = z;
+            o[0] = (float)((double)x * res + ox);
+            o[1] = (float)((double)y * res + oy);
+            o[2] = (float)((double)z * res + oz);
         }
     }
 }
