@@ -535,6 +535,38 @@ int smplgpu_planning_link_ik_position(smplgpu_ctx* ctx, const double* xyz, const
                                       const smplgpu_ik_params* params, double* q_out, uint8_t* ok,
                                       int32_t* iterations);
 
+/* ---- Euclidean-space motions of the path shortcut (ShortcutPath's EUCLID_SPACE type) ----
+ * The motion a -> b between joint states qa = points[idx_a[e]] and qb = points[idx_b[e]] moves the planning link's
+ * target-offset frame on a straight line at a constant rate of turn (the project's own definition; DESIGN.md section 2):
+ *   (pa, Ra), (pb, Rb)  the planning IK's forward map of qa and qb; w = the rotation vector of Rb Ra^T, theta = |w|,
+ *                       d = |pb - pa|
+ *   n                   max(1, ceil(max(d / max_step_m, theta / max_step_rad))); the motion is refused when n > max_steps
+ *   states              qa, q1 .. q(n-1), qb: q_k solves smplgpu_planning_link_ik (full pose, seeded at q(k-1)) for the
+ *                       position pa + (k / n)(pb - pa) and the rotation Rot2(w / theta, (k / n) theta) Ra; the first
+ *                       solve that does not converge or leaves the joint limits refuses the motion
+ *   ok[e]               every consecutive pair of states passes isStateToStateValid (smplgpu_is_edges_valid's verdicts)
+ *   cost[e]             the JointDistance of the consecutive pairs summed in order (post_processing.cpp:48-67) when the
+ *                       IK chain completed, else 0
+ *   n_steps[e]          n, or max_steps + 1 for a motion of more than max_steps steps
+ * With one step per motion (large step bounds) a motion is the straight joint motion qa -> qb.
+ * states (nullable): motion e's n - 1 interior states go to states[state_offsets[e] ..][dof] when its IK chain
+ * completed (nothing is written otherwise).  The motions are deterministic: a second call on some of them returns the
+ * same states, bit for bit.  counters[2] (nullable): IK solves run, and how many converged.  Bad or NaN parameters and
+ * out-of-range indices are SMPLGPU_ERR_INVALID.  The waypoint edges are checked in chunks of at most
+ * SMPLGPU_EUCLID_CHUNK_EDGES. */
+#define SMPLGPU_EUCLID_MAX_STEPS 4096
+#define SMPLGPU_EUCLID_CHUNK_EDGES (1 << 18)
+typedef struct smplgpu_euclid_params {
+    double  max_step_m;       /* > 0; 0.02 by default */
+    double  max_step_rad;     /* > 0; 0.1 by default */
+    int32_t max_steps;        /* 1 .. SMPLGPU_EUCLID_MAX_STEPS; 256 by default */
+    smplgpu_ik_params ik;     /* 100 iterations, tolerance 1e-6 by default */
+} smplgpu_euclid_params;
+int smplgpu_euclid_motions(smplgpu_ctx* ctx, const double* points, int n_points, const int32_t* idx_a,
+                           const int32_t* idx_b, int n, const smplgpu_euclid_params* params, uint8_t* ok, double* cost,
+                           int32_t* n_steps, const int64_t* state_offsets /*nullable*/, double* states /*nullable*/,
+                           int64_t counters[2]);
+
 /* ---- lattice states on the wire as 16-bit coordinates ---- */
 /* The real caller of the validity path, ManipLattice, holds a state as dof small integers (RobotCoord) and forms the
  * joint values with coordToState (manip_lattice.cpp:1245-1261).  These entry points take the coordinates and do

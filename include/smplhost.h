@@ -212,6 +212,19 @@ double smplhost_heur_metric_goal_distance(smplhost_adapters* a, double x, double
 int smplhost_shortcut_paths(smplgpu_ctx* ctx, int dof, const uint8_t* continuous, const double* points,
                             const int32_t* offsets, int n_paths, int type, int32_t* out_idx, int32_t* out_offsets,
                             double* stats);
+/* ShortcutPath(rm, cc, pin, pout, type) with type EUCLID_SPACE for n_paths paths at once, over the project's own
+ * straight planning-link motion (smplgpu_euclid_motions; DESIGN.md section 2, parity unpinned): every motion (i, j),
+ * i < j, of every path is decided in ONE smplgpu_euclid_motions call, shortcut::ShortcutPath's greedy walk (granularity
+ * 1, the original segments costed by JointDistance) runs per path over the answers, and one more call returns the
+ * interior IK states of the motions the walks emitted.  Output points are input points, copied bit for bit, or IK
+ * states: out_points[max_points][dof], out_source[max_points] (the point's index in its input path, or -1 for an IK
+ * state), out_offsets[n_paths+1], *n_out_points = the total.  SMPLGPU_ERR_LIMIT when max_points is too small (the
+ * offsets and *n_out_points are written).  stats[7] (nullable) = motions decided, IK solves, IK solves converged,
+ * waypoint edges checked, device calls, seconds inside smplgpu_* calls, host seconds. */
+int smplhost_shortcut_paths_euclid(smplgpu_ctx* ctx, smplhost_tables* tables, const double* points, const int32_t* offsets,
+                                   int n_paths, const smplgpu_euclid_params* params, double* out_points,
+                                   int32_t* out_source, int max_points, int32_t* out_offsets, int32_t* n_out_points,
+                                   double* stats);
 /* InterpolatePath(cc, path) (post_processing.cpp:476-540) for n_paths paths at once: the waypoints of every
  * segment (CollisionChecker::interpolatePath) are checked in ONE smplgpu_is_states_valid call; a segment whose
  * waypoints are all valid is replaced by them, otherwise its end point is kept.  Returns the total number of

@@ -19,6 +19,8 @@ c_uint16_p = C.POINTER(C.c_uint16)
 _gpu = None
 _host = None
 
+ERR_LIMIT = -5   # SMPLGPU_ERR_LIMIT
+
 
 class SmplGpuError(RuntimeError):
     pass
@@ -128,6 +130,29 @@ class SnapParamsC(C.Structure):
     _fields_ = [("enabled", C.c_int32), ("dist_thresh", C.c_double), ("weight", C.c_double), ("ik", IkParamsC)]
 
 
+class EuclidParamsC(C.Structure):
+    """smplgpu_euclid_params (include/smplgpu.h)."""
+    _fields_ = [("max_step_m", C.c_double), ("max_step_rad", C.c_double), ("max_steps", C.c_int32), ("ik", IkParamsC)]
+
+
+class EuclidParams:
+    """The Euclidean-space motions of the path shortcut (ShortcutPath's EUCLID_SPACE type): a motion between two
+    joint states moves the planning link's target-offset frame on a straight line at a constant rate of turn, in
+    n = max(1, ceil(max(distance / max_step_m, angle / max_step_rad))) steps, each interior state a planning-link IK
+    solution (max_iterations, tolerance) seeded at the one before; a motion of more than max_steps steps is refused."""
+
+    def __init__(self, max_step_m=0.02, max_step_rad=0.1, max_steps=256, max_iterations=100, tolerance=1e-6):
+        self.max_step_m = max_step_m
+        self.max_step_rad = max_step_rad
+        self.max_steps = max_steps
+        self.max_iterations = max_iterations
+        self.tolerance = tolerance
+
+    def c(self):
+        return EuclidParamsC(float(self.max_step_m), float(self.max_step_rad), int(self.max_steps),
+                             IkParamsC(int(self.max_iterations), float(self.tolerance)))
+
+
 SNAP_RPY, SNAP_XYZ, SNAP_XYZ_RPY = 0, 1, 2   # SMPLGPU_SNAP_*: the snap kinds, in successor-word order
 SNAP_KIND_NAMES = ("rpy", "xyz", "xyz_rpy")
 
@@ -232,6 +257,8 @@ def gpu_lib():
         L.smplgpu_planning_frame_fk.argtypes = [vp, dp, i, dp]
         L.smplgpu_planning_link_ik.argtypes = [vp, dp, dp, i, C.POINTER(IkParamsC), dp, bp, ip]
         L.smplgpu_planning_link_ik_position.argtypes = [vp, dp, dp, i, C.POINTER(IkParamsC), dp, bp, ip]
+        L.smplgpu_euclid_motions.argtypes = [vp, dp, i, ip, ip, i, C.POINTER(EuclidParamsC), bp, dp, ip,
+                                             C.POINTER(C.c_int64), dp, C.POINTER(C.c_int64)]
         L.smplgpu_is_mprim_edges_valid.argtypes = [vp, dp, ip, i, dp, i, bp, ip]
         L.smplgpu_is_indexed_edges_valid.argtypes = [vp, dp, i, ip, ip, i, bp, ip]
         L.smplgpu_set_precision_mode.argtypes = [vp, i]
@@ -313,6 +340,8 @@ def host_lib():
                                                 C.POINTER(C.c_int64), c_int32_p]
         H.smplhost_shortcut_paths.argtypes = [vp, C.c_int, c_uint8_p, c_double_p, c_int32_p, C.c_int, C.c_int, c_int32_p,
                                               c_int32_p, c_double_p]
+        H.smplhost_shortcut_paths_euclid.argtypes = [vp, vp, c_double_p, c_int32_p, C.c_int, C.POINTER(EuclidParamsC),
+                                                     c_double_p, c_int32_p, C.c_int, c_int32_p, c_int32_p, c_double_p]
         H.smplhost_interpolate_paths.argtypes = [vp, vp, c_double_p, c_int32_p, C.c_int, c_double_p, C.c_int, c_int32_p,
                                                  c_double_p]
         H.smplhost_tables_attach_box.argtypes = [vp, vp, C.c_char_p, C.c_char_p, c_double_p, c_double_p]
@@ -602,6 +631,38 @@ class GpuContext:
         self._ck(self.L.smplgpu_is_indexed_edges_valid(self.h, _dp(pts), len(pts), _ip(a), _ip(b), len(a), _bp(v),
                                                        _ip(c) if want_counts else None), "is_indexed_edges_valid")
         return (v, c) if want_counts else v
+
+    def euclid_motions(self, points, idx_a, idx_b, params=None, want_states=False):
+        """smplgpu_euclid_motions: the Euclidean-space motions points[idx_a[e]] -> points[idx_b[e]] (EuclidParams;
+        None = the defaults).  Returns dict(ok (n,) bool, cost (n,), n_steps (n,) -- max_steps + 1 for a motion refused
+        for its length --, ik_solves, ik_converged); with want_states also states: per motion its (n_steps - 1, dof)
+        interior states (a second call, for the motions whose step count is within max_steps), NaN where the IK chain
+        did not complete."""
+        prm = (params or EuclidParams()).c()
+        pts = self._q(points)
+        a = np.ascontiguousarray(idx_a, dtype=np.int32)
+        b = np.ascontiguousarray(idx_b, dtype=np.int32)
+        n = len(a)
+        ok = np.zeros(n, np.uint8)
+        cost = np.zeros(n)
+        steps = np.zeros(n, np.int32)
+        ctr = np.zeros(2, np.int64)
+        i64 = C.POINTER(C.c_int64)
+        self._ck(self.L.smplgpu_euclid_motions(self.h, _dp(pts), len(pts), _ip(a), _ip(b), n, C.byref(prm), _bp(ok),
+                                               _dp(cost), _ip(steps), None, None, ctr.ctypes.data_as(i64)),
+                 "euclid_motions")
+        out = dict(ok=ok.astype(bool), cost=cost, n_steps=steps, ik_solves=int(ctr[0]), ik_converged=int(ctr[1]))
+        if want_states:
+            inner = np.where(steps <= prm.max_steps, np.maximum(steps - 1, 0), 0).astype(np.int64)
+            offs = np.zeros(n + 1, np.int64)
+            offs[1:] = np.cumsum(inner)
+            st = np.full((max(1, int(offs[-1])), pts.shape[1]), np.nan)
+            ok2, cost2, steps2 = np.zeros(n, np.uint8), np.zeros(n), np.zeros(n, np.int32)
+            self._ck(self.L.smplgpu_euclid_motions(self.h, _dp(pts), len(pts), _ip(a), _ip(b), n, C.byref(prm),
+                                                   _bp(ok2), _dp(cost2), _ip(steps2), offs.ctypes.data_as(i64), _dp(st),
+                                                   None), "euclid_motions")
+            out["states"] = [st[offs[e]:offs[e + 1]].copy() for e in range(n)]
+        return out
 
     def is_edges_valid_dev(self, q0_ptr, q1_ptr, n, verdict_ptr, counts_ptr=None):
         self._ck(self.L.smplgpu_is_edges_valid_dev(self.h, C.c_void_p(q0_ptr), C.c_void_p(q1_ptr), int(n),
@@ -1099,6 +1160,36 @@ def shortcut_paths(ctx, tables, paths, kind=0):
     st = dict(edges_checked=int(stats[0]), states_checked=int(stats[1]), device_calls=int(stats[2]),
               device_seconds=float(stats[3]), host_seconds=float(stats[4]))
     return [out_idx[out_off[i]:out_off[i + 1]].copy() for i in range(len(paths))], st
+
+
+def shortcut_paths_euclid(ctx, tables, paths, params=None):
+    """smplhost_shortcut_paths_euclid: ShortcutPath with the EUCLID_SPACE type for a list of joint-space paths
+    (EuclidParams; None = the defaults).  Every candidate motion is decided in one device call and the interior IK
+    states of the emitted ones come from a second.  Returns (list of point arrays, list of source arrays -- per output
+    point its index in the input path, -1 for an IK state --, stats dict)."""
+    H = host_lib()
+    dof = tables.dof
+    prm = (params or EuclidParams()).c()
+    flat, offsets = _concat_paths(paths, dof)
+    out_off = np.zeros(len(offsets), np.int32)
+    stats = np.zeros(7)
+    total = C.c_int32(0)
+    room = 2 * int(offsets[-1]) + 64
+    while True:
+        out = np.zeros((room, dof), np.float64)
+        src = np.zeros(room, np.int32)
+        r = H.smplhost_shortcut_paths_euclid(ctx.h, tables.h, _dp(flat), _ip(offsets), len(paths), C.byref(prm),
+                                             _dp(out), _ip(src), room, _ip(out_off), C.byref(total), _dp(stats))
+        if r == ERR_LIMIT and total.value > room:
+            room = total.value
+            continue
+        if r != 0:
+            raise SmplGpuError("shortcut_paths_euclid: " + H.smplhost_last_error().decode())
+        break
+    st = dict(motions=int(stats[0]), ik_solves=int(stats[1]), ik_converged=int(stats[2]), edges_checked=int(stats[3]),
+              device_calls=int(stats[4]), device_seconds=float(stats[5]), host_seconds=float(stats[6]))
+    return ([out[out_off[i]:out_off[i + 1]].copy() for i in range(len(paths))],
+            [src[out_off[i]:out_off[i + 1]].copy() for i in range(len(paths))], st)
 
 
 def interpolate_paths(ctx, tables, paths):

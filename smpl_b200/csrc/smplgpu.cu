@@ -28,6 +28,7 @@
 #include "expand1.cuh"
 #include "lattice.cuh"
 #include "ik.cuh"
+#include "euclid.cuh"
 
 using namespace smplgpu;
 
@@ -3661,6 +3662,123 @@ int smplgpu_planning_link_ik_position(smplgpu_ctx* ctx, const double* xyz, const
                                       const smplgpu_ik_params* params, double* q_out, uint8_t* ok, int32_t* iterations)
 {
     return planning_link_ik(ctx, 3, xyz, seeds, n, params, q_out, ok, iterations);
+}
+
+// The Euclidean-space motions of the path shortcut (euclid.cuh).  All step counts in one launch and one copy back;
+// then the motions in order, packed into chunks of at most SMPLGPU_EUCLID_CHUNK_EDGES waypoint edges: per chunk the
+// IK chains (a warp each), the chunk's edges through launch_edges, and the AND of each motion's verdicts.
+int smplgpu_euclid_motions(smplgpu_ctx* ctx, const double* points, int n_points, const int32_t* idx_a,
+                           const int32_t* idx_b, int n, const smplgpu_euclid_params* params, uint8_t* ok, double* cost,
+                           int32_t* n_steps, const int64_t* state_offsets, double* states, int64_t counters[2])
+{
+    if (!ctx || n < 0 || n_points < 0 || !params) return SMPLGPU_ERR_INVALID;
+    if (!(params->max_step_m > 0.0) || !std::isfinite(params->max_step_m) || !(params->max_step_rad > 0.0) ||
+        !std::isfinite(params->max_step_rad) || params->max_steps < 1 || params->max_steps > SMPLGPU_EUCLID_MAX_STEPS ||
+        bad_ik_params(&params->ik) || !std::isfinite(params->ik.tolerance))
+        return fail(ctx, SMPLGPU_ERR_INVALID, "euclid_motions: step bounds must be positive and finite, max_steps in 1 .. %d, "
+                    "IK max_iterations >= 1 and a positive finite tolerance", SMPLGPU_EUCLID_MAX_STEPS);
+    int r = need_scene(ctx);
+    if (r) return r;
+    if (counters) counters[0] = counters[1] = 0;
+    if (n == 0) return 0;
+    if (!points || !idx_a || !idx_b || !ok || !cost || !n_steps || (states && !state_offsets))
+        return fail(ctx, SMPLGPU_ERR_INVALID, "null pointer");
+    for (int e = 0; e < n; ++e) {
+        if (idx_a[e] < 0 || idx_a[e] >= n_points || idx_b[e] < 0 || idx_b[e] >= n_points)
+            return fail(ctx, SMPLGPU_ERR_INVALID, "motion %d: point index out of range", e);
+        if (states && state_offsets[e] < 0)
+            return fail(ctx, SMPLGPU_ERR_INVALID, "motion %d: negative state offset", e);
+    }
+    const int dof = ctx->h_model->dof;
+    const EuclidParams P{ params->max_step_m, params->max_step_rad, params->max_steps, params->ik.max_iterations,
+                          params->ik.tolerance };
+    // resident for the whole call: points | idx_a | idx_b | steps | edge offsets | cost | chain_ok | ok | counters
+    auto up = [](size_t b) { return (b + 255) / 256 * 256; };
+    const size_t pb = up((size_t)n_points * dof * sizeof(double)), ib = up((size_t)n * sizeof(int));
+    const size_t cb = up((size_t)n * sizeof(double)), vb = up((size_t)n);
+    r = grow(ctx, &ctx->d_misc, &ctx->misc_cap, pb + 4 * ib + cb + 2 * vb + 256);
+    if (r) return r;
+    uint8_t* base = (uint8_t*)ctx->d_misc;
+    double* d_points = (double*)base;
+    int* d_a = (int*)(base + pb);
+    int* d_b = (int*)(base + pb + ib);
+    int* d_steps = (int*)(base + pb + 2 * ib);
+    int* d_off = (int*)(base + pb + 3 * ib);
+    double* d_cost = (double*)(base + pb + 4 * ib);
+    uint8_t* d_chain = base + pb + 4 * ib + cb;
+    uint8_t* d_ok = d_chain + vb;
+    unsigned long long* d_ctr = (unsigned long long*)(d_ok + vb);
+    CU(cudaMemsetAsync(d_ctr, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    CU(cudaMemcpyAsync(d_points, points, (size_t)n_points * dof * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_a, idx_a, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_b, idx_b, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    euclid_steps_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_model, d_points, d_a, d_b, n, P, d_steps);
+    ++ctx->launches;
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(n_steps, d_steps, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+
+    // chunks: consecutive motions while their edges fit (a refused motion has none)
+    std::vector<int> off(n), chunk_begin(1, 0), chunk_edges;
+    int fill = 0, max_fill = 0;
+    for (int e = 0; e < n; ++e) {
+        const int ne = n_steps[e] <= P.max_steps ? n_steps[e] : 0;
+        if (fill + ne > SMPLGPU_EUCLID_CHUNK_EDGES) {
+            chunk_begin.push_back(e);
+            chunk_edges.push_back(fill);
+            fill = 0;
+        }
+        off[e] = fill;
+        fill += ne;
+        max_fill = std::max(max_fill, fill);
+    }
+    chunk_begin.push_back(n);
+    chunk_edges.push_back(fill);
+    CU(cudaMemcpyAsync(d_off, off.data(), (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    r = ensure_state_buffers(ctx, (size_t)std::max(max_fill, 1), dof, true);
+    if (r) return r;
+    CU(cudaMemsetAsync(ctx->d_stats, 0, 4 * sizeof(unsigned long long), ctx->stream));
+    std::vector<double> h_q1;
+    std::vector<uint8_t> h_chain;
+    for (size_t c = 0; c + 1 < chunk_begin.size(); ++c) {
+        const int first = chunk_begin[c], count = chunk_begin[c + 1] - first, edges = chunk_edges[c];
+        euclid_chain_kernel<<<(unsigned)((count + IK_WARPS - 1) / IK_WARPS), 32 * IK_WARPS, 0, ctx->stream>>>(
+            ctx->d_model, d_points, d_a, d_b, first, count, P, d_off, ctx->d_q0, ctx->d_q1, d_chain, d_cost, d_ctr);
+        ++ctx->launches;
+        CU(cudaGetLastError());
+        if (edges > 0) {
+            r = launch_edges(ctx, ctx->d_q0, ctx->d_q1, edges, ctx->d_verdict, nullptr);
+            if (r) return r;
+        }
+        euclid_reduce_kernel<<<(count + 127) / 128, 128, 0, ctx->stream>>>(first, count, P.max_steps, d_steps, d_off,
+                                                                             d_chain, ctx->d_verdict, d_ok);
+        ++ctx->launches;
+        CU(cudaGetLastError());
+        if (states) {
+            // the interior states of the completed chains: state k of motion e is the end of its edge k - 1
+            h_q1.resize((size_t)edges * dof);
+            h_chain.resize((size_t)count);
+            CU(cudaMemcpyAsync(h_q1.data(), ctx->d_q1, h_q1.size() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaMemcpyAsync(h_chain.data(), d_chain + first, (size_t)count, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaStreamSynchronize(ctx->stream));
+            for (int e = first; e < first + count; ++e) {
+                if (h_chain[e - first] && n_steps[e] > 1) {
+                    std::memcpy(states + (size_t)state_offsets[e] * dof, h_q1.data() + (size_t)off[e] * dof,
+                                (size_t)(n_steps[e] - 1) * dof * sizeof(double));
+                }
+            }
+        }
+    }
+    CU(cudaMemcpyAsync(ok, d_ok, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(cost, d_cost, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    unsigned long long ctr[2];
+    CU(cudaMemcpyAsync(ctr, d_ctr, sizeof(ctr), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    if (counters) {
+        counters[0] = (int64_t)ctr[0];
+        counters[1] = (int64_t)ctr[1];
+    }
+    return 0;
 }
 
 int smplgpu_lattice_set_snap(smplgpu_ctx* ctx, const smplgpu_snap_params* p)

@@ -852,7 +852,7 @@ int smplhost_shortcut_paths(smplgpu_ctx* ctx, int dof, const uint8_t* continuous
         return SMPLGPU_ERR_INVALID;
     }
     if (type != smplhost::SHORTCUT_JOINT_SPACE && type != smplhost::SHORTCUT_JOINT_POSITION_VELOCITY_SPACE) {
-        g_err = "smplhost_shortcut_paths: only the joint-space shortcut types run here (EUCLID_SPACE needs the IK plugin)";
+        g_err = "smplhost_shortcut_paths: only the joint-space shortcut types run here (EUCLID_SPACE: smplhost_shortcut_paths_euclid)";
         return SMPLGPU_ERR_INVALID;
     }
     for (int p = 0; p < n_paths; ++p) {
@@ -871,6 +871,52 @@ int smplhost_shortcut_paths(smplgpu_ctx* ctx, int dof, const uint8_t* continuous
     std::copy(idx.begin(), idx.end(), out_idx);
     std::copy(off.begin(), off.end(), out_offsets);
     copy_post_stats(st, stats);
+    return 0;
+}
+
+int smplhost_shortcut_paths_euclid(smplgpu_ctx* ctx, smplhost_tables* tables, const double* points, const int32_t* offsets,
+                                   int n_paths, const smplgpu_euclid_params* params, double* out_points,
+                                   int32_t* out_source, int max_points, int32_t* out_offsets, int32_t* n_out_points,
+                                   double* stats)
+{
+    if (!ctx || !tables || !params || n_paths < 0 || max_points < 0 ||
+        (n_paths > 0 && (!points || !offsets || !out_offsets || !n_out_points))) {
+        g_err = "smplhost_shortcut_paths_euclid: bad argument";
+        return SMPLGPU_ERR_INVALID;
+    }
+    for (int p = 0; p < n_paths; ++p) {
+        if (offsets[p + 1] < offsets[p] || offsets[0] != 0) {
+            g_err = "smplhost_shortcut_paths_euclid: offsets must start at 0 and not decrease";
+            return SMPLGPU_ERR_INVALID;
+        }
+    }
+    const smplgpu_robot_desc* d = tables->t.desc();
+    std::vector<double> pts;
+    std::vector<int32_t> src, off;
+    smplhost::EuclidShortcutStats st;
+    std::string err;
+    if (!smplhost::ShortcutPathsEuclid(ctx, d->dof, d->var_type, *params, points, offsets, n_paths, pts, src, off, &st, &err)) {
+        g_err = err;
+        return SMPLGPU_ERR_CUDA;
+    }
+    const int total = (int)src.size();
+    if (n_out_points) *n_out_points = total;
+    if (stats) {
+        stats[0] = (double)st.motions;
+        stats[1] = (double)st.ik_solves;
+        stats[2] = (double)st.ik_converged;
+        stats[3] = (double)st.edges_checked;
+        stats[4] = (double)st.device_calls;
+        stats[5] = st.device_seconds;
+        stats[6] = st.host_seconds;
+    }
+    if (n_paths > 0) std::copy(off.begin(), off.end(), out_offsets);
+    if (total > max_points || (total > 0 && (!out_points || !out_source))) {
+        g_err = "smplhost_shortcut_paths_euclid: the output needs room for " + std::to_string(total) + " points";
+        return SMPLGPU_ERR_LIMIT;
+    }
+    std::copy(pts.begin(), pts.end(), out_points);
+    std::copy(src.begin(), src.end(), out_source);
     return 0;
 }
 

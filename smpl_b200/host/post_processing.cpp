@@ -95,21 +95,25 @@ std::vector<double> prefixCosts(const PathView& P, CostFn cost)
 }
 
 // shortcut::ShortcutPath (shortcut.hpp:112-283) with granularity 1 and one generator: grow the segment
-// [s, e] one point at a time for as long as the straight motion s -> e+1 exists and costs no more than the
+// [s, e] one point at a time for as long as the generator's motion s -> e+1 exists and costs no more than the
 // best path over [s, e] plus the original step e -> e+1; otherwise emit the best path and open a new segment
-// at e.  The best path over a segment is either its original points or the two end points.
-void greedyShortcut(const PathView& P, CostFn cost, std::vector<int32_t>& out)
+// at e.  The best path over a segment is either its original points or the generator's motion between its end
+// points.  motion(a, b, c) answers the generator: true and the motion's cost c when it has one.  via_motion
+// (nullable) gets, per output point, 1 when the walk reaches it by a generator's motion, 0 by an original step.
+template <class Motion>
+void greedyShortcut(const PathView& P, CostFn cost, Motion motion, std::vector<int32_t>& out,
+                    std::vector<uint8_t>* via_motion = nullptr)
 {
     const int n = P.n;
     const std::vector<double> accum = prefixCosts(P, cost);
     int s = 0, e = 1;
-    bool direct = false;      // best path over [s, e] is the straight motion
+    bool direct = false;      // best path over [s, e] is the generator's motion
     double best = 0.0;
     auto open = [&]() {
         direct = false;
         best = accum[e] - accum[s];
         double c;
-        if (straightMotion(P, cost, s, e, c) && c <= best) {
+        if (motion(s, e, c) && c <= best) {
             direct = true;
             best = c;
         }
@@ -117,17 +121,22 @@ void greedyShortcut(const PathView& P, CostFn cost, std::vector<int32_t>& out)
     auto emit = [&]() {       // the best path over [s, e] without its first point
         if (direct) {
             out.push_back(e);
+            if (via_motion) via_motion->push_back(1);
         } else {
-            for (int i = s + 1; i <= e; ++i) out.push_back(i);
+            for (int i = s + 1; i <= e; ++i) {
+                out.push_back(i);
+                if (via_motion) via_motion->push_back(0);
+            }
         }
     };
     open();
     out.push_back(0);
+    if (via_motion) via_motion->push_back(0);
     while (e != n - 1) {
         // the reference's last iteration (look-ahead 0 at the final point) only terminates the loop
         double extended = best + (accum[e + 1] - accum[e]);
         double c;
-        if (straightMotion(P, cost, s, e + 1, c) && c <= extended) {
+        if (motion(s, e + 1, c) && c <= extended) {
             direct = true;
             best = c;
             ++e;
@@ -159,6 +168,35 @@ void divideShortcut(const PathView& P, CostFn cost, const std::vector<double>& a
     divideShortcut(P, cost, accum, mid, last, out);
 }
 
+// All motions (i, j), i < j, of every path as point indices; those of path p start at pair_begin[p], row i first
+bool allPairs(const int32_t* offsets, int n_paths, std::vector<size_t>& pair_begin, std::vector<int32_t>& ia,
+              std::vector<int32_t>& ib, const char* who, std::string* err)
+{
+    pair_begin.assign(n_paths + 1, 0);
+    for (int p = 0; p < n_paths; ++p) {
+        const size_t n = (size_t)(offsets[p + 1] - offsets[p]);
+        pair_begin[p + 1] = pair_begin[p] + (n >= 2 ? n * (n - 1) / 2 : 0);
+    }
+    const size_t n_pairs = pair_begin[n_paths];
+    if (n_pairs > 0x7FFFFFFFull) {
+        if (err) *err = std::string(who) + ": more than 2^31 candidate motions";
+        return false;
+    }
+    ia.resize(n_pairs);
+    ib.resize(n_pairs);
+    for (int p = 0; p < n_paths; ++p) {
+        const int base = offsets[p], n = offsets[p + 1] - offsets[p];
+        size_t k = pair_begin[p];
+        for (int i = 0; i < n; ++i) {
+            for (int j = i + 1; j < n; ++j, ++k) {
+                ia[k] = base + i;
+                ib[k] = base + j;
+            }
+        }
+    }
+    return true;
+}
+
 } // namespace
 
 bool ShortcutPaths(smplgpu_ctx* ctx, int dof, const uint8_t* continuous, const double* points,
@@ -175,27 +213,12 @@ bool ShortcutPaths(smplgpu_ctx* ctx, int dof, const uint8_t* continuous, const d
     }
     // every motion the generators can be asked for: all (i, j), i < j, of every path -- ONE device batch
     const int n_points = offsets[n_paths];
-    std::vector<size_t> pair_begin(n_paths + 1, 0);
-    for (int p = 0; p < n_paths; ++p) {
-        const size_t n = (size_t)(offsets[p + 1] - offsets[p]);
-        pair_begin[p + 1] = pair_begin[p] + (n >= 2 ? n * (n - 1) / 2 : 0);
-    }
-    const size_t n_pairs = pair_begin[n_paths];
-    if (n_pairs > 0x7FFFFFFFull) {
-        if (err) *err = "ShortcutPaths: more than 2^31 candidate motions";
+    std::vector<size_t> pair_begin;
+    std::vector<int32_t> ia, ib;
+    if (!allPairs(offsets, n_paths, pair_begin, ia, ib, "ShortcutPaths", err)) {
         return false;
     }
-    std::vector<int32_t> ia(n_pairs), ib(n_pairs);
-    for (int p = 0; p < n_paths; ++p) {
-        const int base = offsets[p], n = offsets[p + 1] - offsets[p];
-        size_t k = pair_begin[p];
-        for (int i = 0; i < n; ++i) {
-            for (int j = i + 1; j < n; ++j, ++k) {
-                ia[k] = base + i;
-                ib[k] = base + j;
-            }
-        }
-    }
+    const size_t n_pairs = pair_begin[n_paths];
     std::vector<uint8_t> ok(n_pairs);
     st.host_seconds += clk.lap();
     if (n_pairs > 0) {
@@ -219,7 +242,9 @@ bool ShortcutPaths(smplgpu_ctx* ctx, int dof, const uint8_t* continuous, const d
         if (P.n < 2) {   // "pout = pin" (post_processing.cpp:291-294)
             for (int i = 0; i < P.n; ++i) out_idx.push_back(i);
         } else if (type == SHORTCUT_JOINT_SPACE) {
-            greedyShortcut(P, &PathView::posDistance, out_idx);
+            greedyShortcut(P, &PathView::posDistance, [&](int a, int b, double& c) {
+                return straightMotion(P, &PathView::posDistance, a, b, c);
+            }, out_idx);
         } else {
             // CreatePositionVelocityPath (post_processing.cpp:367-401): the sign of the motion into each point
             P.vel.assign((size_t)P.n * dof, 0.0);
@@ -230,7 +255,9 @@ bool ShortcutPaths(smplgpu_ctx* ctx, int dof, const uint8_t* continuous, const d
                 }
             }
             std::vector<int32_t> greedy, dnc;
-            greedyShortcut(P, &PathView::pvDistance, greedy);
+            greedyShortcut(P, &PathView::pvDistance, [&](int a, int b, double& c) {
+                return straightMotion(P, &PathView::pvDistance, a, b, c);
+            }, greedy);
             dnc.push_back(0);
             divideShortcut(P, &PathView::pvDistance, prefixCosts(P, &PathView::pvDistance), 0, P.n - 1, dnc);
             auto total = [&](const std::vector<int32_t>& idx) {
@@ -243,6 +270,135 @@ bool ShortcutPaths(smplgpu_ctx* ctx, int dof, const uint8_t* continuous, const d
         }
         (void)first_out;
         out_offsets.push_back((int32_t)out_idx.size());
+    }
+    st.host_seconds += clk.lap();
+    if (stats) *stats = st;
+    return true;
+}
+
+bool ShortcutPathsEuclid(smplgpu_ctx* ctx, int dof, const int32_t* var_types, const smplgpu_euclid_params& params,
+                         const double* points, const int32_t* offsets, int n_paths, std::vector<double>& out_points,
+                         std::vector<int32_t>& out_source, std::vector<int32_t>& out_offsets, EuclidShortcutStats* stats,
+                         std::string* err)
+{
+    out_points.clear();
+    out_source.clear();
+    out_offsets.assign(1, 0);
+    EuclidShortcutStats st;
+    Clock clk;
+    if (n_paths <= 0) {
+        if (stats) *stats = st;
+        return true;
+    }
+    std::vector<uint8_t> continuous(dof);
+    for (int v = 0; v < dof; ++v) continuous[v] = var_types[v] == SMPLGPU_VAR_CONTINUOUS ? 1 : 0;
+    // 1. every motion (i, j), i < j, of every path decided in ONE device call
+    const int n_points = offsets[n_paths];
+    std::vector<size_t> pair_begin;
+    std::vector<int32_t> ia, ib;
+    if (!allPairs(offsets, n_paths, pair_begin, ia, ib, "ShortcutPathsEuclid", err)) {
+        return false;
+    }
+    const size_t n_pairs = pair_begin[n_paths];
+    std::vector<uint8_t> ok(n_pairs);
+    std::vector<double> cost(n_pairs);
+    std::vector<int32_t> steps(n_pairs);
+    int64_t ctr[2] = { 0, 0 };
+    st.host_seconds += clk.lap();
+    if (n_pairs > 0) {
+        if (smplgpu_euclid_motions(ctx, points, n_points, ia.data(), ib.data(), (int)n_pairs, &params, ok.data(),
+                                   cost.data(), steps.data(), nullptr, nullptr, ctr) != 0) {
+            if (err) *err = smplgpu_last_error(ctx);
+            return false;
+        }
+        ++st.device_calls;
+        st.motions += (long long)n_pairs;
+        st.ik_solves += ctr[0];
+        st.ik_converged += ctr[1];
+        for (size_t k = 0; k < n_pairs; ++k) {
+            st.edges_checked += steps[k] <= params.max_steps ? steps[k] : 0;
+        }
+    }
+    st.device_seconds += clk.lap();
+
+    // 2. the greedy walk of each path over the answers
+    std::vector<std::vector<int32_t>> idx(n_paths);
+    std::vector<std::vector<uint8_t>> via(n_paths);
+    std::vector<std::vector<int>> emitted(n_paths);   // per output point: the emitted motion into it, or -1
+    std::vector<int32_t> sa, sb, sn;  // the emitted motions that have interior states, and their step counts
+    std::vector<int64_t> soff;        // where their states go
+    int64_t n_states = 0;
+    for (int p = 0; p < n_paths; ++p) {
+        PathView P;
+        P.dof = dof;
+        P.continuous = continuous.data();
+        P.pts = points + (size_t)offsets[p] * dof;
+        P.n = offsets[p + 1] - offsets[p];
+        P.ok = ok.data() + pair_begin[p];
+        if (P.n < 2) {   // "pout = pin"
+            for (int i = 0; i < P.n; ++i) {
+                idx[p].push_back(i);
+                via[p].push_back(0);
+            }
+            continue;
+        }
+        const double* pc = cost.data() + pair_begin[p];
+        greedyShortcut(P, &PathView::posDistance, [&](int a, int b, double& c) {
+            if (!P.valid(a, b)) return false;
+            c = pc[P.tri(a, b)];
+            return true;
+        }, idx[p], &via[p]);
+        emitted[p].assign(idx[p].size(), -1);
+        for (size_t i = 1; i < idx[p].size(); ++i) {
+            const size_t k = pair_begin[p] + P.tri(idx[p][i - 1], idx[p][i]);
+            if (via[p][i] && steps[k] > 1) {
+                emitted[p][i] = (int)sa.size();
+                sa.push_back(ia[k]);
+                sb.push_back(ib[k]);
+                sn.push_back(steps[k]);
+                soff.push_back(n_states);
+                n_states += steps[k] - 1;
+            }
+        }
+    }
+    st.host_seconds += clk.lap();
+
+    // 3. the interior states of the emitted motions: the same motions again, deterministic
+    std::vector<double> states((size_t)n_states * dof);
+    if (!sa.empty()) {
+        const int m = (int)sa.size();
+        std::vector<uint8_t> ok2(m);
+        std::vector<double> cost2(m);
+        std::vector<int32_t> steps2(m);
+        if (smplgpu_euclid_motions(ctx, points, n_points, sa.data(), sb.data(), m, &params, ok2.data(), cost2.data(),
+                                   steps2.data(), soff.data(), states.data(), ctr) != 0) {
+            if (err) *err = smplgpu_last_error(ctx);
+            return false;
+        }
+        ++st.device_calls;
+        for (int k = 0; k < m; ++k) {
+            if (!ok2[k] || steps2[k] != sn[k]) {
+                if (err) *err = "ShortcutPathsEuclid: a motion changed between the two device calls";
+                return false;
+            }
+        }
+    }
+    st.device_seconds += clk.lap();
+
+    // 4. the output: input points copied, IK states where a motion was emitted
+    for (int p = 0; p < n_paths; ++p) {
+        const int base = offsets[p];
+        for (size_t i = 0; i < idx[p].size(); ++i) {
+            const int m = emitted[p].empty() ? -1 : emitted[p][i];
+            if (m >= 0) {
+                out_points.insert(out_points.end(), states.begin() + soff[m] * dof, states.begin() + (soff[m] + sn[m] - 1) * dof);
+                out_source.insert(out_source.end(), (size_t)(sn[m] - 1), -1);
+            }
+            const int j = base + idx[p][i];
+            out_points.insert(out_points.end(), points + (size_t)j * dof, points + (size_t)(j + 1) * dof);
+            out_source.push_back(idx[p][i]);
+        }
+        out_offsets.push_back((int32_t)out_source.size());
     }
     st.host_seconds += clk.lap();
     if (stats) *stats = st;
