@@ -43,6 +43,15 @@ int smplhost_tables_detach(smplhost_tables* h, const char* id);
 int smplhost_tables_set_planning_chain(smplhost_tables* h, const char* root, const char* tip,
                                        const char* planning_link, const double* T_kin_to_planning /*[12] or NULL*/,
                                        const double* xyz_offset /*[3] or NULL*/);
+/* A planning chain over a subset of the planning variables (the project's own rule; KDLRobotModel, and so
+ * smplhost_tables_set_planning_chain, refuses such models): every movable joint of the root -> tip chain must be a
+ * planning variable, at any index and in any order; planning variables off the chain are allowed and move collision
+ * geometry only (their limits are configure's).  The planning link must be a segment of the chain.  When the planning
+ * variables are exactly the chain's movable joints in chain order, the tables equal those of
+ * smplhost_tables_set_planning_chain.  Returns 0, or -1 with smplhost_last_error set. */
+int smplhost_tables_set_planning_chain_subset(smplhost_tables* h, const char* root, const char* tip,
+                                              const char* planning_link, const double* T_kin_to_planning /*[12] or NULL*/,
+                                              const double* xyz_offset /*[3] or NULL*/);
 int smplhost_tables_dof(smplhost_tables* h);
 int smplhost_tables_limits(smplhost_tables* h, double* mins, double* maxs, uint8_t* continuous);
 const smplgpu_robot_desc* smplhost_tables_desc(smplhost_tables* h);

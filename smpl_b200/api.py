@@ -313,6 +313,8 @@ def host_lib():
         H.smplhost_tables_attach_spheres.argtypes = [vp, C.c_char_p, C.c_char_p, c_double_p, C.c_int, C.c_double]
         H.smplhost_tables_detach.argtypes = [vp, C.c_char_p]
         H.smplhost_tables_set_planning_chain.argtypes = [vp, C.c_char_p, C.c_char_p, C.c_char_p, c_double_p, c_double_p]
+        H.smplhost_tables_set_planning_chain_subset.argtypes = [vp, C.c_char_p, C.c_char_p, C.c_char_p, c_double_p,
+                                                                c_double_p]
         H.smplhost_tables_dof.argtypes = [vp]
         H.smplhost_tables_limits.argtypes = [vp, c_double_p, c_double_p, c_uint8_p]
         H.smplhost_tables_apply.argtypes = [vp, vp]
@@ -420,12 +422,15 @@ class RobotTables:
     def detach(self, body_id):
         return self.H.smplhost_tables_detach(self.h, body_id.encode()) == 0
 
-    def set_planning_chain(self, root, tip, planning_link, T_kin_to_planning=None, xyz_offset=None):
+    def set_planning_chain(self, root, tip, planning_link, T_kin_to_planning=None, xyz_offset=None, subset=False):
+        """subset=False: KDLRobotModel's rule, the planning variables are exactly the chain's movable joints in chain
+        order.  subset=True: the chain's movable joints are planning variables at any index, and planning variables
+        off the chain are allowed (smplhost_tables_set_planning_chain_subset)."""
         T = np.eye(4)[:3] if T_kin_to_planning is None else np.asarray(T_kin_to_planning, np.float64).reshape(3, 4)
         T = np.ascontiguousarray(T, dtype=np.float64)
         off = np.ascontiguousarray(np.zeros(3) if xyz_offset is None else np.asarray(xyz_offset, np.float64))
-        self._ck(self.H.smplhost_tables_set_planning_chain(self.h, root.encode(), tip.encode(), planning_link.encode(),
-                                                           _dp(T), _dp(off)), "set_planning_chain")
+        f = self.H.smplhost_tables_set_planning_chain_subset if subset else self.H.smplhost_tables_set_planning_chain
+        self._ck(f(self.h, root.encode(), tip.encode(), planning_link.encode(), _dp(T), _dp(off)), "set_planning_chain")
 
     @property
     def dof(self):
@@ -1237,7 +1242,7 @@ def build_tables(scene):
         t.attach_spheres(body_id, link, centers, radius)
     if scene.chain_root is not None:
         t.set_planning_chain(scene.chain_root, scene.chain_tip, scene.planning_link, scene.T_kin_to_planning,
-                             scene.xyz_offset)
+                             scene.xyz_offset, subset=scene.chain_subset)
     return t
 
 

@@ -6,6 +6,7 @@
 #include <array>
 #include <atomic>
 #include <memory>
+#include <mutex>
 #include <thread>
 #include <cmath>
 #include <cstdarg>
@@ -206,6 +207,23 @@ static bool warp_resolve()
                         __FILE__, __LINE__);                                                       \
         }                                                                                          \
     } while (0)
+
+// A kernel's dynamic shared memory cap (cudaFuncAttributeMaxDynamicSharedMemorySize) belongs to the process and the
+// device, not to a context: contexts of different robots size the same kernels differently, so a context only ever
+// raises the cap to what its own launches need.  Setting it to a smaller context's size would make every launch of a
+// larger context in the same process fail with an invalid argument.
+template <class K>
+static cudaError_t raise_smem_cap(K* kernel, int smem)
+{
+    static std::mutex mu;
+    std::lock_guard<std::mutex> lock(mu);
+    cudaFuncAttributes a;
+    cudaError_t e = cudaFuncGetAttributes(&a, kernel);
+    if (e != cudaSuccess || a.maxDynamicSharedSizeBytes >= smem) {
+        return e;
+    }
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+}
 
 static int grow(smplgpu_ctx* ctx, void** p, size_t* cap, size_t need)
 {
@@ -883,14 +901,14 @@ static int build_model32(smplgpu_ctx* ctx)
     }
     ctx->v32_threads = threads;
     const int smem = (int)std::max(fixed + per_thread * threads, (size_t)1024);
-    CU(cudaFuncSetAttribute(states_valid32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    CU(cudaFuncSetAttribute(edges_valid32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    CU(raise_smem_cap(states_valid32_kernel, smem));
+    CU(raise_smem_cap(edges_valid32_kernel, smem));
     ctx->v32_edge_batch_blocks_per_sm = 0;
     {
         const size_t smem_b = (size_t)w * 4 + ((size_t)n_slots32 * 12 + (size_t)n_ptrees * 3) * sizeof(float) * threads +
                               (2 * (size_t)V32_EDGE_EPT * threads + 4) * sizeof(int);   // == v32_smem_edge_batch once blob_words is set
         if (smem_b <= smem_max) {
-            CU(cudaFuncSetAttribute(edges_valid32b_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+            CU(raise_smem_cap(edges_valid32b_kernel, (int)smem_b));
             int per_sm = 0;
             CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, edges_valid32b_kernel, threads, smem_b));
             ctx->v32_edge_batch_blocks_per_sm = per_sm;
@@ -902,9 +920,9 @@ static int build_model32(smplgpu_ctx* ctx)
             }
         }
     }
-    CU(cudaFuncSetAttribute(fk_centers32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    CU(cudaFuncSetAttribute(states_valid32p_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    CU(cudaFuncSetAttribute(edges_valid32p_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    CU(raise_smem_cap(fk_centers32_kernel, smem));
+    CU(raise_smem_cap(states_valid32p_kernel, smem));
+    CU(raise_smem_cap(edges_valid32p_kernel, smem));
     {
         int per_sm = 0;
         if (v32_persistent()) {
@@ -1130,12 +1148,12 @@ int smplgpu_set_robot(smplgpu_ctx* ctx, const smplgpu_robot_desc* d)
         if (per_thread * threads > smem_max) return fail(ctx, SMPLGPU_ERR_LIMIT, "%d link slots need %zu B of shared memory per warp", slots, per_thread * 32);
         ctx->validity_threads = threads;
         const size_t smem = per_thread * threads + 16;
-        CU(cudaFuncSetAttribute(states_valid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)1024)));
-        CU(cudaFuncSetAttribute(edges_valid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)1024)));
-        CU(cudaFuncSetAttribute(fk_centers_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)1024)));
+        CU(raise_smem_cap(states_valid_kernel, (int)std::max(smem, (size_t)1024)));
+        CU(raise_smem_cap(edges_valid_kernel, (int)std::max(smem, (size_t)1024)));
+        CU(raise_smem_cap(fk_centers_kernel, (int)std::max(smem, (size_t)1024)));
         const size_t smem_x1 = (size_t)slots * 12 * sizeof(double) * EXPAND1_THREADS;
         if (smem_x1 <= smem_max - 1024) {
-            CU(cudaFuncSetAttribute(expand_state_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem_x1, (size_t)1024)));
+            CU(raise_smem_cap(expand_state_kernel, (int)std::max(smem_x1, (size_t)1024)));
         }
     }
     ctx->has_robot = true;
@@ -3317,7 +3335,7 @@ int smplgpu_lattice_create(smplgpu_ctx* ctx, const smplgpu_lattice_params* p, in
         ctx->lat_fused = want && use_f32(ctx) && smem <= (size_t)200 * 1024;
         ctx->lat_round_smem = smem;
         if (ctx->lat_fused) {
-            CU(cudaFuncSetAttribute(lattice_round_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)1024)));
+            CU(raise_smem_cap(lattice_round_kernel, (int)std::max(smem, (size_t)1024)));
         }
     }
     ctx->has_lat = true;
@@ -3970,7 +3988,7 @@ int smplgpu_expand_state(smplgpu_ctx* ctx, const double* parent, int cost_per_ce
     }
     if (smem > (size_t)226 * 1024) return fail(ctx, SMPLGPU_ERR_LIMIT, "%d link slots do not fit the expansion kernel", ctx->h_model->n_slots);
     if (smem > ctx->x1_smem_set) {
-        CU(cudaFuncSetAttribute(expand_state_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, (size_t)1024)));
+        CU(raise_smem_cap(expand_state_kernel, (int)std::max(smem, (size_t)1024)));
         ctx->x1_smem_set = smem;
     }
     expand_state_kernel<<<ctx->x1_prims + 1, EXPAND1_THREADS, smem, ctx->stream>>>(

@@ -142,6 +142,14 @@ int smplhost_tables_set_planning_chain(smplhost_tables* h, const char* root, con
     return h->t.setPlanningChain(root, tip, planning_link, T_kin_to_planning, xyz_offset, &g_err) ? 0 : -1;
 }
 
+int smplhost_tables_set_planning_chain_subset(smplhost_tables* h, const char* root, const char* tip,
+                                              const char* planning_link, const double* T_kin_to_planning,
+                                              const double* xyz_offset)
+{
+    if (!h || !root || !tip || !planning_link) return -1;
+    return h->t.setPlanningChain(root, tip, planning_link, T_kin_to_planning, xyz_offset, &g_err, true) ? 0 : -1;
+}
+
 int smplhost_tables_dof(smplhost_tables* h) { return h ? h->t.dof() : -1; }
 
 int smplhost_tables_limits(smplhost_tables* h, double* mins, double* maxs, uint8_t* continuous)

@@ -744,7 +744,7 @@ std::vector<double> RobotTables::outsideGroupVoxels() const
 ///////////////////////////////////////////////////////////////////////////////
 
 bool RobotTables::setPlanningChain(const std::string& root, const std::string& tip, const std::string& planning_link,
-                                   const double T_kin[12], const double xyz_offset[3], std::string* err)
+                                   const double T_kin[12], const double xyz_offset[3], std::string* err, bool subset)
 {
     std::vector<int> chain; // joint recs root -> tip
     std::string link = tip;
@@ -757,12 +757,19 @@ bool RobotTables::setPlanningChain(const std::string& root, const std::string& t
         chain.insert(chain.begin(), m_link_joint[it->second]);
         link = m_links[m_link_parent[it->second]];
     }
-    // every movable chain joint must be a planning variable, in chain order
+    // every movable chain joint must be a planning variable, in chain order (subset mode: at any index)
     std::vector<int> seg_var;
     int k = 0;
     for (int jr : chain) {
         if (m_joint_recs[jr].kind == J_FIXED) {
             seg_var.push_back(-1);
+        } else if (subset) {
+            auto it = std::find(m_planning_joint.begin(), m_planning_joint.end(), jr);
+            if (it == m_planning_joint.end()) {
+                if (err) *err = "chain joint '" + m_joint_recs[jr].name + "' is not a planning variable";
+                return false;
+            }
+            seg_var.push_back((int)(it - m_planning_joint.begin()));
         } else {
             if (k >= (int)m_planning_joint.size() || m_planning_joint[k] != jr) {
                 if (err) *err = "planning joints do not match the movable joints of the chain at '" + m_joint_recs[jr].name + "'";
@@ -771,7 +778,7 @@ bool RobotTables::setPlanningChain(const std::string& root, const std::string& t
             seg_var.push_back(k++);
         }
     }
-    if (k != (int)m_planning_joint.size()) {
+    if (!subset && k != (int)m_planning_joint.size()) {
         if (err) *err = "a planning joint is not part of the kinematic chain";
         return false;
     }

@@ -64,8 +64,12 @@ public:
     void setAcmEntry(const std::string& a, const std::string& b, bool allowed);
     bool attachSpheres(const std::string& id, const std::string& link, const double* centers, int n, double radius);
     bool detach(const std::string& id);
+    /// subset = false: KDLRobotModel's rule, the planning variables are exactly the chain's movable joints in chain
+    /// order.  subset = true: every movable chain joint is a planning variable at any index; planning variables off
+    /// the chain are allowed (they move collision geometry only).
     bool setPlanningChain(const std::string& root, const std::string& tip, const std::string& planning_link,
-                          const double T_kin_to_planning[12], const double xyz_offset[3], std::string* err);
+                          const double T_kin_to_planning[12], const double xyz_offset[3], std::string* err,
+                          bool subset = false);
 
     /// flat tables for smplgpu_set_robot (valid until the next mutating call)
     const smplgpu_robot_desc* desc();

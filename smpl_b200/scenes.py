@@ -63,6 +63,7 @@ class Scene:
         self.planning_link = None
         self.T_kin_to_planning = np.eye(4)[:3].copy()
         self.xyz_offset = (0.0, 0.0, 0.0)
+        self.chain_subset = False      # True: the chain moves only some of the planning variables (set_planning_chain)
         self.inflation_radius = 0.02   # planning_link_sphere_radius, call_planner.cpp:1715
         self.cost_per_cell = 250       # planning_params.h:68 default... set by callers
         self.attached = None           # (id, link, centers[n,3], radius)
@@ -196,6 +197,11 @@ def pr2_dual_arm_scene(seed=17):
     s = Scene("pr2", "torso", joints, (-1.0, -1.5, 0.0), (3.0, 3.0, 2.0), 0.01, 0.2)
     s.use_desc_acm = True
     s.cost_per_cell = 100
+    _dual_arm_shelf(s, seed)
+    return s
+
+
+def _dual_arm_shelf(s, seed):
     rng = np.random.Generator(np.random.PCG64(seed))
     # shelf unit in front of the robot: 5 shelves x 4 bays of 2-cell-thick planes
     x0, x1, y0, y1 = 0.75, 1.25, -1.0, 1.0
@@ -209,7 +215,33 @@ def pr2_dual_arm_scene(seed=17):
         size = rng.uniform(0.04, 0.2, 3)
         c = np.array([rng.uniform(x0 + 0.1, x1 - 0.1), rng.uniform(y0 + 0.1, y1 - 0.1), rng.uniform(0.35, 1.7)])
         s.add_box(c, size)
+
+
+def pr2_dual_arm_planning_scene(res=0.01, planning_link="r_gripper_palm_link", seed=17):
+    """Config 5 as a planning problem: pr2_dual_arm_scene's robot, group and shelf at `res`, planned over all 15
+    variables with the chain base_link -> planning_link (torso and one arm); the other arm moves collision geometry
+    only (Scene.chain_subset).  Planning frame base_footprint, as in the 7-DOF fixtures."""
+    joints = ["torso_lift_joint"] + PR2_RIGHT_ARM_JOINTS + PR2_LEFT_ARM_JOINTS
+    s = Scene("pr2", "torso", joints, (-1.0, -1.5, 0.0), (3.0, 3.0, 2.0), res, 0.2)
+    s.use_desc_acm = True
+    s.cost_per_cell = 100
+    _dual_arm_shelf(s, seed)
+    s.chain_root = "base_link"
+    s.chain_tip = planning_link
+    s.planning_link = planning_link
+    T = np.eye(4)[:3].copy()
+    T[:, 3] = (0.0, 0.0, 0.051)                                   # base_footprint_joint
+    s.T_kin_to_planning = T
+    s.chain_subset = True
     return s
+
+
+# OUR fixture: the right arm at PR2_DEMO_START and the left arm its mirror image (pan and roll joints negated); the torso
+# at 0.25 m, mid-range (below about 0.18 m the torso link's spheres meet the base's voxels, so the 7-DOF scenes' fixed
+# 0.16825 m is not collision-free in this group)
+DUAL_ARM_START = (0.25,
+                  -0.5, 0.3, 0.0, -1.0, 0.0, -0.5, 0.0,
+                  0.5, 0.3, 0.0, -1.0, 0.0, -0.5, 0.0)
 
 
 def random_states(n, lo, hi, continuous, seed):
@@ -262,6 +294,31 @@ class PlanParams:
         self.epsilon = 100.0
         self.max_expansions = 200000
         self.xyz_tolerance = [0.015, 0.015, 0.015]
+
+
+class DualArmPlanParams(PlanParams):
+    """Lattice of the 15-DOF planning scene (torso, right arm, left arm): resolutions 0.01 m for the torso and 1 degree
+    for the arm joints; long primitives torso +-0.02 m and joints 1-4 of each arm +-7 degrees (18 successor words),
+    short primitives every arm joint +-4 degrees (28 words).  Stride 28: with the 3 snap words 31 successors, within the
+    lattice kernels' 32."""
+
+    def __init__(self):
+        super().__init__(15)
+        deg = math.pi / 180.0
+        self.resolutions = [0.01] + [0.017453292519943295] * 14
+        prims, flags = [], []
+        for j, d in [(0, 0.02)] + [(a + j, 7.0 * deg) for a in (1, 8) for j in range(4)]:
+            v = [0.0] * 15
+            v[j] = d
+            prims.append(v)
+            flags.append(0)
+        for j in range(1, 15):
+            v = [0.0] * 15
+            v[j] = 4.0 * deg
+            prims.append(v)
+            flags.append(1)
+        self.mprims = np.array(prims)
+        self.short_flags = np.array(flags, np.uint8)
 
 
 def mprim_edges(q, deltas=None):
