@@ -858,9 +858,11 @@ static int build_model32(smplgpu_ctx* ctx)
         BI[h.off_link_n + 2 * l] = link_nbeg[l];
         BI[h.off_link_n + 2 * l + 1] = link_nend[l];
         for (int k = 0; k < 12; ++k) {
-            const bool t = k % 4 == 3;
-            B[h.off_origin + 12 * l + k] = (float)(t ? sc * J[k] : J[k]);
-            B[h.off_base + 12 * l + k] = (float)(t ? base_t(l, k / 4) : m.link_base[l][k]);
+            // row-major k = 4 i + j; the kernels keep rows 0 and 1 as (m[0][j], m[1][j]) pairs, then row 2 (Xf32)
+            const int i = k / 4, j = k % 4, word = i < 2 ? 2 * j + i : 8 + j;
+            const bool t = j == 3;
+            B[h.off_origin + 12 * l + word] = (float)(t ? sc * J[k] : J[k]);
+            B[h.off_base + 12 * l + word] = (float)(t ? base_t(l, i) : m.link_base[l][k]);
         }
         for (int k = 0; k < 3; ++k) {
             B[h.off_axis + 4 * l + k] = (float)(fn == 5 ? sc * J[4 * k + 2] : m.link_axis[l][k]);
@@ -901,8 +903,11 @@ static int build_model32(smplgpu_ctx* ctx)
     }
     ctx->v32_threads = threads;
     const int smem = (int)std::max(fixed + per_thread * threads, (size_t)1024);
-    CU(raise_smem_cap(states_valid32_kernel, smem));
-    CU(raise_smem_cap(edges_valid32_kernel, smem));
+    // the two hot kernels are compiled per pair mode (validity32.cuh: PairMode)
+    const auto states_k = roots_only ? states_valid32_kernel<PAIRS_ROOTS> : states_valid32_kernel<PAIRS_DESCENT>;
+    const auto edges_k = roots_only ? edges_valid32_kernel<PAIRS_ROOTS> : edges_valid32_kernel<PAIRS_DESCENT>;
+    CU(raise_smem_cap(states_k, smem));
+    CU(raise_smem_cap(edges_k, smem));
     ctx->v32_edge_batch_blocks_per_sm = 0;
     {
         const size_t smem_b = (size_t)w * 4 + ((size_t)n_slots32 * 12 + (size_t)n_ptrees * 3) * sizeof(float) * threads +
@@ -914,7 +919,7 @@ static int build_model32(smplgpu_ctx* ctx)
             ctx->v32_edge_batch_blocks_per_sm = per_sm;
             if (getenv("SMPLGPU_V32_VERBOSE")) {
                 int per_sm_old = 0;
-                cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_old, edges_valid32_kernel, threads, (size_t)smem);
+                cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_old, edges_k, threads, (size_t)smem);
                 fprintf(stderr, "[smplgpu] edge kernels: %d threads, shared memory %d B (block form, %d blocks/SM) / %zu B (batched, %d blocks/SM)\n",
                         threads, smem, per_sm_old, smem_b, per_sm);
             }
@@ -928,7 +933,7 @@ static int build_model32(smplgpu_ctx* ctx)
         if (v32_persistent()) {
             CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, states_valid32p_kernel, threads, (size_t)smem));
         } else
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, states_valid32_kernel, threads, (size_t)smem));
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, states_k, threads, (size_t)smem));
         ctx->v32_blocks_per_sm = std::max(1, per_sm);
     }
     int r = grow(ctx, (void**)&ctx->d_blob, &ctx->blob_cap, (size_t)w * 4);
@@ -1610,7 +1615,8 @@ static int launch_states(smplgpu_ctx* ctx, const double* dq, int n, uint8_t* dv)
             ctx->d_blob, ctx->blob_words, ctx->d_model, ctx->d_df, ctx->grid32, dq, n, dv, ctx->d_unc_list,
             ctx->d_unc_count, ctx->d_stats);
     } else
-    states_valid32_kernel<<<std::min((n + t32 - 1) / t32, wave), t32, v32_smem(ctx), ctx->stream>>>(
+    (ctx->v32_ptrees > 0 ? states_valid32_kernel<PAIRS_ROOTS> : states_valid32_kernel<PAIRS_DESCENT>)
+        <<<std::min((n + t32 - 1) / t32, wave), t32, v32_smem(ctx), ctx->stream>>>(
         ctx->d_blob, ctx->blob_words, ctx->d_model, ctx->d_df, ctx->grid32, dq, n, dv, ctx->d_unc_list,
         ctx->d_unc_count, ctx->d_stats);
     if (warp_resolve()) {
@@ -1657,7 +1663,8 @@ static int launch_edges(smplgpu_ctx* ctx, const double* dq0, const double* dq1, 
             ctx->d_unc_count, ctx->d_stats);
     } else
     {
-        edges_valid32_kernel<<<(n + t32 - 1) / t32, t32, v32_smem(ctx), ctx->stream>>>(
+        (ctx->v32_ptrees > 0 ? edges_valid32_kernel<PAIRS_ROOTS> : edges_valid32_kernel<PAIRS_DESCENT>)
+            <<<(n + t32 - 1) / t32, t32, v32_smem(ctx), ctx->stream>>>(
             ctx->d_blob, ctx->blob_words, ctx->d_model, ctx->d_df, ctx->grid32, dq0, dq1, n, dv, dc, ctx->d_unc_list,
             ctx->d_unc_count, ctx->d_stats, ctx->d_unc_mask);
         masked = true;

@@ -40,11 +40,18 @@
 namespace smplgpu {
 
 constexpr int V32_THREADS = 128;
-// -DV32_MIN_BLOCKS=n asks ptxas for n resident blocks per SM (tuning experiments; the default lets it choose)
+// -DV32_MIN_BLOCKS=n asks ptxas for n resident blocks per SM (tuning experiments).  By default the state and edge
+// kernels ask for 9 and 8 (56 and 64 registers): left to itself ptxas picks the same counts but keeps the shared-memory
+// addresses of the model's tables in local memory and reloads them on every link; with the target given, the edge kernel
+// has no local memory and the state kernel 16 bytes (DESIGN.md section 5).
 #ifdef V32_MIN_BLOCKS
 #define V32_BOUNDS __launch_bounds__(V32_THREADS, V32_MIN_BLOCKS)
+#define V32_STATES_BOUNDS V32_BOUNDS
+#define V32_EDGES_BOUNDS V32_BOUNDS
 #else
 #define V32_BOUNDS __launch_bounds__(V32_THREADS)
+#define V32_STATES_BOUNDS __launch_bounds__(V32_THREADS, 9)
+#define V32_EDGES_BOUNDS __launch_bounds__(V32_THREADS, 8)
 #endif
 constexpr float V32_MAX_ANGLE = 64.0f;   // beyond this the hi/lo split no longer keeps the sin/cos argument exact enough
 
@@ -56,9 +63,9 @@ struct Model32Header
     int n_links, n_nodes, n_pairs, n_allowed, n_slots, dof;   // n_slots: transforms kept for branching parents
     int off_link_i;       // int4 per link: parent, fn, var, slot
     int off_link_n;       // int2 per link: first node, end node (pre-order ids of the trees riding on the link)
-    int off_origin;       // float[12] per link (joint origin; constant joints pre-multiplied; translation in cells)
+    int off_origin;       // float[12] per link, Xf32 word order (joint origin; constant joints pre-multiplied; translation in cells)
     int off_axis;         // float4 per link: joint axis (general revolute); prismatic: inv_res * third origin column
-    int off_base;         // float[12] per link (used when parent < 0): world -> grid coordinates less K (Grid32)
+    int off_base;         // float[12] per link, Xf32 word order (used when parent < 0): world -> grid coordinates less K (Grid32)
     int off_node_c;       // float4 per node: centre xyz, radius (cells)
     int off_node_i;       // int4 per node: skip, threshold, z, rank of the (double) radius; z = pair-tree index of a
                           // paired tree's root (else -1) in roots-only mode, slot of the node's link in full mode
@@ -83,25 +90,44 @@ struct Grid32
     int kx, ky, kz;
 };
 
-struct Xf32 { float m[12]; };
+// A link transform [R | t] (3x4, grid units).  Rows 0 and 1 are kept as float2 pairs column by column,
+// c[j] = (m[0][j], m[1][j]), row 2 as scalars, r2[j] = m[2][j]: a product or a point transform then does rows 0 and 1 in
+// one packed FP32 instruction (FFMA2 / FMUL2, two IEEE single-precision operations) with the other operand a broadcast
+// scalar, and row 2 in scalar instructions.  Each element is the same IEEE operation on the same operands, in the same
+// nesting order, as in the scalar form, so centres are bit for bit those the error bound of build_model32 covers.
+// Blob and slot words of a transform: c[0].x c[0].y c[1].x c[1].y c[2].x c[2].y c[3].x c[3].y r2[0..3].
+struct Xf32
+{
+    float2 c[4];
+    float r2[4];
+};
+
+__device__ __forceinline__ float2 bcast2(float s) { return make_float2(s, s); }
+// s * a + b and s * a, in one rounding each, on a scalar or (packed) on a pair
+__device__ __forceinline__ float vfma(float s, float a, float b) { return fmaf(s, a, b); }
+__device__ __forceinline__ float2 vfma(float s, float2 a, float2 b) { return __ffma2_rn(bcast2(s), a, b); }
+__device__ __forceinline__ float vmul(float s, float a) { return __fmul_rn(s, a); }
+__device__ __forceinline__ float2 vmul(float s, float2 a) { return __fmul2_rn(bcast2(s), a); }
 
 __device__ __forceinline__ void xf32_mul(const Xf32& a, const Xf32& b, Xf32& r)
 {
+    // r[i][j] = a[i][0] b[0][j] + a[i][1] b[1][j] + a[i][2] b[2][j] (+ a[i][3] for j = 3), innermost product first
 #pragma unroll
-    for (int i = 0; i < 3; ++i) {
-#pragma unroll
-        for (int j = 0; j < 3; ++j) {
-            r.m[4 * i + j] = fmaf(a.m[4 * i], b.m[j], fmaf(a.m[4 * i + 1], b.m[4 + j], a.m[4 * i + 2] * b.m[8 + j]));
-        }
-        r.m[4 * i + 3] = fmaf(a.m[4 * i], b.m[3], fmaf(a.m[4 * i + 1], b.m[7], fmaf(a.m[4 * i + 2], b.m[11], a.m[4 * i + 3])));
+    for (int j = 0; j < 3; ++j) {
+        const float b0 = b.c[j].x, b1 = b.c[j].y, b2 = b.r2[j];
+        r.c[j] = vfma(b0, a.c[0], vfma(b1, a.c[1], vmul(b2, a.c[2])));
+        r.r2[j] = vfma(b0, a.r2[0], vfma(b1, a.r2[1], vmul(b2, a.r2[2])));
     }
+    const float b0 = b.c[3].x, b1 = b.c[3].y, b2 = b.r2[3];
+    r.c[3] = vfma(b0, a.c[0], vfma(b1, a.c[1], vfma(b2, a.c[2], a.c[3])));
+    r.r2[3] = vfma(b0, a.r2[0], vfma(b1, a.r2[1], vfma(b2, a.r2[2], a.r2[3])));
 }
 
-__device__ __forceinline__ void xf32_point(const Xf32& a, float x, float y, float z, float& px, float& py, float& pz)
+// p = T (x, y, z): (p.x, p.y) packed, p.z scalar
+__device__ __forceinline__ void xf32_point(const Xf32& a, float x, float y, float z, float2& pxy, float& pz)
 {
-    px = fmaf(a.m[0], x, fmaf(a.m[1], y, fmaf(a.m[2], z, a.m[3])));
-    py = fmaf(a.m[4], x, fmaf(a.m[5], y, fmaf(a.m[6], z, a.m[7])));
-    pz = fmaf(a.m[8], x, fmaf(a.m[9], y, fmaf(a.m[10], z, a.m[11])));
+    pxy = vfma(x, a.c[0], vfma(y, a.c[1], vfma(z, a.c[2], a.c[3])));
+    pz = vfma(x, a.r2[0], vfma(y, a.r2[1], vfma(z, a.r2[2], a.r2[3])));
 }
 
 __device__ __forceinline__ void load12(const float* __restrict__ p, Xf32& t)
@@ -109,23 +135,30 @@ __device__ __forceinline__ void load12(const float* __restrict__ p, Xf32& t)
     const float4 a = *reinterpret_cast<const float4*>(p);
     const float4 b = *reinterpret_cast<const float4*>(p + 4);
     const float4 c = *reinterpret_cast<const float4*>(p + 8);
-    t.m[0] = a.x; t.m[1] = a.y; t.m[2] = a.z; t.m[3] = a.w;
-    t.m[4] = b.x; t.m[5] = b.y; t.m[6] = b.z; t.m[7] = b.w;
-    t.m[8] = c.x; t.m[9] = c.y; t.m[10] = c.z; t.m[11] = c.w;
+    t.c[0] = make_float2(a.x, a.y); t.c[1] = make_float2(a.z, a.w);
+    t.c[2] = make_float2(b.x, b.y); t.c[3] = make_float2(b.z, b.w);
+    t.r2[0] = c.x; t.r2[1] = c.y; t.r2[2] = c.z; t.r2[3] = c.w;
 }
 
 __device__ __forceinline__ void slot32_store(float* slots, int slot, const Xf32& t)
 {
     float* p = slots + (size_t)slot * 12 * blockDim.x + threadIdx.x;
 #pragma unroll
-    for (int e = 0; e < 12; ++e) p[e * blockDim.x] = t.m[e];
+    for (int j = 0; j < 4; ++j) {
+        p[(2 * j) * blockDim.x] = t.c[j].x;
+        p[(2 * j + 1) * blockDim.x] = t.c[j].y;
+        p[(8 + j) * blockDim.x] = t.r2[j];
+    }
 }
 
 __device__ __forceinline__ void slot32_load(const float* slots, int slot, Xf32& t)
 {
     const float* p = slots + (size_t)slot * 12 * blockDim.x + threadIdx.x;
 #pragma unroll
-    for (int e = 0; e < 12; ++e) t.m[e] = p[e * blockDim.x];
+    for (int j = 0; j < 4; ++j) {
+        t.c[j] = make_float2(p[(2 * j) * blockDim.x], p[(2 * j + 1) * blockDim.x]);
+        t.r2[j] = p[(8 + j) * blockDim.x];
+    }
 }
 
 // Cell and remainder of a grid coordinate c, on the FMA pipe.  For |c| < 2^22, c + 1.5 * 2^23 lies in (2^23, 2^24),
@@ -141,8 +174,18 @@ __device__ __forceinline__ int round_cell(float c, int k, float& rem)
     return __float_as_int(t) - k;
 }
 
+// round_cell of x and y at once, packed; c - s is formed as fma(s, -1, c), the same single rounding of the same exact
+// difference
+__device__ __forceinline__ void round_cell2(float2 c, int kx, int ky, int& ix, int& iy, float2& rem)
+{
+    const float2 t = __fadd2_rn(c, bcast2(ROUND_MAGIC));
+    rem = __ffma2_rn(__fadd2_rn(t, bcast2(-ROUND_MAGIC)), bcast2(-1.0f), c);
+    ix = __float_as_int(t.x) - kx;
+    iy = __float_as_int(t.y) - ky;
+}
+
 // Sphere vs field with certification.  Returns 1 = passes, 0 = fails, 2 = ambiguous.
-//   (x, y, z): the centre in grid coordinates c = inv_res (p - o) - 1, less K, so the reference's cell
+//   (xy, z): the centre in grid coordinates c = inv_res (p - o) - 1, less K, so the reference's cell
 //   (int)(inv_res (p - o) + 0.5) - 1 is round(c) and the cell boundaries are the half-integers (for c < -1/2 both
 //   are outside the grid); K is whole, so rem and the boundaries are the same for c - K.  c is within eps of a
 //   boundary iff |rem| > lim = 1/2 - eps; an exact tie (|rem| = 1/2, rounded to either side) is one of those, and the
@@ -150,10 +193,14 @@ __device__ __forceinline__ int round_cell(float c, int k, float& rem)
 //   every centre the kernels evaluate has |c - K| < 2^21, so round_cell is exact for all of them, the index does not
 //   overflow, and an out-of-grid centre keeps its out-of-grid index and reads d2 = 0 as in the reference.
 __device__ __forceinline__ int lookup32(const uint16_t* __restrict__ df, const Grid32& G, float lim,
-                                        float x, float y, float z, int thresh)
+                                        float2 xy, float z, int thresh)
 {
-    float rx, ry, rz;
-    const int ix = round_cell(x, G.kx, rx), iy = round_cell(y, G.ky, ry), iz = round_cell(z, G.kz, rz);
+    int ix, iy;
+    float2 rxy;
+    float rz;
+    round_cell2(xy, G.kx, G.ky, ix, iy, rxy);
+    const int iz = round_cell(z, G.kz, rz);
+    const float rx = rxy.x, ry = rxy.y;
     const bool near = (fabsf(rx) > lim) | (fabsf(ry) > lim) | (fabsf(rz) > lim);
     if (!near) {
         int d2 = 0;
@@ -232,125 +279,146 @@ __device__ __forceinline__ void copy_blob(float* dst, const float* __restrict__ 
     }
 }
 
-// One link of one state in single precision: joint transform, T = T_parent * J, the sphere trees riding on the link.
-// `T` holds the previous link's transform on entry and this link's on exit.
+// How a kernel tests sphere-tree pairs (build_model32 picks the mode per robot: Model32Header::n_ptrees > 0 is
+// roots-only).  The two hot kernels are compiled for the mode they run in, so the roots-only form carries neither the
+// descent nor its stack; the other callers read the mode at run time.
+enum PairMode { PAIRS_RUNTIME, PAIRS_ROOTS, PAIRS_DESCENT };
+
+// Forward kinematics of link l in single precision: joint transform J(q), T = T_parent J, kept in the link's slot when
+// a later link branches from it.  `T` holds the previous link's transform on entry and this link's on exit.
+// Returns false, with T unchanged, when the joint value is beyond what the error bound covers (|angle| > V32_MAX_ANGLE,
+// |q| > q_lin_max of a prismatic joint, NaN): the double-precision path decides those.
+//   INTERP: the joint value is qa + alpha (qb - qa), continuous variables along the shortest arc (qb = nullptr: qa);
+//   else qa.  var_type: SMPLGPU_VAR_* per planning variable
+template <bool INTERP>
+__device__ __forceinline__ bool link_fk32(const S32& S, const int* __restrict__ var_type, const double* __restrict__ qa,
+                                          const double* __restrict__ qb, double alpha, float* slots, int l, Xf32& T)
+{
+    const Model32Header* H = S.h;
+    const int4 li = S.link_i[l];   // parent, fn, var, slot
+    const int fn = li.y;
+    float sn = 0.0f, cs = 1.0f, lin = 0.0f;
+    if (li.z >= 0) {
+        double val = qa[li.z];
+        if (INTERP && qb != nullptr) {
+            const double a = val, b = qb[li.z];
+            const double diff = (var_type[li.z] == 1) ? normalize_angle(b - a) : (b - a);
+            val = a + alpha * diff;
+        }
+        const double h = hi_part(val);
+        const float hi = (float)h;
+        if (fn == 5) {
+            if (!(fabsf(hi) <= H->q_lin_max)) {
+                return false;
+            }
+            lin = hi;
+        } else {
+            if (!(fabsf(hi) <= V32_MAX_ANGLE)) {
+                return false;   // also catches NaN / inf
+            }
+            const float lo = (float)(val - h);
+            float s0, c0;
+            sincosf(hi, &s0, &c0);
+            sn = fmaf(lo, c0, s0);
+            cs = fmaf(-lo, s0, c0);
+        }
+    }
+    Xf32 O, J;
+    load12(S.origin + 12 * l, O);
+    if (fn == 0) {
+        J = O;
+    } else if (fn <= 3) {
+        // rotation about x (1), y (2), z (3): two columns of the origin's rotation mix; rows 0 and 1 packed, row 2
+        // scalar, (-sn) o = -(sn o) exactly
+        const float nsn = -sn;
+        J = O;
+        if (fn == 1) {
+            J.c[1] = vfma(cs, O.c[1], vmul(sn, O.c[2]));
+            J.c[2] = vfma(cs, O.c[2], vmul(nsn, O.c[1]));
+            J.r2[1] = vfma(cs, O.r2[1], vmul(sn, O.r2[2]));
+            J.r2[2] = vfma(cs, O.r2[2], vmul(nsn, O.r2[1]));
+        } else if (fn == 2) {
+            J.c[0] = vfma(cs, O.c[0], vmul(nsn, O.c[2]));
+            J.c[2] = vfma(sn, O.c[0], vmul(cs, O.c[2]));
+            J.r2[0] = vfma(cs, O.r2[0], vmul(nsn, O.r2[2]));
+            J.r2[2] = vfma(sn, O.r2[0], vmul(cs, O.r2[2]));
+        } else {
+            J.c[0] = vfma(cs, O.c[0], vmul(sn, O.c[1]));
+            J.c[1] = vfma(cs, O.c[1], vmul(nsn, O.c[0]));
+            J.r2[0] = vfma(cs, O.r2[0], vmul(sn, O.r2[1]));
+            J.r2[1] = vfma(cs, O.r2[1], vmul(nsn, O.r2[0]));
+        }
+    } else if (fn == 4) {
+        const float4 ax = S.axis[l];
+        const float k = 1.0f - cs;
+        const float cx = k * ax.x, cy = k * ax.y, cz = k * ax.z;
+        Xf32 A;
+        A.c[0] = make_float2(fmaf(cx, ax.x, cs), fmaf(cx, ax.y, sn * ax.z));
+        A.c[1] = make_float2(fmaf(cx, ax.y, -sn * ax.z), fmaf(cy, ax.y, cs));
+        A.c[2] = make_float2(fmaf(cx, ax.z, sn * ax.y), fmaf(cy, ax.z, -sn * ax.x));
+        A.c[3] = make_float2(0.0f, 0.0f);
+        A.r2[0] = fmaf(cx, ax.z, -sn * ax.y); A.r2[1] = fmaf(cy, ax.z, sn * ax.x); A.r2[2] = fmaf(cz, ax.z, cs); A.r2[3] = 0.0f;
+        xf32_mul(O, A, J);
+    } else {
+        const float4 ax = S.axis[l];   // inv_res * third column of the origin
+        J = O;   // origin * Translate(0, 0, q): translation += third column * q, in cells
+        J.c[3] = vfma(lin, make_float2(ax.x, ax.y), O.c[3]);
+        J.r2[3] = vfma(lin, ax.z, O.r2[3]);
+    }
+    Xf32 P;
+    if (li.x < 0) {
+        load12(S.base + 12 * l, P);
+    } else if (li.x == l - 1) {
+        P = T;
+    } else {
+        slot32_load(slots, S.link_i[li.x].w, P);
+    }
+    xf32_mul(P, J, T);
+    if (li.w >= 0) {
+        slot32_store(slots, li.w, T);
+    }
+    return true;
+}
+
+// One link of one state in single precision: link_fk32, then the sphere trees riding on the link.
 // Returns 1 = go on with the next link, 0 = certainly invalid, 2 = needs double precision right away; `amb` collects
 // undecidable tests.
-//   var_type: SMPLGPU_VAR_* per planning variable (continuous variables interpolate along the shortest arc)
+template <bool INTERP, int PM>
 __device__ __forceinline__ int link_step32(const S32& S, const int* __restrict__ var_type, const uint16_t* __restrict__ df,
                                            const Grid32& G, const double* __restrict__ qa, const double* __restrict__ qb,
                                            double alpha, float* slots, int l, Xf32& T, bool& amb, Counters& cnt)
 {
     const Model32Header* H = S.h;
+    if (!link_fk32<INTERP>(S, var_type, qa, qb, alpha, slots, l, T)) {
+        return 2;
+    }
     const float lim = 0.5f - H->eps_cells;
-    {
-        const int4 li = S.link_i[l];   // parent, fn, var, slot
-        const int fn = li.y;
-        float sn = 0.0f, cs = 1.0f, lin = 0.0f;
-        if (li.z >= 0) {
-            const double a = qa[li.z];
-            double val = a;
-            if (qb != nullptr) {
-                const double b = qb[li.z];
-                const double diff = (var_type[li.z] == 1) ? normalize_angle(b - a) : (b - a);
-                val = a + alpha * diff;
-            }
-            const double h = hi_part(val);
-            const float hi = (float)h;
-            if (fn == 5) {
-                if (!(fabsf(hi) <= H->q_lin_max)) {
-                    return 2;
-                }
-                lin = hi;
-            } else {
-                if (!(fabsf(hi) <= V32_MAX_ANGLE)) {
-                    return 2;   // also catches NaN / inf
-                }
-                const float lo = (float)(val - h);
-                float s0, c0;
-                sincosf(hi, &s0, &c0);
-                sn = fmaf(lo, c0, s0);
-                cs = fmaf(-lo, s0, c0);
-            }
+    const bool save_roots = PM == PAIRS_ROOTS || (PM == PAIRS_RUNTIME && H->n_ptrees > 0);
+    // sphere trees riding on this link: stackless pre-order descent
+    const int2 nr = S.link_n[l];
+    int node = nr.x;
+    while (node < nr.y) {
+        const float4 c = S.node_c[node];
+        const int4 ni = S.node_i[node];   // skip, thresh, pair-tree index, -
+        float2 xy;
+        float z;
+        xf32_point(T, c.x, c.y, c.z, xy, z);
+        if (save_roots && ni.z >= 0) {
+            // root of a tree that takes part in pair tests: keep its centre
+            float* o = slots + ((size_t)H->n_slots * 12 + (size_t)ni.z * 3) * blockDim.x + threadIdx.x;
+            o[0] = xy.x; o[blockDim.x] = xy.y; o[2 * blockDim.x] = z;
         }
-        Xf32 O, J;
-        load12(S.origin + 12 * l, O);
-        if (fn == 0) {
-            J = O;
-        } else if (fn <= 3) {
-#pragma unroll
-            for (int r = 0; r < 3; ++r) {
-                const float o0 = O.m[4 * r], o1 = O.m[4 * r + 1], o2 = O.m[4 * r + 2];
-                float t0, t1, t2;
-                if (fn == 1) {
-                    t0 = o0;
-                    t1 = fmaf(cs, o1, sn * o2);
-                    t2 = fmaf(cs, o2, -sn * o1);
-                } else if (fn == 2) {
-                    t0 = fmaf(cs, o0, -sn * o2);
-                    t1 = o1;
-                    t2 = fmaf(sn, o0, cs * o2);
-                } else {
-                    t0 = fmaf(o0, cs, o1 * sn);
-                    t1 = fmaf(o1, cs, -o0 * sn);
-                    t2 = o2;
-                }
-                J.m[4 * r] = t0; J.m[4 * r + 1] = t1; J.m[4 * r + 2] = t2; J.m[4 * r + 3] = O.m[4 * r + 3];
-            }
-        } else if (fn == 4) {
-            const float4 ax = S.axis[l];
-            const float k = 1.0f - cs;
-            const float cx = k * ax.x, cy = k * ax.y, cz = k * ax.z;
-            Xf32 A;
-            A.m[0] = fmaf(cx, ax.x, cs);       A.m[1] = fmaf(cx, ax.y, -sn * ax.z); A.m[2] = fmaf(cx, ax.z, sn * ax.y);  A.m[3] = 0.0f;
-            A.m[4] = fmaf(cx, ax.y, sn * ax.z); A.m[5] = fmaf(cy, ax.y, cs);         A.m[6] = fmaf(cy, ax.z, -sn * ax.x); A.m[7] = 0.0f;
-            A.m[8] = fmaf(cx, ax.z, -sn * ax.y); A.m[9] = fmaf(cy, ax.z, sn * ax.x); A.m[10] = fmaf(cz, ax.z, cs);        A.m[11] = 0.0f;
-            xf32_mul(O, A, J);
+        ++cnt.lookups;
+        const int r = lookup32(df, G, lim, xy, z, ni.y);
+        if (r == 1) {
+            node = ni.x;
+        } else if (r == 2) {
+            amb = true;       // undecidable here: do not descend, let double precision decide unless a
+            node = ni.x;      // certain collision shows up elsewhere
+        } else if (ni.x == node + 1) {
+            return 0;         // failing leaf below certainly failing ancestors
         } else {
-            const float4 ax = S.axis[l];   // inv_res * third column of the origin
-            J = O;   // origin * Translate(0, 0, q): translation += third column * q, in cells
-            J.m[3] = fmaf(ax.x, lin, O.m[3]);
-            J.m[7] = fmaf(ax.y, lin, O.m[7]);
-            J.m[11] = fmaf(ax.z, lin, O.m[11]);
-        }
-        Xf32 P;
-        if (li.x < 0) {
-            load12(S.base + 12 * l, P);
-        } else if (li.x == l - 1) {
-            P = T;
-        } else {
-            slot32_load(slots, S.link_i[li.x].w, P);
-        }
-        xf32_mul(P, J, T);
-        if (li.w >= 0) {
-            slot32_store(slots, li.w, T);
-        }
-
-        // sphere trees riding on this link: stackless pre-order descent
-        const int2 nr = S.link_n[l];
-        int node = nr.x;
-        while (node < nr.y) {
-            const float4 c = S.node_c[node];
-            const int4 ni = S.node_i[node];   // skip, thresh, pair-tree index, -
-            float x, y, z;
-            xf32_point(T, c.x, c.y, c.z, x, y, z);
-            if (H->n_ptrees > 0 && ni.z >= 0) {
-                // root of a tree that takes part in pair tests: keep its centre
-                float* o = slots + ((size_t)H->n_slots * 12 + (size_t)ni.z * 3) * blockDim.x + threadIdx.x;
-                o[0] = x; o[blockDim.x] = y; o[2 * blockDim.x] = z;
-            }
-            ++cnt.lookups;
-            const int r = lookup32(df, G, lim, x, y, z, ni.y);
-            if (r == 1) {
-                node = ni.x;
-            } else if (r == 2) {
-                amb = true;       // undecidable here: do not descend, let double precision decide unless a
-                node = ni.x;      // certain collision shows up elsewhere
-            } else if (ni.x == node + 1) {
-                return 0;         // failing leaf below certainly failing ancestors
-            } else {
-                ++node;
-            }
+            ++node;
         }
     }
     return 1;
@@ -358,47 +426,51 @@ __device__ __forceinline__ int link_step32(const S32& S, const int* __restrict__
 
 // The sphere-tree pairs of one state whose link chain is done (transforms / root centres in `slots`).
 // Returns 1 = certainly valid, 0 = certainly invalid, 2 = needs double precision.
-__device__ __forceinline__ int pairs32(const S32& S, float* slots, bool amb, Counters& cnt)
+__device__ __forceinline__ int pairs32_roots(const S32& S, float* slots, bool amb, Counters& cnt)
 {
     const Model32Header* H = S.h;
     const int np = H->n_pairs;
-    if (H->n_ptrees > 0) {
-        // Sphere-tree pairs: only the root spheres are tested here, from the root centres saved above.  Roots that
-        // are certainly apart prune the pair, which is what happens in all but a handful of states; a pair of
-        // overlapping single-sphere trees is a certain collision; anything else (overlapping roots that need the
-        // descent, or an undecidable distance) goes to the double-precision kernel, which keeps the link
-        // transforms the descent needs.
-        const float* rp = slots + (size_t)H->n_slots * 12 * blockDim.x + threadIdx.x;
-        for (int pi = 0; pi < np; ++pi) {
-            const int4 pr = S.pair[pi];   // pair-tree index a, b; root node a, b
-            const float* pa = rp + (size_t)pr.x * 3 * blockDim.x;
-            const float* pb = rp + (size_t)pr.y * 3 * blockDim.x;
-            const float dx = pb[0] - pa[0], dy = pb[blockDim.x] - pa[blockDim.x], dz = pb[2 * blockDim.x] - pa[2 * blockDim.x];
-            ++cnt.pairs;
-            const float cd2 = fmaf(dx, dx, fmaf(dy, dy, dz * dz));
-            const float rr = S.node_c[pr.z].w + S.node_c[pr.w].w;
-            const float rr2 = rr * rr;
-            const float tol = fmaf(H->pair_k, sqrtf(cd2) + rr, 2e-6f * (cd2 + rr2));
-            const float d = cd2 - rr2;
-            if (d > tol) {
-                continue;
-            }
-            const int4 i1 = S.node_i[pr.z], i2 = S.node_i[pr.w];
-            if (d < -tol && i1.x == pr.z + 1 && i2.x == pr.w + 1) {
-                bool allowed = false;
-                for (int k = 0; k < H->n_allowed; ++k) {
-                    const int2 al = S.allowed[k];
-                    allowed |= (al.x == pr.z && al.y == pr.w) || (al.x == pr.w && al.y == pr.z);
-                }
-                if (!allowed) {
-                    return 0;
-                }
-                continue;
-            }
-            amb = true;
+    // Sphere-tree pairs: only the root spheres are tested here, from the root centres saved above.  Roots that
+    // are certainly apart prune the pair, which is what happens in all but a handful of states; a pair of
+    // overlapping single-sphere trees is a certain collision; anything else (overlapping roots that need the
+    // descent, or an undecidable distance) goes to the double-precision kernel, which keeps the link
+    // transforms the descent needs.
+    const float* rp = slots + (size_t)H->n_slots * 12 * blockDim.x + threadIdx.x;
+    for (int pi = 0; pi < np; ++pi) {
+        const int4 pr = S.pair[pi];   // pair-tree index a, b; root node a, b
+        const float* pa = rp + (size_t)pr.x * 3 * blockDim.x;
+        const float* pb = rp + (size_t)pr.y * 3 * blockDim.x;
+        const float dx = pb[0] - pa[0], dy = pb[blockDim.x] - pa[blockDim.x], dz = pb[2 * blockDim.x] - pa[2 * blockDim.x];
+        ++cnt.pairs;
+        const float cd2 = fmaf(dx, dx, fmaf(dy, dy, dz * dz));
+        const float rr = S.node_c[pr.z].w + S.node_c[pr.w].w;
+        const float rr2 = rr * rr;
+        const float tol = fmaf(H->pair_k, sqrtf(cd2) + rr, 2e-6f * (cd2 + rr2));
+        const float d = cd2 - rr2;
+        if (d > tol) {
+            continue;
         }
-        return amb ? 2 : 1;
+        const int4 i1 = S.node_i[pr.z], i2 = S.node_i[pr.w];
+        if (d < -tol && i1.x == pr.z + 1 && i2.x == pr.w + 1) {
+            bool allowed = false;
+            for (int k = 0; k < H->n_allowed; ++k) {
+                const int2 al = S.allowed[k];
+                allowed |= (al.x == pr.z && al.y == pr.w) || (al.x == pr.w && al.y == pr.z);
+            }
+            if (!allowed) {
+                return 0;
+            }
+            continue;
+        }
+        amb = true;
     }
+    return amb ? 2 : 1;
+}
+
+__device__ __forceinline__ int pairs32_descent(const S32& S, float* slots, bool amb, Counters& cnt)
+{
+    const Model32Header* H = S.h;
+    const int np = H->n_pairs;
     // Sphere-tree pairs, full descent (robots whose pair roots overlap often, e.g. two arms + torso): the
     // transforms of all links with paired trees are in the slots.
     int stack[MAX_TREE_DEPTH];
@@ -412,13 +484,14 @@ __device__ __forceinline__ int pairs32(const S32& S, float* slots, bool amb, Cou
             const float4 c1 = S.node_c[n1], c2 = S.node_c[n2];
             const int4 i1 = S.node_i[n1], i2 = S.node_i[n2];
             Xf32 A;
-            float x1, y1, z1, x2, y2, z2;
+            float2 xy1, xy2;
+            float z1, z2;
             slot32_load(slots, i1.z, A);
-            xf32_point(A, c1.x, c1.y, c1.z, x1, y1, z1);
+            xf32_point(A, c1.x, c1.y, c1.z, xy1, z1);
             slot32_load(slots, i2.z, A);
-            xf32_point(A, c2.x, c2.y, c2.z, x2, y2, z2);
+            xf32_point(A, c2.x, c2.y, c2.z, xy2, z2);
             ++cnt.pairs;
-            const float dx = x2 - x1, dy = y2 - y1, dz = z2 - z1;
+            const float dx = xy2.x - xy1.x, dy = xy2.y - xy1.y, dz = z2 - z1;
             const float cd2 = fmaf(dx, dx, fmaf(dy, dy, dz * dz));
             const float rr = c1.w + c2.w;
             const float rr2 = rr * rr;
@@ -468,21 +541,43 @@ __device__ __forceinline__ int pairs32(const S32& S, float* slots, bool amb, Cou
     return amb ? 2 : 1;
 }
 
+template <int PM>
+__device__ __forceinline__ int pairs32(const S32& S, float* slots, bool amb, Counters& cnt)
+{
+    if constexpr (PM == PAIRS_ROOTS) {
+        return pairs32_roots(S, slots, amb, cnt);
+    } else if constexpr (PM == PAIRS_DESCENT) {
+        return pairs32_descent(S, slots, amb, cnt);
+    } else {
+        return S.h->n_ptrees > 0 ? pairs32_roots(S, slots, amb, cnt) : pairs32_descent(S, slots, amb, cnt);
+    }
+}
+
 // One state in single precision.  Returns 1 = certainly valid, 0 = certainly invalid, 2 = needs double precision.
-__device__ int check_state32(const S32& S, const int* __restrict__ var_type, const uint16_t* __restrict__ df,
-                             const Grid32& G, const double* __restrict__ qa, const double* __restrict__ qb,
-                             double alpha, float* slots, Counters& cnt)
+template <bool INTERP, int PM>
+__device__ __forceinline__ int check_state32_t(const S32& S, const int* __restrict__ var_type,
+                                               const uint16_t* __restrict__ df, const Grid32& G,
+                                               const double* __restrict__ qa, const double* __restrict__ qb,
+                                               double alpha, float* slots, Counters& cnt)
 {
     Xf32 T;
     bool amb = false;
     const int nl = S.h->n_links;
     for (int l = 0; l < nl; ++l) {
-        const int r = link_step32(S, var_type, df, G, qa, qb, alpha, slots, l, T, amb, cnt);
+        const int r = link_step32<INTERP, PM>(S, var_type, df, G, qa, qb, alpha, slots, l, T, amb, cnt);
         if (r != 1) {
             return r;
         }
     }
-    return pairs32(S, slots, amb, cnt);
+    return pairs32<PM>(S, slots, amb, cnt);
+}
+
+// the general form (the planner's kernels): a waypoint qa + alpha (qb - qa) (qb = nullptr: the state qa), either pair mode
+__device__ int check_state32(const S32& S, const int* __restrict__ var_type, const uint16_t* __restrict__ df,
+                             const Grid32& G, const double* __restrict__ qa, const double* __restrict__ qb,
+                             double alpha, float* slots, Counters& cnt)
+{
+    return check_state32_t<true, PAIRS_RUNTIME>(S, var_type, df, G, qa, qb, alpha, slots, cnt);
 }
 
 // warp-aggregated append of item ids to the list of items that need double precision
@@ -509,7 +604,8 @@ __device__ __forceinline__ void append_uncertain(bool push, int item, int* __res
 
 // dynamic shared memory: blob | slots (n_slots * 12 * blockDim floats) | root centres (n_ptrees * 3 * blockDim floats)
 //                        | edges: (blockDim + 1) offsets, blockDim ok, blockDim unc, blockDim counts
-__global__ void V32_BOUNDS
+template <int PM>
+__global__ void V32_STATES_BOUNDS
 states_valid32_kernel(const float* __restrict__ blob_g, int blob_words, const DevModel* __restrict__ M,
                       const uint16_t* __restrict__ df, Grid32 G, const double* __restrict__ q, int n,
                       uint8_t* __restrict__ verdict, int* __restrict__ unc_list, int* __restrict__ unc_count,
@@ -540,7 +636,7 @@ states_valid32_kernel(const float* __restrict__ blob_g, int blob_words, const De
         int r = 0;
         if (i < n) {
             ++cnt.waypoints;
-            r = check_state32(S, M->var_type, df, G, q + (size_t)i * S.h->dof, nullptr, 0.0, slots, cnt);
+            r = check_state32_t<false, PM>(S, M->var_type, df, G, q + (size_t)i * S.h->dof, nullptr, 0.0, slots, cnt);
             verdict[i] = r == 1 ? 1 : 0;
         }
         append_uncertain(i < n && r == 2, i, unc_list, unc_count, stats);
@@ -548,7 +644,8 @@ states_valid32_kernel(const float* __restrict__ blob_g, int blob_words, const De
     flush_counters(cnt, stats);
 }
 
-__global__ void V32_BOUNDS
+template <int PM>
+__global__ void V32_EDGES_BOUNDS
 edges_valid32_kernel(const float* __restrict__ blob_g, int blob_words, const DevModel* __restrict__ M,
                      const uint16_t* __restrict__ df, Grid32 G, const double* __restrict__ q0,
                      const double* __restrict__ q1, int n, uint8_t* __restrict__ verdict, int* __restrict__ counts,
@@ -604,7 +701,8 @@ edges_valid32_kernel(const float* __restrict__ blob_g, int blob_words, const Dev
     int ok = 1, unc = 0;
     if (count > 0) {
         ++cnt.waypoints;
-        const int r = check_state32(S, M->var_type, df, G, q0 + (size_t)i * dof, q1 + (size_t)i * dof, 0.0, slots, cnt);
+        const int r = check_state32_t<true, PM>(S, M->var_type, df, G, q0 + (size_t)i * dof, q1 + (size_t)i * dof, 0.0,
+                                                slots, cnt);
         ok = r != 0;
         unc = r == 2;
     }
@@ -662,8 +760,8 @@ edges_valid32_kernel(const float* __restrict__ blob_g, int blob_words, const Dev
                 const double inv = 1.0 / (double)(s_cnt[e] - 1); // m_waypoint_count_inv
                 const double alpha = (double)w * inv;
                 ++cnt.waypoints;
-                const int r = check_state32(S, M->var_type, df, G, q0 + (size_t)(first + e) * dof, q1 + (size_t)(first + e) * dof,
-                                            alpha, slots, cnt);
+                const int r = check_state32_t<true, PM>(S, M->var_type, df, G, q0 + (size_t)(first + e) * dof,
+                                                        q1 + (size_t)(first + e) * dof, alpha, slots, cnt);
                 // several lanes may hold waypoints of one edge: atomics make the concurrent same-value writes a
                 // defined (racecheck-clean) update; they only run on a failing / undecided waypoint
                 if (r == 0) {
@@ -947,9 +1045,9 @@ __device__ __forceinline__ void persistent_items32(const S32& S, const int* __re
             if (!live_fn(item)) {
                 item = -1;                       // abandoned: its edge is invalid anyway, nothing to report
             } else {
-                int r = link_step32(S, var_type, df, G, qa, qb, alpha, slots, l, T, amb, cnt);
+                int r = link_step32<true, PAIRS_RUNTIME>(S, var_type, df, G, qa, qb, alpha, slots, l, T, amb, cnt);
                 if (r == 1 && ++l == nl) {
-                    r = pairs32(S, slots, amb, cnt);
+                    r = pairs32<PAIRS_RUNTIME>(S, slots, amb, cnt);
                     fin = true;
                     res = r;
                 } else if (r != 1) {
@@ -1198,76 +1296,22 @@ fk_centers32_kernel(const float* __restrict__ blob_g, int blob_words, const doub
     const double* qa = q + (size_t)i * H->dof;
     Xf32 T;
     for (int l = 0; l < H->n_links; ++l) {
-        const int4 li = S.link_i[l];
-        const int fn = li.y;
-        float sn = 0.0f, cs = 1.0f, lin = 0.0f;
-        if (li.z >= 0) {
-            const double val = qa[li.z];
-            const double h = hi_part(val);
-            const float hi = (float)h;
-            if (fn == 5) {
-                lin = hi;
-            } else {
-                const float lo = (float)(val - h);
-                float s0, c0;
-                sincosf(hi, &s0, &c0);
-                sn = fmaf(lo, c0, s0);
-                cs = fmaf(-lo, s0, c0);
+        if (!link_fk32<false>(S, nullptr, qa, nullptr, 0.0, slots, l, T)) {
+            // a joint value the bound does not cover: the kernels leave this state to double precision
+            for (int k = 0; k < 3 * H->n_nodes; ++k) {
+                out[(size_t)i * H->n_nodes * 3 + k] = __int_as_float(0x7fffffff);
             }
-        }
-        Xf32 O, J;
-        load12(S.origin + 12 * l, O);
-        if (fn == 0) {
-            J = O;
-        } else if (fn <= 3) {
-            for (int r = 0; r < 3; ++r) {
-                const float o0 = O.m[4 * r], o1 = O.m[4 * r + 1], o2 = O.m[4 * r + 2];
-                float t0, t1, t2;
-                if (fn == 1) {
-                    t0 = o0; t1 = fmaf(cs, o1, sn * o2); t2 = fmaf(cs, o2, -sn * o1);
-                } else if (fn == 2) {
-                    t0 = fmaf(cs, o0, -sn * o2); t1 = o1; t2 = fmaf(sn, o0, cs * o2);
-                } else {
-                    t0 = fmaf(o0, cs, o1 * sn); t1 = fmaf(o1, cs, -o0 * sn); t2 = o2;
-                }
-                J.m[4 * r] = t0; J.m[4 * r + 1] = t1; J.m[4 * r + 2] = t2; J.m[4 * r + 3] = O.m[4 * r + 3];
-            }
-        } else if (fn == 4) {
-            const float4 ax = S.axis[l];
-            const float k = 1.0f - cs;
-            const float cx = k * ax.x, cy = k * ax.y, cz = k * ax.z;
-            Xf32 A;
-            A.m[0] = fmaf(cx, ax.x, cs);       A.m[1] = fmaf(cx, ax.y, -sn * ax.z); A.m[2] = fmaf(cx, ax.z, sn * ax.y);  A.m[3] = 0.0f;
-            A.m[4] = fmaf(cx, ax.y, sn * ax.z); A.m[5] = fmaf(cy, ax.y, cs);         A.m[6] = fmaf(cy, ax.z, -sn * ax.x); A.m[7] = 0.0f;
-            A.m[8] = fmaf(cx, ax.z, -sn * ax.y); A.m[9] = fmaf(cy, ax.z, sn * ax.x); A.m[10] = fmaf(cz, ax.z, cs);        A.m[11] = 0.0f;
-            xf32_mul(O, A, J);
-        } else {
-            const float4 ax = S.axis[l];
-            J = O;
-            J.m[3] = fmaf(ax.x, lin, O.m[3]);
-            J.m[7] = fmaf(ax.y, lin, O.m[7]);
-            J.m[11] = fmaf(ax.z, lin, O.m[11]);
-        }
-        Xf32 P;
-        if (li.x < 0) {
-            load12(S.base + 12 * l, P);
-        } else if (li.x == l - 1) {
-            P = T;
-        } else {
-            slot32_load(slots, S.link_i[li.x].w, P);
-        }
-        xf32_mul(P, J, T);
-        if (li.w >= 0) {
-            slot32_store(slots, li.w, T);
+            return;
         }
         const int2 nr = S.link_n[l];
         for (int node = nr.x; node < nr.y; ++node) {
             const float4 c = S.node_c[node];
-            float x, y, z;
-            xf32_point(T, c.x, c.y, c.z, x, y, z);
+            float2 xy;
+            float z;
+            xf32_point(T, c.x, c.y, c.z, xy, z);
             float* o = out + ((size_t)i * H->n_nodes + S.node_orig[node]) * 3;
-            o[0] = (float)((double)x * res + ox);
-            o[1] = (float)((double)y * res + oy);
+            o[0] = (float)((double)xy.x * res + ox);
+            o[1] = (float)((double)xy.y * res + oy);
             o[2] = (float)((double)z * res + oz);
         }
     }

@@ -75,9 +75,9 @@ def sass():
     cur, name = [], None
     def flush():
         if name and cur:
-            # "void bfs_tiles_kernel<4>" -> bfs_tiles_kernel_rpt4
+            # "void bfs_tiles_kernel<4>" -> bfs_tiles_kernel_rpt4, "void states_valid32_kernel<1>" -> states_valid32_kernel_1
             short = re.sub(r"^void\s+", "", name)
-            short = re.sub(r"<(\d+)>", r"_rpt\1", short)
+            short = re.sub(r"<(\d+)>", r"_rpt\1" if short.startswith("bfs_tiles_kernel") else r"_\1", short)
             short = re.sub(r"[^A-Za-z0-9_]", "", short)
             with open(os.path.join(d, short + ".sass"), "w") as f:
                 f.write("\n".join(cur) + "\n")
